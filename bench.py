@@ -12,7 +12,12 @@ state of the timed run checked against the CPU oracle).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload rollout|train]
                   [--precision f32|f16_tc] [--envs 8192] [--humans 5] [--query-env 0|1] [--sim circle|square]
-                  [--no-extra] [--sustained-seconds 3]
+                  [--no-extra] [--sustained-seconds 3] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step of the main configuration computed (rank 0's envs) as
+DIR/<name>.npy, so that two builds can be compared output for output: the same arguments give the same inputs.
+It covers the rollout workload of --impl ours only (--workload train and --impl reference refuse it), and with
+several GPUs only rank 0's envs are written.
 
 --impl reference times the reference's CPU algorithm (the oracle port, oracle/crowdnav_oracle.c -- the
 reference itself is Python + an un-vendored rvo2 and cannot travel to the GPU box) on the host cores.
@@ -201,6 +206,34 @@ def parity_sample(o, pol, env, query_env, weights, n, seed=0):
             "checker": "oracle/crowdnav_oracle.c (CPU), same state, same weights"}
 
 
+DUMP_LIMIT = 64 * 10**6     # bytes written by --dump-outputs in all
+
+
+def step_outputs(env, pol):
+    """What a caller of cn_rollout_step receives from the last step: the next state (auto-reset envs already regenerated),
+    the step's reward / done / info / dmin, the chosen action and the lookahead's action values."""
+    agents, times = env.get_state()
+    reward, done, info, dmin = env.read_outputs()
+    action_xy, action_idx = env.pending_actions()
+    _, values = pol.read(env)
+    return {"agents": agents, "times": times, "reward": reward, "done": done.astype(np.float32),
+            "info": info.astype(np.float32), "dmin": dmin, "action_xy": action_xy,
+            "action_index": action_idx.astype(np.float32), "values": values}
+
+
+def dump_outputs(path, outs, limit=DUMP_LIMIT):
+    """(E, ...) arrays -> path/<name>.npy.  Above `limit` bytes, a fixed seeded sample of the envs; env_index.npy says which."""
+    E = len(outs["reward"])
+    per_env = sum(v.nbytes for v in outs.values()) // E + 8
+    n = min(E, (limit - 4096 * (len(outs) + 1)) // per_env)
+    idx = np.arange(E) if n == E else np.sort(np.random.RandomState(0).choice(E, n, replace=False))
+    outs = {k: v[idx] for k, v in outs.items()}
+    outs["env_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in outs.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -224,7 +257,12 @@ def main():
     ap.add_argument("--train-batches", type=int, default=100, help="--workload train: SGD batches per iteration")
     ap.add_argument("--trainer", default="fused", choices=["eager", "graph", "fused"],
                     help="--workload train: fused = csrc/trainer.cu (SARL, parity-tested against the reference Trainer), graph = CUDA-graph replay of torch autograd")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "ours" or a.workload != "rollout"):
+        ap.error("--dump-outputs needs --impl ours --workload rollout")
     a.warmup = max(a.warmup, 3)
     if a.impl == "reference":
         return run_reference(a)
@@ -290,9 +328,9 @@ def main():
                             "ms": la_ms, "flops_per_env_step": F, "kernels_ms": kms}
         return out
 
-    def measure(E, H, sim, query_env, steps, warmup, clocks=False):
+    def measure(E, H, sim, query_env, steps, warmup, clocks=False, dump=None):
         """K timed rollout steps of one configuration (device time per step, L2 flushed between steps, max over ranks),
-        then the per-phase / per-kernel breakdown of the same step."""
+        then the per-phase / per-kernel breakdown of the same step.  dump: directory for the last timed step's outputs."""
         env, pol = make(E, H, sim)
         # pre-roll: the envs start in lock step (all episodes at t = 0, humans far apart, trivially feasible ORCA problems);
         # 64 untimed steps spread them over the episode (crossings, dangers, finished + re-generated episodes) before timing
@@ -314,6 +352,8 @@ def main():
         launches = pol.lib.cn_launch_count() - launches0
         dev_ms = sum(s.elapsed_time(e) for s, e in ev)
         clk = sampler.stop() if sampler else None
+        if dump and rank == 0:                       # before the breakdown below steps the envs further
+            dump_outputs(dump, step_outputs(env, pol))
         # per-phase breakdown (events around each phase) and per-kernel durations of the lookahead
         phases = {"orca": 0.0, "lookahead": 0.0, "step": 0.0}
         kms = {"features": 0.0, "rows": 0.0, "mlp3": 0.0, "argmax": 0.0} if tc else None
@@ -345,7 +385,7 @@ def main():
 
     # ---------------- main configuration (BASELINE.json configs[1]) ----------------
     E, H = a.envs, a.humans
-    env, pol, main_res = measure(E, H, a.sim, a.query_env, a.steps, a.warmup, clocks=True)
+    env, pol, main_res = measure(E, H, a.sim, a.query_env, a.steps, a.warmup, clocks=True, dump=a.dump_outputs)
 
     # ---- parity of what was just timed: the state the loop left behind vs the CPU oracle (rank 0) ----
     parity = None

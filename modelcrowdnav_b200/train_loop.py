@@ -193,7 +193,7 @@ def bench_train(a):
     barrier()
     timers = {}
     steps0 = loop.env_steps
-    n_iter = min(a.steps, 20)
+    n_iter = a.steps
     t0 = time.perf_counter()
     for _ in range(n_iter):
         loop.rl_iteration(0.5, a.train_batches, timers=timers)
