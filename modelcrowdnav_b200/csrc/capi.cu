@@ -38,6 +38,48 @@ void cn_trace_mark(const char *name, cudaStream_t s)
     g_trace.push_back({name, s, ev});
 }
 
+// ---- network shapes and state-dict layer lists ---------------------------------------------------
+// The network shape of a configuration (om_dim = 0 without occupancy maps)
+static SarlDims dims_of(const cn_sarl_cfg *c, int om_dim)
+{
+    SarlDims d;
+    memset(&d, 0, sizeof(d));
+    d.in = c->input_dim; d.self_dim = c->self_state_dim;
+    for (int i = 0; i < 2; ++i) { d.m1[i] = c->mlp1_dims[i]; d.m2[i] = c->mlp2_dims[i]; }
+    for (int i = 0; i < 3; ++i) d.at[i] = c->attn_dims[i];
+    for (int i = 0; i < 4; ++i) d.m3[i] = c->mlp3_dims[i];
+    d.net = c->network; d.lstm_h = c->network == CN_NET_LSTM_RL ? c->lstm_hidden : 0;
+    for (int i = 0; i < 4; ++i) d.lm1[i] = c->network == CN_NET_LSTM_RL ? c->lstm_mlp1_dims[i] : 0;
+    d.lstm_in = d.lm1[0] > 0 ? d.lm1[3] : d.in;
+    d.om_dim = om_dim; d.cell_num = c->cell_num; d.om_ch = c->om_channel_size; d.cell_size = c->cell_size;
+    return d;
+}
+
+std::vector<LayerSpec> cn_layers(const SarlDims &d, SarlWeightsDev &w)
+{
+    std::vector<LayerSpec> L;
+    int in = d.in;
+    auto chain = [&](int n, const int *outs, LinearDev *dst) {
+        for (int i = 0; i < n; ++i) { L.push_back({in, outs[i], &dst[i], nullptr}); in = outs[i]; }
+    };
+    if (d.net == CN_NET_CADRL) {                          // value_network.{0,2,4,6} (cadrl.py:22-26)
+        chain(4, d.m3, w.m3);
+    } else if (d.net == CN_NET_LSTM_RL) {                 // [mlp1.*] mlp.* lstm.* (lstm_rl.py:9-16,37-45)
+        if (d.lm1[0] > 0) chain(4, d.lm1, w.lm1);
+        in = d.self_dim + d.lstm_h;
+        chain(4, d.m3, w.m3);
+        L.push_back({d.lstm_in, 4 * d.lstm_h, &w.lih, &w.lhh});
+    } else {                                              // mlp1.* mlp2.* attention.* mlp3.*
+        chain(2, d.m1, w.m1);
+        chain(2, d.m2, w.m2);
+        in = 2 * d.m1[1];
+        chain(3, d.at, w.at);
+        in = d.m2[1] + d.self_dim;
+        chain(4, d.m3, w.m3);
+    }
+    return L;
+}
+
 extern "C" {
 
 /* Developer diagnostic: on = 1 starts recording a timeline of the library's stream operations (one CUDA event per mark),
@@ -450,30 +492,9 @@ static int pad4i(int x) { return (x + 3) & ~3; }
 int64_t cn_policy_param_count(const cn_sarl_cfg *c)
 {
     if (!c) return 0;
+    SarlWeightsDev w;        // only the destinations of the layer list, never written here
     int64_t n = 0;
-    int in = c->input_dim;
-    if (c->network == CN_NET_CADRL) {                       // value_network.{0,2,4,6} (cadrl.py:22-26)
-        for (int i = 0; i < 4; ++i) { n += (int64_t)in * c->mlp3_dims[i] + c->mlp3_dims[i]; in = c->mlp3_dims[i]; }
-        return n;
-    }
-    if (c->network == CN_NET_LSTM_RL) {                     // [mlp1.*] mlp.* lstm.* (lstm_rl.py:9-16,37-45)
-        int lstm_in = c->input_dim;
-        if (c->lstm_mlp1_dims[0] > 0) {
-            for (int i = 0; i < 4; ++i) { n += (int64_t)in * c->lstm_mlp1_dims[i] + c->lstm_mlp1_dims[i]; in = c->lstm_mlp1_dims[i]; }
-            lstm_in = c->lstm_mlp1_dims[3];
-        }
-        in = c->self_state_dim + c->lstm_hidden;
-        for (int i = 0; i < 4; ++i) { n += (int64_t)in * c->mlp3_dims[i] + c->mlp3_dims[i]; in = c->mlp3_dims[i]; }
-        const int64_t G = 4 * (int64_t)c->lstm_hidden;
-        return n + G * lstm_in + G * c->lstm_hidden + 2 * G;
-    }
-    for (int i = 0; i < 2; ++i) { n += (int64_t)in * c->mlp1_dims[i] + c->mlp1_dims[i]; in = c->mlp1_dims[i]; }
-    in = c->mlp1_dims[1];
-    for (int i = 0; i < 2; ++i) { n += (int64_t)in * c->mlp2_dims[i] + c->mlp2_dims[i]; in = c->mlp2_dims[i]; }
-    in = c->mlp1_dims[1] * 2;
-    for (int i = 0; i < 3; ++i) { n += (int64_t)in * c->attn_dims[i] + c->attn_dims[i]; in = c->attn_dims[i]; }
-    in = c->mlp2_dims[1] + c->self_state_dim;
-    for (int i = 0; i < 4; ++i) { n += (int64_t)in * c->mlp3_dims[i] + c->mlp3_dims[i]; in = c->mlp3_dims[i]; }
+    for (const LayerSpec &l : cn_layers(dims_of(c, 0), w)) n += (int64_t)cn_layer_floats(l);
     return n;
 }
 
@@ -554,31 +575,15 @@ int cn_policy_create(const cn_sarl_cfg *cfg, int device, cn_policy **out)
     cn_policy *p = new cn_policy();
     memset(p, 0, sizeof(*p));
     p->device = device; p->cfg = *cfg;
+    p->d = dims_of(cfg, om_dim);
     SarlDims &d = p->d;
-    d.in = cfg->input_dim; d.self_dim = cfg->self_state_dim;
-    for (int i = 0; i < 2; ++i) { d.m1[i] = cfg->mlp1_dims[i]; d.m2[i] = cfg->mlp2_dims[i]; }
-    for (int i = 0; i < 3; ++i) d.at[i] = cfg->attn_dims[i];
-    for (int i = 0; i < 4; ++i) d.m3[i] = cfg->mlp3_dims[i];
-    d.net = cfg->network; d.lstm_h = cfg->network == CN_NET_LSTM_RL ? cfg->lstm_hidden : 0;
-    for (int i = 0; i < 4; ++i) d.lm1[i] = cfg->network == CN_NET_LSTM_RL ? cfg->lstm_mlp1_dims[i] : 0;
-    d.lstm_in = d.lm1[0] > 0 ? d.lm1[3] : d.in;
-    d.om_dim = om_dim; d.cell_num = cfg->cell_num; d.om_ch = cfg->om_channel_size; d.cell_size = cfg->cell_size;
     d.A = build_action_table(cfg, p->action_host);
     p->n_params = cn_policy_param_count(cfg);
 
-    // transposed/padded block: sum over layers of in * pad4(out) + pad4(out)
+    // transposed/padded block: per layer in * pad4(out) + pad4(out) (the LSTM block: for W_ih and for W_hh)
     size_t tsize = 0;
-    {
-        auto add = [&](int in, int o) { tsize += (size_t)in * pad4i(o) + pad4i(o); };
-        add(d.in, d.m1[0]); add(d.m1[0], d.m1[1]);
-        add(d.m1[1], d.m2[0]); add(d.m2[0], d.m2[1]);
-        add(2 * d.m1[1], d.at[0]); add(d.at[0], d.at[1]); add(d.at[1], d.at[2]);
-        add(d.m2[1] + d.self_dim, d.m3[0]); add(d.m3[0], d.m3[1]); add(d.m3[1], d.m3[2]); add(d.m3[2], d.m3[3]);
-        // CADRL / LSTM-RL layouts are subsets of this plus the LSTM block and ValueNetwork2's mlp1
-        add(d.in, d.m3[0]); add(d.self_dim + d.lstm_h, d.m3[0]);
-        add(d.lstm_in, 4 * d.lstm_h); add(d.lstm_h, 4 * d.lstm_h);
-        if (d.lm1[0] > 0) { add(d.in, d.lm1[0]); add(d.lm1[0], d.lm1[1]); add(d.lm1[1], d.lm1[2]); add(d.lm1[2], d.lm1[3]); }
-    }
+    for (const LayerSpec &l : cn_layers(d, p->w))
+        tsize += (size_t)(l.in + 1) * pad4i(l.out) + (l.dst_hh ? (size_t)(l.out / 4 + 1) * pad4i(l.out) : 0);
     cudaError_t e1 = cudaMalloc((void **)&p->action_dev, sizeof(double) * 2 * d.A);
     cudaError_t e2 = cudaMalloc((void **)&p->w_raw, sizeof(float) * p->n_params);
     cudaError_t e3 = cudaMalloc((void **)&p->w_t, sizeof(float) * tsize);
@@ -615,70 +620,31 @@ int cn_policy_load_weights(cn_policy *p, const float *flat, int64_t n, void *str
     if (n != p->n_params) { cn_set_error("expected %lld parameters, got %lld", (long long)p->n_params, (long long)n); return CN_EINVAL; }
     CN_CUDA_CHECK(cudaSetDevice(p->device));
     cudaStream_t s = (cudaStream_t)stream;
-    const SarlDims &d = p->d;
     // host-side transpose to [in][pad4(out)] + bias, one contiguous block
     std::vector<float> t;
-    struct Spec { int in, out; LinearDev *dst; };
-    if (d.net != CN_NET_SARL) {
-        // CADRL: value_network.{0,2,4,6}.  LSTM-RL: [mlp1.{0,2,4,6}] mlp.{0,2,4,6} lstm.weight_ih_l0 [4h][in], weight_hh_l0
-        // [4h][h], bias_ih_l0, bias_hh_l0 (state-dict order of cadrl.py:22-26 / lstm_rl.py:9-16,37-45)
-        std::vector<Spec> sp;
-        if (d.net == CN_NET_CADRL) {
-            int in = d.in;
-            for (int i = 0; i < 4; ++i) { sp.push_back({in, d.m3[i], &p->w.m3[i]}); in = d.m3[i]; }
-        } else {
-            int in = d.in;
-            if (d.lm1[0] > 0) for (int i = 0; i < 4; ++i) { sp.push_back({in, d.lm1[i], &p->w.lm1[i]}); in = d.lm1[i]; }
-            in = d.self_dim + d.lstm_h;
-            for (int i = 0; i < 4; ++i) { sp.push_back({in, d.m3[i], &p->w.m3[i]}); in = d.m3[i]; }
-        }
-        const float *src = flat;
-        auto put = [&](int in, int out, const float *w, const float *b, LinearDev *dst) {
-            const int ld = pad4i(out);
-            const size_t off = t.size();
-            t.resize(off + (size_t)in * ld + ld, 0.0f);
-            for (int o = 0; o < out; ++o)
-                for (int k = 0; k < in; ++k) t[off + (size_t)k * ld + o] = w[(size_t)o * in + k];
-            for (int o = 0; o < out; ++o) t[off + (size_t)in * ld + o] = b[o];
-            dst->wt = p->w_t + off; dst->b = p->w_t + off + (size_t)in * ld;
-            dst->in = in; dst->out = out; dst->ld = ld;
-        };
-        for (auto &x : sp) { put(x.in, x.out, src, src + (size_t)x.in * x.out, x.dst); src += (size_t)x.in * x.out + x.out; }
-        if (d.net == CN_NET_LSTM_RL) {
-            const int G = 4 * d.lstm_h;
-            const float *w_ih = src, *w_hh = w_ih + (size_t)G * d.lstm_in, *b_ih = w_hh + (size_t)G * d.lstm_h, *b_hh = b_ih + G;
-            put(d.lstm_in, G, w_ih, b_ih, &p->w.lih);
-            put(d.lstm_h, G, w_hh, b_hh, &p->w.lhh);
-        }
-        CN_CUDA_CHECK(cudaMemcpyAsync(p->w_t, t.data(), sizeof(float) * t.size(), cudaMemcpyHostToDevice, s));
-        CN_CUDA_CHECK(cudaMemcpyAsync(p->w_raw, flat, sizeof(float) * n, cudaMemcpyHostToDevice, s));
-        CN_CUDA_CHECK(cudaStreamSynchronize(s));
-        if (p->cfg.precision == CN_PREC_F16_TC) {            // CADRL on tensor cores (tc_mlp3_pair_kernel<1>)
-            int rc = cn_tc_load_weights(p, flat, s);
-            if (rc) return rc;
-        }
-        p->weights_loaded = 1;
-        return CN_OK;
-    }
-    Spec specs[11] = {
-        {d.in, d.m1[0], &p->w.m1[0]}, {d.m1[0], d.m1[1], &p->w.m1[1]},
-        {d.m1[1], d.m2[0], &p->w.m2[0]}, {d.m2[0], d.m2[1], &p->w.m2[1]},
-        {2 * d.m1[1], d.at[0], &p->w.at[0]}, {d.at[0], d.at[1], &p->w.at[1]}, {d.at[1], d.at[2], &p->w.at[2]},
-        {d.m2[1] + d.self_dim, d.m3[0], &p->w.m3[0]}, {d.m3[0], d.m3[1], &p->w.m3[1]},
-        {d.m3[1], d.m3[2], &p->w.m3[2]}, {d.m3[2], d.m3[3], &p->w.m3[3]}};
-    const float *src = flat;
-    for (auto &sp : specs) {
-        const int ld = pad4i(sp.out);
+    auto put = [&](int in, int out, const float *w, const float *b, LinearDev *dst) {
+        const int ld = pad4i(out);
         const size_t off = t.size();
-        t.resize(off + (size_t)sp.in * ld + ld, 0.0f);
-        for (int o = 0; o < sp.out; ++o)
-            for (int k = 0; k < sp.in; ++k) t[off + (size_t)k * ld + o] = src[(size_t)o * sp.in + k];
-        src += (size_t)sp.in * sp.out;
-        for (int o = 0; o < sp.out; ++o) t[off + (size_t)sp.in * ld + o] = src[o];
-        src += sp.out;
-        sp.dst->wt = p->w_t + off;
-        sp.dst->b = p->w_t + off + (size_t)sp.in * ld;
-        sp.dst->in = sp.in; sp.dst->out = sp.out; sp.dst->ld = ld;
+        t.resize(off + (size_t)in * ld + ld, 0.0f);
+        for (int o = 0; o < out; ++o)
+            for (int k = 0; k < in; ++k) t[off + (size_t)k * ld + o] = w[(size_t)o * in + k];
+        for (int o = 0; o < out; ++o) t[off + (size_t)in * ld + o] = b[o];
+        dst->wt = p->w_t + off; dst->b = p->w_t + off + (size_t)in * ld;
+        dst->in = in; dst->out = out; dst->ld = ld;
+    };
+    const float *src = flat;
+    for (const LayerSpec &l : cn_layers(p->d, p->w)) {
+        const float *w = src, *b = src + (size_t)l.in * l.out;
+        if (l.dst_hh) {                                   // weight_ih_l0, weight_hh_l0, bias_ih_l0, bias_hh_l0
+            const int h = l.out / 4;
+            const float *w_hh = b;
+            b = w_hh + (size_t)l.out * h;
+            put(l.in, l.out, w, b, l.dst);
+            put(h, l.out, w_hh, b + l.out, l.dst_hh);
+        } else {
+            put(l.in, l.out, w, b, l.dst);
+        }
+        src += cn_layer_floats(l);
     }
     CN_CUDA_CHECK(cudaMemcpyAsync(p->w_t, t.data(), sizeof(float) * t.size(), cudaMemcpyHostToDevice, s));
     CN_CUDA_CHECK(cudaMemcpyAsync(p->w_raw, flat, sizeof(float) * n, cudaMemcpyHostToDevice, s));
@@ -711,6 +677,23 @@ static int check_pair(cn_policy *p, cn_env *env)
     return CN_OK;
 }
 
+// the lookahead of the policy's precision; tail: see cn_lookahead_tc (the FP32 lookahead runs on s alone)
+static int lookahead(cn_policy *p, cn_env *env, int query_env, double epsilon, cudaStream_t s, cudaStream_t tail = nullptr)
+{
+    if (p->cfg.precision == CN_PREC_F16_TC) return cn_lookahead_tc(p, env, query_env, epsilon, s, tail);
+    return cn_lookahead_f32(p, env, query_env, epsilon, s);
+}
+
+// waits for s, then refuses the last lookahead when some env had no finite value (multi_human_rl.py:57-58)
+static int sync_and_check_values(cn_policy *p, cudaStream_t s)
+{
+    int32_t bad = 0;
+    CN_CUDA_CHECK(cudaMemcpyAsync(&bad, p->bad_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CN_CUDA_CHECK(cudaStreamSynchronize(s));
+    if (bad) { cn_set_error("Value network is not well trained. "); return CN_EVALUE; }
+    return CN_OK;
+}
+
 int cn_policy_lookahead(cn_policy *p, cn_env *env, int query_env, double epsilon, void *stream)
 {
     int rc = check_pair(p, env);
@@ -721,8 +704,7 @@ int cn_policy_lookahead(cn_policy *p, cn_env *env, int query_env, double epsilon
         cn_set_error("query_env lookahead needs cn_env_orca for the current state");
         return CN_EINVAL;
     }
-    if (p->cfg.precision == CN_PREC_F16_TC) return cn_lookahead_tc(p, env, query_env, epsilon, s);
-    return cn_lookahead_f32(p, env, query_env, epsilon, s);
+    return lookahead(p, env, query_env, epsilon, s);
 }
 
 int cn_policy_read(cn_policy *p, cn_env *env, int32_t *best_idx, double *values, void *stream)
@@ -732,16 +714,12 @@ int cn_policy_read(cn_policy *p, cn_env *env, int32_t *best_idx, double *values,
     CN_CUDA_CHECK(cudaSetDevice(p->device));
     cudaStream_t s = (cudaStream_t)stream;
     const size_t E = env->p.d.E;
-    int32_t bad = 0;
     if (best_idx) CN_CUDA_CHECK(cudaMemcpyAsync(best_idx, env->action_idx, sizeof(int32_t) * E, cudaMemcpyDeviceToHost, s));
     if (values) {
         if (!p->values) { cn_set_error("no lookahead has been run"); return CN_EINVAL; }
         CN_CUDA_CHECK(cudaMemcpyAsync(values, p->values, sizeof(double) * E * p->d.A, cudaMemcpyDeviceToHost, s));
     }
-    CN_CUDA_CHECK(cudaMemcpyAsync(&bad, p->bad_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    CN_CUDA_CHECK(cudaStreamSynchronize(s));
-    if (bad) { cn_set_error("Value network is not well trained. "); return CN_EVALUE; }
-    return CN_OK;
+    return sync_and_check_values(p, s);
 }
 
 int cn_policy_bad_count(cn_policy *p, int64_t *count, int reset, void *stream)
@@ -831,7 +809,7 @@ static int rollout_step_impl(cn_policy *p, cn_env *env, int query_env, double ep
     // the ORCA result, so ORCA (a latency-bound 16 us kernel) runs on a forked stream beside the lookahead and joins
     // before the env step.  Event fork/join keeps the whole step capturable in a CUDA graph.
     const bool fork = !query_env;
-    cn_trace_mark("orca", fork ? s : s);
+    cn_trace_mark("orca", s);
     if (fork) {
         if (!env->side_stream) {
             CN_CUDA_CHECK(cudaStreamCreateWithFlags(&env->side_stream, cudaStreamNonBlocking));
@@ -843,9 +821,7 @@ static int rollout_step_impl(cn_policy *p, cn_env *env, int query_env, double ep
         if ((rc = cn_launch_orca(env, env->side_stream))) return rc;
         CN_CUDA_CHECK(cudaEventRecord(env->ev_join, env->side_stream));
     } else if ((rc = cn_launch_orca(env, s))) return rc;
-    if (p->cfg.precision == CN_PREC_F16_TC) rc = cn_lookahead_tc(p, env, query_env, epsilon, s, tail);
-    else rc = cn_lookahead_f32(p, env, query_env, epsilon, s);
-    if (rc) return rc;
+    if ((rc = lookahead(p, env, query_env, epsilon, s, tail))) return rc;
     if (tail) s = tail;
     *cur = s;
     if (fork) CN_CUDA_CHECK(cudaStreamWaitEvent(s, env->ev_join, 0));
@@ -918,7 +894,7 @@ int cn_rollout_episodes(cn_policy *p, cn_env *env, cn_world *world, int robot_mo
             else rc = cn_launch_orca(env, s);
             if (rc) return rc;
             if (robot_mode == CN_ROBOT_POLICY)
-                rc = p->cfg.precision == CN_PREC_F16_TC ? cn_lookahead_tc(p, env, query_env, epsilon, s) : cn_lookahead_f32(p, env, query_env, epsilon, s);
+                rc = lookahead(p, env, query_env, epsilon, s);
             else if (robot_mode == CN_ROBOT_ORCA) rc = cn_launch_robot_orca(env, safety_space, s);
             if (rc) return rc;
             if ((rc = cn_launch_step(env, nullptr, 1, s, 0))) return rc;
@@ -971,11 +947,7 @@ int cn_rollout_step_host(cn_policy *p, cn_env *env, int query_env, double epsilo
     if (done) CN_CUDA_CHECK(cudaMemcpyAsync(done, env->done, E, cudaMemcpyDeviceToHost, s));
     if (info) CN_CUDA_CHECK(cudaMemcpyAsync(info, env->info, E, cudaMemcpyDeviceToHost, s));
     if (action_idx) CN_CUDA_CHECK(cudaMemcpyAsync(action_idx, env->action_idx, sizeof(int32_t) * E, cudaMemcpyDeviceToHost, s));
-    int32_t bad = 0;
-    CN_CUDA_CHECK(cudaMemcpyAsync(&bad, p->bad_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    CN_CUDA_CHECK(cudaStreamSynchronize(s));
-    if (bad) { cn_set_error("Value network is not well trained. "); return CN_EVALUE; }   // multi_human_rl.py:57-58
-    return CN_OK;
+    return sync_and_check_values(p, s);
 }
 
 int64_t cn_host_step_bytes(const cn_env *env, int out)
@@ -1016,13 +988,7 @@ static int rollout_step_host_packed(cn_policy *p, cn_env *env, int query_env, do
         CN_CUDA_CHECK(cudaStreamWaitEvent(s0, env->ev_tail, 0));
         s = s0;
     }
-    if (sync) {
-        int32_t bad = 0;
-        CN_CUDA_CHECK(cudaMemcpyAsync(&bad, p->bad_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        CN_CUDA_CHECK(cudaStreamSynchronize(s));
-        if (bad) { cn_set_error("Value network is not well trained. "); return CN_EVALUE; }   // multi_human_rl.py:57-58
-    }
-    return CN_OK;
+    return sync ? sync_and_check_values(p, s) : CN_OK;
 }
 
 int cn_rollout_step_host_packed(cn_policy *p, cn_env *env, int query_env, double epsilon, const void *host_in, void *host_out,

@@ -2,6 +2,8 @@
 #pragma once
 #include <atomic>
 #include <stdlib.h>
+#include <utility>
+#include <vector>
 
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -157,11 +159,23 @@ struct SarlWeightsDev {
     LinearDev lm1[4], lih, lhh;      // LSTM-RL: mlp1 (ValueNetwork2), weight_ih / bias_ih, weight_hh / bias_hh as [in][4h]
 };
 
+// One layer of a value network's state dict: a Linear (weight [out][in], then bias [out]) whose device copy is *dst, or
+// (dst_hh != nullptr) LSTM-RL's LSTM block: weight_ih_l0 [out][in], weight_hh_l0 [out][out / 4], bias_ih_l0, bias_hh_l0 with
+// out = 4 * hidden, device copies *dst (weight_ih / bias_ih) and *dst_hh (weight_hh / bias_hh).
+struct LayerSpec {
+    int in, out;
+    LinearDev *dst, *dst_hh;
+};
+std::vector<LayerSpec> cn_layers(const SarlDims &d, SarlWeightsDev &w);   // state-dict order of d.net (capi.cu)
+inline size_t cn_layer_floats(const LayerSpec &l)
+{
+    return (size_t)l.in * l.out + l.out + (l.dst_hh ? (size_t)(l.out / 4) * l.out + l.out : 0);
+}
+
 struct cn_policy {
     int device;
     cn_sarl_cfg cfg;
     SarlDims d;
-    double gamma_bar;          // pow(gamma, time_step * v_pref), set per lookahead from the env
     double action_host[CN_MAX_ACTIONS * 2];
     double *action_dev;        // A x 2
     float *w_raw;              // flat state-dict order copy (device)
@@ -173,7 +187,7 @@ struct cn_policy {
     double *values;            // E x A
     int32_t *bad_flag;         // [0]: some env of the LAST lookahead had no finite value (cleared per lookahead); [1]: sticky count
                                // of such envs since the handle was created / cn_policy_bad_count(reset)
-    int values_E;
+    size_t values_cap;         // envs `values` has room for
     // tcgen05 path (lookahead_tc.cu)
     void *tc;                  // opaque, owned by the TC module
 };
@@ -212,6 +226,36 @@ void cn_trace_mark(const char *name, cudaStream_t s);
             return CN_ECUDA;                                                                    \
         }                                                                                       \
     } while (0)
+
+// Kernel launch with an optional programmatic dependent launch (pdl): the grid may become resident while the previous
+// kernel on s is still running, so the kernel must griddepcontrol.wait before it reads that kernel's output.
+template <typename... KArgs, typename... Args>
+int cn_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool pdl, Args &&...args)
+{
+    cudaLaunchConfig_t lc = {};
+    lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = smem; lc.stream = s;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    lc.attrs = at; lc.numAttrs = pdl ? 1 : 0;
+    CN_CUDA_CHECK(cudaLaunchKernelEx(&lc, kern, std::forward<Args>(args)...));
+    CN_LAUNCH_CHECK();
+    return CN_OK;
+}
+
+// Grow-on-demand scratch buffer: makes buf hold at least n items of item_bytes each.  A buffer that grows loses its contents;
+// zero = true clears the new one on stream s.
+template <typename T>
+int cn_grow(T *&buf, size_t &cap, size_t n, size_t item_bytes, bool zero = false, cudaStream_t s = 0)
+{
+    if (n <= cap) return CN_OK;
+    if (buf) cudaFree(buf);
+    buf = nullptr; cap = 0;
+    CN_CUDA_CHECK(cudaMalloc((void **)&buf, n * item_bytes));
+    if (zero) CN_CUDA_CHECK(cudaMemsetAsync(buf, 0, n * item_bytes, s));
+    cap = n;
+    return CN_OK;
+}
 
 // ---- Philox4x32-10 (counter-based RNG; Salmon et al. 2011) ------------------------------------
 struct Philox {
@@ -284,7 +328,6 @@ int cn_launch_step(cn_env *env, const double *action_xy_dev, int update, cudaStr
 int cn_launch_reset(cn_env *env, int only_done, cudaStream_t s);
 int cn_launch_pack(cn_env *env, int to_soa, cudaStream_t s);  // stage (AoS) <-> state (SoA)
 int cn_launch_io(cn_env *env, double *blk, int unpack, cudaStream_t s);   // packed host exchange block <-> device state
-int cn_launch_stats_reduce(cn_env *env, cn_stats *out_dev_as_host, int reset, cudaStream_t s);
 
 int cn_lookahead_f32(cn_policy *p, cn_env *env, int query_env, double epsilon, cudaStream_t s);
 int cn_transform_f32(cn_policy *p, cn_env *env, float *out_dev, int sort_humans, cudaStream_t s);
@@ -294,5 +337,6 @@ int cn_f32_configure_device(void);   // per-device kernel attributes (call after
 int cn_tc_init(cn_policy *p);
 void cn_tc_destroy(cn_policy *p);
 int cn_tc_load_weights(cn_policy *p, const float *flat_host, cudaStream_t s);
-// tail != nullptr: the kernels after the row kernel (mlp3, argmax) go to `tail`, ordered after `s` by env->ev_rows
+// tail != nullptr: the scoring stage (mlp3, or CADRL's minimum over the humans) and the argmax of every network go to `tail`,
+// ordered after `s` by env->ev_rows
 int cn_lookahead_tc(cn_policy *p, cn_env *env, int query_env, double epsilon, cudaStream_t s, cudaStream_t tail = nullptr);

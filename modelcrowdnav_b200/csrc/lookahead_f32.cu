@@ -523,30 +523,11 @@ F32Plan make_plan(const SarlDims &d, int H, int A, int A1)
 
 }  // namespace
 
-static int ensure_values(cn_policy *p, int E)
-{
-    if (p->values && p->values_E >= E) return CN_OK;
-    if (p->values) cudaFree(p->values);
-    p->values = nullptr;
-    CN_CUDA_CHECK(cudaMalloc(&p->values, sizeof(double) * (size_t)E * p->d.A));
-    p->values_E = E;
-    return CN_OK;
-}
-
 int cn_lookahead_argmax(cn_policy *p, cn_env *env, double epsilon, cudaStream_t s, bool pdl)
 {
-    const int E = env->p.d.E;
-    cudaLaunchConfig_t lc = {};
-    lc.gridDim = dim3((E + 3) / 4); lc.blockDim = dim3(128); lc.dynamicSmemBytes = 0; lc.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = at; lc.numAttrs = pdl ? 1 : 0;           // pipelined shards (several handles sharing the SMs): plain launches
-    CN_CUDA_CHECK(cudaLaunchKernelEx(&lc, argmax_kernel, env->p, (int)p->d.A, (const double *)env->state, (const uint8_t *)env->frozen,
-                                     (const double *)p->values, (const double *)p->action_dev, epsilon, env->step_ctr, env->action_xy,
-                                     env->action_idx, p->bad_flag));
-    CN_LAUNCH_CHECK();
-    return CN_OK;
+    // pdl = false for pipelined shards (several handles sharing the SMs): plain launches
+    return cn_launch(argmax_kernel, (env->p.d.E + 3) / 4, 128, 0, s, pdl, env->p, p->d.A, env->state, env->frozen, p->values,
+                     p->action_dev, epsilon, env->step_ctr, env->action_xy, env->action_idx, p->bad_flag);
 }
 
 // cudaFuncSetAttribute applies to the CURRENT device only: called from cn_policy_create after cudaSetDevice, so that every
@@ -561,7 +542,7 @@ int cn_f32_configure_device(void)
 
 int cn_lookahead_prepare(cn_policy *p, cn_env *env, cudaStream_t s)
 {
-    int rc = ensure_values(p, env->p.d.E);
+    int rc = cn_grow(p->values, p->values_cap, env->p.d.E, sizeof(double) * p->d.A);
     if (rc) return rc;
     CN_CUDA_CHECK(cudaMemsetAsync(p->bad_flag, 0, sizeof(int32_t), s));
     return CN_OK;

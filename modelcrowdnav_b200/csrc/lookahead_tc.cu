@@ -52,28 +52,25 @@ constexpr uint32_t OFF_W3 = OFF_W2 + bytes_of(N_M1, N_H1);
 constexpr uint32_t OFF_W4 = OFF_W3 + bytes_of(N_M1, N_M1);
 constexpr uint32_t OFF_WA1 = OFF_W4 + bytes_of(N_F, N_M1);
 constexpr uint32_t OFF_WA2 = OFF_WA1 + bytes_of(N_M1, K_A1);
-constexpr uint32_t OFF_TAILA = OFF_WA2 + bytes_of(N_M1, N_M1);   // fp32: attention.4 weight[100], bias
-constexpr uint32_t TAIL_BYTES = 416;
-constexpr uint32_t IMG_A_BYTES = OFF_TAILA + TAIL_BYTES;
+constexpr uint32_t IMG_A_BYTES = OFF_WA2 + bytes_of(N_M1, N_M1);
+constexpr uint32_t TAIL_BYTES = 416;   // fp32 tail of a 100 -> 1 layer: weight[100], bias, 3 pad
 // full weight image of mlp3
 constexpr uint32_t OFF_M1 = 0;
 constexpr uint32_t OFF_M2 = OFF_M1 + bytes_of(N_H1, K_J);
 constexpr uint32_t OFF_M3 = OFF_M2 + bytes_of(N_M1, N_H1);
-constexpr uint32_t OFF_TAILB = OFF_M3 + bytes_of(N_M1, N_M1);    // fp32: mlp3.6 weight[100], bias
-constexpr uint32_t IMG_B_BYTES = OFF_TAILB + TAIL_BYTES;
+constexpr uint32_t IMG_B_BYTES = OFF_M3 + bytes_of(N_M1, N_M1);
 
 constexpr uint32_t J_TILE_BYTES = bytes_of(ROWS, K_J);
 
-
-struct TailW;
 struct TcState {
     uint8_t *img_pair;        // two half images of the row network for tc_rows_pair_kernel (rank 0 | rank 1)
     long long *dbg;           // optional phase timestamps of CTA 0 (cn_debug_tc_timing)
     uint8_t *X;               // layer-1 operand tiles of the CTA-pair path (tc_features_kernel -> tc_rows_pair_kernel)
     size_t cap_xtiles;
-    uint8_t *J;               // joint-state tiles
+    uint8_t *J;               // joint-state tiles, zero-initialised (the mlp3 kernel reads whole rounds of tiles)
+    size_t cap_jtiles;
     double *rew;              // NG rewards
-    size_t cap_groups;
+    size_t cap_rew;
     int num_sms;
     float tail_a[104];        // attention.4 weight[100] + bias (kernel parameter of tc_rows_pair_kernel)
     float tail_b[104];        // mlp3.6 weight[100] + bias (kernel parameter of tc_mlp3_pair_kernel)
@@ -88,7 +85,7 @@ struct TcState {
     float *omP;               // with_om: mlp1.0's occupancy-map product per (env, human), N_H1 floats each (tc_om_bias_kernel)
     size_t cap_om;
     int ktime_on;             // cn_debug_kernel_ms: CUDA events around each kernel of the lookahead, on the launching stream
-    cudaEvent_t kev[5];       // before features | before rows | before mlp3 | before argmax | after argmax
+    cudaEvent_t kev[5];       // before features | before the middle stage | before scoring | before argmax | after argmax
 };
 
 __device__ __forceinline__ void copy_image_to_smem(uint8_t *dst, const uint8_t *__restrict__ src, uint32_t bytes)
@@ -219,6 +216,130 @@ void split_rows(uint8_t *dst, const uint8_t *src, int N, int K, int rank)
         memcpy(dst + (size_t)c * hn * 16, src + (size_t)c * N * 16 + (size_t)rank * hn * 16, (size_t)hn * 16);
 }
 
+// fp32 tail of a 100 -> 1 output layer (kernel parameter TailW): weight[100], bias at [100]
+void fill_tail(const HostLinear &L, float *tail)
+{
+    memset(tail, 0, TAIL_BYTES);
+    for (int k = 0; k < 100; ++k) tail[k] = L.w[k];
+    tail[100] = L.b[0];
+}
+
+// The row network (mlp1, mlp2, attention: L[0..6]) as the two half images of tc_rows_pair_kernel (CTA `rank` holds output
+// rows [rank N/2, (rank+1) N/2) of every layer); attention.4 goes to `tail`.
+std::vector<uint8_t> rows_image(const HostLinear *L, float *tail)
+{
+    std::vector<uint8_t> a(IMG_A_BYTES, 0);
+    // mlp1.0: K = [x_hi(13) 1 1 0 | x_lo(13) 0 0 0]; bias at k = 13,14; ones -> n = 150,151
+    fill_layer(a, OFF_W1, N_H1, L[0], 0, 13, 0, 13, 150);
+    fill_layer(a, OFF_W1, N_H1, L[0], 0, 13, 16, -1, -1);
+    fill_layer(a, OFF_W2, N_M1, L[1], 0, 150, 0, 150, 100);          // mlp1.2
+    fill_layer(a, OFF_W3, N_M1, L[2], 0, 100, 0, 100, 100);          // mlp2.0
+    fill_layer(a, OFF_W4, N_F, L[3], 0, 100, 0, 100, -1);            // mlp2.2 (no ones needed downstream)
+    fill_layer(a, OFF_WA1, N_M1, L[4], 0, 100, 0, 100, 100);         // attention.0, mlp1_out half
+    fill_layer(a, OFF_WA1, N_M1, L[4], 100, 100, N_M1, -1, -1);      //              group-mean half
+    fill_layer(a, OFF_WA2, N_M1, L[5], 0, 100, 0, 100, -1);          // attention.2
+    fill_tail(L[6], tail);
+    std::vector<uint8_t> hp(2 * IMG_H_BYTES, 0);
+    for (int rank = 0; rank < 2; ++rank) {
+        uint8_t *h = hp.data() + (size_t)rank * IMG_H_BYTES;
+        split_rows(h + H_W1, a.data() + OFF_W1, N_H1, K_X, rank);
+        split_rows(h + H_W2, a.data() + OFF_W2, N_M1, N_H1, rank);
+        // stage 2 is ONE N = 224 UMMA: rank 0's half = attention.0 (mlp1_out half of K) -> D [0,112), rank 1's = mlp2.0 -> [112,224)
+        memcpy(h + H_W3A, rank == 0 ? a.data() + OFF_WA1 : a.data() + OFF_W3, bytes_of(N_M1, N_M1));
+        split_rows(h + H_WB, a.data() + OFF_WA1 + bytes_of(N_M1, N_M1), N_M1, N_M1, rank);   // group-mean half of K
+        split_rows(h + H_W4, a.data() + OFF_W4, N_F, N_M1, rank);
+        split_rows(h + H_WA2, a.data() + OFF_WA2, N_M1, N_M1, rank);
+        memcpy(h + H_TAIL, tail, TAIL_BYTES);      // copied to shared memory by the kernel, which reads the TailW parameter
+    }
+    return hp;
+}
+
+// A 150, 100, 100, 1 mlp (M[0..3]) as the two half images of tc_mlp3_pair_kernel; the last layer goes to `tail`.  Stage 0 reads
+// the X tiles (x_input: CADRL's value network on every row) or the joint-state tiles J (SARL's mlp3, LSTM-RL's mlp).
+std::vector<uint8_t> mlp3_image(const HostLinear *M, bool x_input, float *tail)
+{
+    std::vector<uint8_t> b(IMG_B_BYTES, 0);
+    if (x_input) {
+        // X = [x_hi(13) 1 1 0 | x_lo(13) 0 0 0]: bias at k = 13, 14; ones -> n = 150, 151
+        fill_layer(b, OFF_M1, N_H1, M[0], 0, 13, 0, 13, 150);
+        fill_layer(b, OFF_M1, N_H1, M[0], 0, 13, 16, -1, -1);
+    } else {
+        // J = [weighted or h_n(50) pad6 | self_hi(6) 1 1 | self_lo(6) 0 0 | pad8]; torch input = [self(6), weighted or h_n(50)]
+        fill_layer(b, OFF_M1, N_H1, M[0], 6, 50, 0, -1, -1);
+        fill_layer(b, OFF_M1, N_H1, M[0], 0, 6, 56, 62, 150);
+        fill_layer(b, OFF_M1, N_H1, M[0], 0, 6, 64, -1, -1);
+    }
+    fill_layer(b, OFF_M2, N_M1, M[1], 0, 150, 0, 150, 100);
+    fill_layer(b, OFF_M3, N_M1, M[2], 0, 100, 0, 100, -1);
+    fill_tail(M[3], tail);
+    std::vector<uint8_t> hb(2 * IMG_HM_BYTES, 0);
+    for (int rank = 0; rank < 2; ++rank) {
+        uint8_t *h = hb.data() + (size_t)rank * IMG_HM_BYTES;
+        split_rows(h + HM_M1, b.data() + OFF_M1, N_H1, K_J, rank);
+        split_rows(h + HM_M2, b.data() + OFF_M2, N_M1, N_H1, rank);
+        split_rows(h + HM_M3, b.data() + OFF_M3, N_M1, N_M1, rank);
+    }
+    return hb;
+}
+
+// LSTM-RL's LSTM block (lstm_rl.py:9-16: weight_ih_l0 [200][13], weight_hh_l0 [200][50], bias_ih_l0, bias_hh_l0 from src) as
+// the two half images [W_ih | W_hh] of tc_lstm_pair_kernel
+std::vector<uint8_t> lstm_image(const float *src)
+{
+    const int G4 = 4 * L_HIDDEN;
+    const float *w_ih = src, *w_hh = w_ih + (size_t)G4 * 13, *b_ih = w_hh + (size_t)G4 * L_HIDDEN, *b_hh = b_ih + G4;
+    // gate column n of the pair = half * 128 + gate * 32 + cl  <-  torch row gate * 50 + cell, cell = cl (half 0, cl < 24)
+    // or 24 + cl (half 1, cl < 26); the other columns keep zero weights and bias (their cells stay at c = h = 0)
+    std::vector<float> wi((size_t)N_LG * 13, 0.0f), wh((size_t)N_LG * L_HIDDEN, 0.0f), bb(N_LG, 0.0f);
+    for (int n = 0; n < N_LG; ++n) {
+        const int half = n / 128, gate = (n % 128) / 32, cl = n % 32;
+        const int ncell = half ? L_HIDDEN - L_CELLS0 : L_CELLS0;
+        if (cl >= ncell) continue;
+        const int r = gate * L_HIDDEN + (half ? L_CELLS0 + cl : cl);
+        memcpy(&wi[(size_t)n * 13], w_ih + (size_t)r * 13, sizeof(float) * 13);
+        memcpy(&wh[(size_t)n * L_HIDDEN], w_hh + (size_t)r * L_HIDDEN, sizeof(float) * L_HIDDEN);
+        bb[n] = b_ih[r] + b_hh[r];
+    }
+    const HostLinear Li = {wi.data(), bb.data(), 13, N_LG}, Lh = {wh.data(), bb.data(), L_HIDDEN, N_LG};
+    std::vector<uint8_t> li(bytes_of(N_LG, K_X), 0), lh(bytes_of(N_LG, K_LH), 0);
+    // X_t = [x_hi(13) 1 1 0 | x_lo(13) 0 0 0]: bias (b_ih + b_hh, hi / lo) at k = 13, 14
+    fill_layer(li, 0, N_LG, Li, 0, 13, 0, 13, -1);
+    fill_layer(li, 0, N_LG, Li, 0, 13, 16, -1, -1);
+    // h = [h_hi(50) pad6 | h_lo(50) pad6]
+    fill_layer(lh, 0, N_LG, Lh, 0, L_HIDDEN, 0, -1, -1);
+    fill_layer(lh, 0, N_LG, Lh, 0, L_HIDDEN, 56, -1, -1);
+    std::vector<uint8_t> hl(2 * IMG_HL_BYTES, 0);
+    for (int rank = 0; rank < 2; ++rank) {
+        uint8_t *h = hl.data() + (size_t)rank * IMG_HL_BYTES;
+        split_rows(h + HL_WIH, li.data(), N_LG, K_X, rank);
+        split_rows(h + HL_WHH, lh.data(), N_LG, K_LH, rank);
+    }
+    return hl;
+}
+
+// CTA-pair grid over ntiles tiles: every (cluster, rank, context) slot runs the same number of rounds; tiles past the end
+// (up to `tiles`) are all padding
+struct PairGrid {
+    int clusters, rounds;
+    size_t tiles;
+};
+PairGrid pair_grid(int num_sms, int ntiles)
+{
+    int clusters = num_sms / 2;
+    const int slots_needed = (ntiles + 3) / 4;
+    if (clusters > slots_needed) clusters = slots_needed;
+    const int rounds = (ntiles + 4 * clusters - 1) / (4 * clusters);
+    return {clusters, rounds, (size_t)rounds * 4 * clusters};
+}
+
+// developer timeline mark (nullptr: none) and, with cn_debug_kernel_ms on, the timing event kev[i], on stream s
+int stamp(TcState *t, int i, const char *name, cudaStream_t s)
+{
+    if (name) cn_trace_mark(name, s);
+    if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[i], s));
+    return CN_OK;
+}
+
 }  // namespace
 
 // with_om: P[e][h][n] = sum_k W_mlp1.0[n][13 + k] * om[e][h][k]  (fp32), om = the occupancy map of human h built from the
@@ -315,6 +436,7 @@ int cn_tc_init(cn_policy *p)
     }
     TcState *t = new TcState();
     memset(t, 0, sizeof(*t));
+    p->tc = t;                 // from here on a failure leaves everything allocated to cn_policy_destroy
     cudaDeviceProp prop;
     CN_CUDA_CHECK(cudaGetDeviceProperties(&prop, p->device));
     t->num_sms = prop.multiProcessorCount;
@@ -333,7 +455,6 @@ int cn_tc_init(cn_policy *p)
         cn_set_error("cudaMalloc failed for the tensor-core weight images");
         return CN_ENOMEM;
     }
-    p->tc = t;
     return CN_OK;
 }
 
@@ -361,159 +482,32 @@ int cn_tc_load_weights(cn_policy *p, const float *flat, cudaStream_t s)
 {
     TcState *t = (TcState *)p->tc;
     const SarlDims &d = p->d;
-    if (d.net == CN_NET_CADRL) {
-        // value_network.{0,2,4,6} (cadrl.py:22-26) as the three UMMA stages + the fp32 tail of tc_mlp3_pair_kernel<1>
-        HostLinear C[4];
-        const int ins[4] = {d.in, d.m3[0], d.m3[1], d.m3[2]};
-        const float *src = flat;
-        for (int i = 0; i < 4; ++i) {
-            C[i].w = src; src += (size_t)ins[i] * d.m3[i];
-            C[i].b = src; src += d.m3[i];
-            C[i].in = ins[i]; C[i].out = d.m3[i];
-        }
-        std::vector<uint8_t> b(IMG_B_BYTES, 0);
-        // layer 0 on X = [x_hi(13) 1 1 0 | x_lo(13) 0 0 0]: bias at k = 13, 14; ones -> n = 150, 151
-        fill_layer(b, OFF_M1, N_H1, C[0], 0, 13, 0, 13, 150);
-        fill_layer(b, OFF_M1, N_H1, C[0], 0, 13, 16, -1, -1);
-        fill_layer(b, OFF_M2, N_M1, C[1], 0, 150, 0, 150, 100);
-        fill_layer(b, OFF_M3, N_M1, C[2], 0, 100, 0, 100, -1);
-        float tail[TAIL_BYTES / 4] = {0};
-        for (int k = 0; k < 100; ++k) tail[k] = C[3].w[k];
-        tail[100] = C[3].b[0];
-        memcpy(t->tail_b, tail, sizeof(t->tail_b));
-        std::vector<uint8_t> hb(2 * IMG_HM_BYTES, 0);
-        for (int rank = 0; rank < 2; ++rank) {
-            uint8_t *h = hb.data() + (size_t)rank * IMG_HM_BYTES;
-            split_rows(h + HM_M1, b.data() + OFF_M1, N_H1, K_J, rank);
-            split_rows(h + HM_M2, b.data() + OFF_M2, N_M1, N_H1, rank);
-            split_rows(h + HM_M3, b.data() + OFF_M3, N_M1, N_M1, rank);
-        }
-        CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair_b, hb.data(), 2 * IMG_HM_BYTES, cudaMemcpyHostToDevice, s));
-        CN_CUDA_CHECK(cudaStreamSynchronize(s));
-        return CN_OK;
+    std::vector<HostLinear> L;           // the Linear layers in state-dict order
+    const float *lstm = nullptr, *src = flat;
+    for (const LayerSpec &l : cn_layers(d, p->w)) {
+        if (l.dst_hh) lstm = src;
+        else L.push_back({src, src + (size_t)l.in * l.out, l.in, l.out});
+        src += cn_layer_floats(l);
     }
-    if (d.net == CN_NET_LSTM_RL) {
-        // state-dict order (lstm_rl.py:9-16): mlp.{0,2,4,6}, lstm.weight_ih_l0 [200][13], weight_hh_l0 [200][50], bias_ih_l0, bias_hh_l0
-        HostLinear M[4];
-        const int ins[4] = {d.self_dim + d.lstm_h, d.m3[0], d.m3[1], d.m3[2]};
-        const float *src = flat;
-        for (int i = 0; i < 4; ++i) {
-            M[i].w = src; src += (size_t)ins[i] * d.m3[i];
-            M[i].b = src; src += d.m3[i];
-            M[i].in = ins[i]; M[i].out = d.m3[i];
-        }
-        const int G4 = 4 * L_HIDDEN;
-        const float *w_ih = src, *w_hh = w_ih + (size_t)G4 * 13, *b_ih = w_hh + (size_t)G4 * L_HIDDEN, *b_hh = b_ih + G4;
-        // gate column n of the pair = half * 128 + gate * 32 + cl  <-  torch row gate * 50 + cell, cell = cl (half 0, cl < 24)
-        // or 24 + cl (half 1, cl < 26); the other columns keep zero weights and bias (their cells stay at c = h = 0)
-        std::vector<float> wi((size_t)N_LG * 13, 0.0f), wh((size_t)N_LG * L_HIDDEN, 0.0f), bb(N_LG, 0.0f);
-        for (int n = 0; n < N_LG; ++n) {
-            const int half = n / 128, gate = (n % 128) / 32, cl = n % 32;
-            const int ncell = half ? L_HIDDEN - L_CELLS0 : L_CELLS0;
-            if (cl >= ncell) continue;
-            const int r = gate * L_HIDDEN + (half ? L_CELLS0 + cl : cl);
-            memcpy(&wi[(size_t)n * 13], w_ih + (size_t)r * 13, sizeof(float) * 13);
-            memcpy(&wh[(size_t)n * L_HIDDEN], w_hh + (size_t)r * L_HIDDEN, sizeof(float) * L_HIDDEN);
-            bb[n] = b_ih[r] + b_hh[r];
-        }
-        const HostLinear Li = {wi.data(), bb.data(), 13, N_LG}, Lh = {wh.data(), bb.data(), L_HIDDEN, N_LG};
-        std::vector<uint8_t> li(bytes_of(N_LG, K_X), 0), lh(bytes_of(N_LG, K_LH), 0);
-        // X_t = [x_hi(13) 1 1 0 | x_lo(13) 0 0 0]: bias (b_ih + b_hh, hi / lo) at k = 13, 14
-        fill_layer(li, 0, N_LG, Li, 0, 13, 0, 13, -1);
-        fill_layer(li, 0, N_LG, Li, 0, 13, 16, -1, -1);
-        // h = [h_hi(50) pad6 | h_lo(50) pad6]
-        fill_layer(lh, 0, N_LG, Lh, 0, L_HIDDEN, 0, -1, -1);
-        fill_layer(lh, 0, N_LG, Lh, 0, L_HIDDEN, 56, -1, -1);
-        std::vector<uint8_t> hl(2 * IMG_HL_BYTES, 0);
-        for (int rank = 0; rank < 2; ++rank) {
-            uint8_t *h = hl.data() + (size_t)rank * IMG_HL_BYTES;
-            split_rows(h + HL_WIH, li.data(), N_LG, K_X, rank);
-            split_rows(h + HL_WHH, lh.data(), N_LG, K_LH, rank);
-        }
-        // mlp on J = [h_n(50) pad6 | self_hi(6) 1 1 | self_lo(6) 0 0 | pad8]; torch input = [self(6), h_n(50)] (lstm_rl.py:32-33)
-        std::vector<uint8_t> b(IMG_B_BYTES, 0);
-        fill_layer(b, OFF_M1, N_H1, M[0], 6, 50, 0, -1, -1);
-        fill_layer(b, OFF_M1, N_H1, M[0], 0, 6, 56, 62, 150);
-        fill_layer(b, OFF_M1, N_H1, M[0], 0, 6, 64, -1, -1);
-        fill_layer(b, OFF_M2, N_M1, M[1], 0, 150, 0, 150, 100);
-        fill_layer(b, OFF_M3, N_M1, M[2], 0, 100, 0, 100, -1);
-        float tail[TAIL_BYTES / 4] = {0};
-        for (int k = 0; k < 100; ++k) tail[k] = M[3].w[k];
-        tail[100] = M[3].b[0];
-        memcpy(t->tail_b, tail, sizeof(t->tail_b));
-        std::vector<uint8_t> hb(2 * IMG_HM_BYTES, 0);
-        for (int rank = 0; rank < 2; ++rank) {
-            uint8_t *h = hb.data() + (size_t)rank * IMG_HM_BYTES;
-            split_rows(h + HM_M1, b.data() + OFF_M1, N_H1, K_J, rank);
-            split_rows(h + HM_M2, b.data() + OFF_M2, N_M1, N_H1, rank);
-            split_rows(h + HM_M3, b.data() + OFF_M3, N_M1, N_M1, rank);
-        }
-        CN_CUDA_CHECK(cudaMemcpyAsync(t->img_lstm, hl.data(), 2 * IMG_HL_BYTES, cudaMemcpyHostToDevice, s));
-        CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair_b, hb.data(), 2 * IMG_HM_BYTES, cudaMemcpyHostToDevice, s));
-        CN_CUDA_CHECK(cudaStreamSynchronize(s));
-        return CN_OK;
+    // the last four Linears: SARL's mlp3, CADRL's value_network (cadrl.py:22-26), LSTM-RL's mlp (lstm_rl.py:9-16)
+    const std::vector<uint8_t> hb = mlp3_image(&L[L.size() - 4], d.net == CN_NET_CADRL, t->tail_b);
+    std::vector<uint8_t> hp, hl;
+    CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair_b, hb.data(), hb.size(), cudaMemcpyHostToDevice, s));
+    if (d.net == CN_NET_SARL) {
+        hp = rows_image(L.data(), t->tail_a);
+        CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair, hp.data(), hp.size(), cudaMemcpyHostToDevice, s));
+    } else if (d.net == CN_NET_LSTM_RL) {
+        hl = lstm_image(lstm);
+        CN_CUDA_CHECK(cudaMemcpyAsync(t->img_lstm, hl.data(), hl.size(), cudaMemcpyHostToDevice, s));
     }
-    HostLinear L[11];
-    const int ins[11] = {d.in, d.m1[0], d.m1[1], d.m2[0], 2 * d.m1[1], d.at[0], d.at[1], d.m2[1] + d.self_dim, d.m3[0], d.m3[1], d.m3[2]};
-    const int outs[11] = {d.m1[0], d.m1[1], d.m2[0], d.m2[1], d.at[0], d.at[1], d.at[2], d.m3[0], d.m3[1], d.m3[2], d.m3[3]};
-    const float *src = flat;
-    for (int i = 0; i < 11; ++i) {
-        L[i].w = src; src += (size_t)ins[i] * outs[i];
-        L[i].b = src; src += outs[i];
-        L[i].in = ins[i]; L[i].out = outs[i];
-    }
-    std::vector<uint8_t> a(IMG_A_BYTES, 0), b(IMG_B_BYTES, 0);
-    // mlp1.0: K = [x_hi(13) 1 1 0 | x_lo(13) 0 0 0]; bias at k = 13,14; ones -> n = 150,151
-    fill_layer(a, OFF_W1, N_H1, L[0], 0, 13, 0, 13, 150);
-    fill_layer(a, OFF_W1, N_H1, L[0], 0, 13, 16, -1, -1);
-    fill_layer(a, OFF_W2, N_M1, L[1], 0, 150, 0, 150, 100);          // mlp1.2
-    fill_layer(a, OFF_W3, N_M1, L[2], 0, 100, 0, 100, 100);          // mlp2.0
-    fill_layer(a, OFF_W4, N_F, L[3], 0, 100, 0, 100, -1);            // mlp2.2 (no ones needed downstream)
-    fill_layer(a, OFF_WA1, N_M1, L[4], 0, 100, 0, 100, 100);         // attention.0, mlp1_out half
-    fill_layer(a, OFF_WA1, N_M1, L[4], 100, 100, N_M1, -1, -1);      //              group-mean half
-    fill_layer(a, OFF_WA2, N_M1, L[5], 0, 100, 0, 100, -1);          // attention.2
-    float tail[TAIL_BYTES / 4] = {0};
-    for (int k = 0; k < 100; ++k) tail[k] = L[6].w[k];
-    tail[100] = L[6].b[0];
-    memcpy(&a[OFF_TAILA], tail, TAIL_BYTES);
-    memcpy(t->tail_a, tail, sizeof(t->tail_a));
-    // mlp3.0 on J = [weighted(50) pad6 | self_hi(6) 1 1 | self_lo(6) 0 0 | pad8]; joint = [self(6), weighted(50)]
-    fill_layer(b, OFF_M1, N_H1, L[7], 6, 50, 0, -1, -1);
-    fill_layer(b, OFF_M1, N_H1, L[7], 0, 6, 56, 62, 150);
-    fill_layer(b, OFF_M1, N_H1, L[7], 0, 6, 64, -1, -1);
-    fill_layer(b, OFF_M2, N_M1, L[8], 0, 150, 0, 150, 100);          // mlp3.2
-    fill_layer(b, OFF_M3, N_M1, L[9], 0, 100, 0, 100, -1);           // mlp3.4
-    for (int k = 0; k < 100; ++k) tail[k] = L[10].w[k];
-    tail[100] = L[10].b[0];
-    memcpy(&b[OFF_TAILB], tail, TAIL_BYTES);
-    memcpy(t->tail_b, tail, sizeof(t->tail_b));
-    std::vector<uint8_t> hb(2 * IMG_HM_BYTES, 0);
-    for (int rank = 0; rank < 2; ++rank) {
-        uint8_t *h = hb.data() + (size_t)rank * IMG_HM_BYTES;
-        split_rows(h + HM_M1, b.data() + OFF_M1, N_H1, K_J, rank);
-        split_rows(h + HM_M2, b.data() + OFF_M2, N_M1, N_H1, rank);
-        split_rows(h + HM_M3, b.data() + OFF_M3, N_M1, N_M1, rank);
-    }
-    CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair_b, hb.data(), 2 * IMG_HM_BYTES, cudaMemcpyHostToDevice, s));
-    // half images for the CTA-pair kernel: CTA `rank` holds output rows [rank N/2, (rank+1) N/2) of every layer
-    std::vector<uint8_t> hp(2 * IMG_H_BYTES, 0);
-    for (int rank = 0; rank < 2; ++rank) {
-        uint8_t *h = hp.data() + (size_t)rank * IMG_H_BYTES;
-        split_rows(h + H_W1, a.data() + OFF_W1, N_H1, K_X, rank);
-        split_rows(h + H_W2, a.data() + OFF_W2, N_M1, N_H1, rank);
-        // stage 2, N = 224: rank 0 = mlp2.0 (all 112 rows), rank 1 = attention.0 rows on the mlp1_out half of K
-        // stage 2 is ONE N = 224 UMMA: rank 0's half = attention.0 (mlp1_out half of K) -> D [0,112), rank 1's = mlp2.0 -> [112,224)
-        memcpy(h + H_W3A, rank == 0 ? a.data() + OFF_WA1 : a.data() + OFF_W3, bytes_of(N_M1, N_M1));
-        split_rows(h + H_WB, a.data() + OFF_WA1 + bytes_of(N_M1, N_M1), N_M1, N_M1, rank);   // group-mean half of K
-        split_rows(h + H_W4, a.data() + OFF_W4, N_F, N_M1, rank);
-        split_rows(h + H_WA2, a.data() + OFF_WA2, N_M1, N_M1, rank);
-        memcpy(h + H_TAIL, a.data() + OFF_TAILA, TAIL_BYTES);
-    }
-    CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair, hp.data(), 2 * IMG_H_BYTES, cudaMemcpyHostToDevice, s));
     CN_CUDA_CHECK(cudaStreamSynchronize(s));
     return CN_OK;
 }
 
+// One lookahead of every network: feature kernel, the network's middle stage, the hand-over to `tail`, the scoring stage,
+// argmax.  Middle stage: SARL [tc_om_bias_kernel] tc_rows_pair_kernel; CADRL tc_mlp3_pair_kernel<1> (its whole network on
+// the X tiles, one value per row); LSTM-RL lstm_order_kernel, tc_features_lstm_kernel, tc_lstm_pair_kernel.  Scoring stage:
+// tc_mlp3_pair_kernel<0> on the joint-state tiles (SARL, LSTM-RL) or cadrl_min_kernel (CADRL: minimum over each group's humans).
 int cn_lookahead_tc(cn_policy *p, cn_env *env, int query_env, double epsilon, cudaStream_t s, cudaStream_t tail)
 {
     TcState *t = (TcState *)p->tc;
@@ -525,182 +519,83 @@ int cn_lookahead_tc(cn_policy *p, cn_env *env, int query_env, double epsilon, cu
     // (PipelinedHostRollout: tail stream set) a row kernel that becomes resident early and waits keeps another shard's kernels
     // off the SMs (measured: end to end 1.18e7 -> 1.14e7 env-steps/s)
     const bool pipelined = tail && tail != s;
-    const int A = p->d.A;
+    const int net = p->d.net, A = p->d.A;
+    const bool om = p->d.om_dim > 0;
     const size_t NG = (size_t)ed.E * A;
-    if (NG > t->cap_groups) {
-        if (t->J) cudaFree(t->J);
-        if (t->rew) cudaFree(t->rew);
-        t->J = nullptr; t->rew = nullptr; t->cap_groups = 0;
-        // the CTA-pair mlp3 kernel reads whole rounds of tiles: pad with up to one round of (zero) tiles
-        const size_t jtiles = (NG + ROWS - 1) / ROWS + 4 * (size_t)(t->num_sms / 2);
-        CN_CUDA_CHECK(cudaMalloc((void **)&t->J, jtiles * J_TILE_BYTES));
-        CN_CUDA_CHECK(cudaMalloc((void **)&t->rew, sizeof(double) * NG));
-        CN_CUDA_CHECK(cudaMemsetAsync(t->J, 0, jtiles * J_TILE_BYTES, s));
-        t->cap_groups = NG;
-    }
     int G = ROWS / ed.H;
     if (G > 64) G = 64;                      // H = 1: two rows of padding per group keep the group loops within 64 items
-    const int ntiles_a = (int)((NG + G - 1) / G);
-    const int ntiles_b = (int)((NG + ROWS - 1) / ROWS);
+    const PairGrid ga = pair_grid(t->num_sms, (int)((NG + G - 1) / G));       // tiles of (env, action, human) rows
+    const PairGrid gb = pair_grid(t->num_sms, (int)((NG + ROWS - 1) / ROWS));  // tiles of (env, action) rows
+    // the CTA-pair mlp3 kernel reads whole rounds of tiles: pad with up to one round of (zero) tiles
+    if ((rc = cn_grow(t->J, t->cap_jtiles, (NG + ROWS - 1) / ROWS + 4 * (size_t)(t->num_sms / 2), J_TILE_BYTES, true, s))) return rc;
+    if ((rc = cn_grow(t->rew, t->cap_rew, NG, sizeof(double)))) return rc;
+    if ((rc = cn_grow(t->X, t->cap_xtiles, ga.tiles, X_TILE_BYTES))) return rc;
     const double gamma_bar = pow(p->cfg.gamma, env->p.time_step * p->cfg.v_pref);
-    {
-        // CTA pairs: every (cluster, rank, context) slot runs the same number of rounds; tiles past the end are all padding
-        int nclusters = t->num_sms / 2;
-        const int slots_needed = (ntiles_a + 3) / 4;
-        if (nclusters > slots_needed) nclusters = slots_needed;
-        const int rounds = (ntiles_a + 4 * nclusters - 1) / (4 * nclusters);
-        const size_t xtiles = (size_t)rounds * 4 * nclusters;
-        if (xtiles > t->cap_xtiles) {
-            if (t->X) cudaFree(t->X);
-            t->X = nullptr; t->cap_xtiles = 0;
-            CN_CUDA_CHECK(cudaMalloc((void **)&t->X, xtiles * X_TILE_BYTES));
-            t->cap_xtiles = xtiles;
-        }
-        TailW tw;
-        memcpy(tw.w, t->tail_a, sizeof(tw.w));
-        const int ht = (ed.H == 5 && G == ROWS / 5) ? 5 : ((ed.H == 10 && G == ROWS / 10) ? 10 : 0);
-        auto feat = ht == 5 ? tc_features_kernel<5> : (ht == 10 ? tc_features_kernel<10> : tc_features_kernel<0>);
-        const bool om = p->d.om_dim > 0;
-        auto kern = om ? (ht == 5 ? tc_rows_pair_kernel<5, true> : (ht == 10 ? tc_rows_pair_kernel<10, true> : tc_rows_pair_kernel<0, true>))
-                       : (ht == 5 ? tc_rows_pair_kernel<5, false> : (ht == 10 ? tc_rows_pair_kernel<10, false> : tc_rows_pair_kernel<0, false>));
-        cn_trace_mark("features", s);
-        if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[0], s));
-        feat<<<(unsigned)xtiles, ROWS, 0, s>>>(env->p, env->state, env->time, env->human_v, p->action_dev, A, query_env, (int)NG, G,
-                                              env->theta, t->X, t->J, t->rew);
+    TailW twa, twb;
+    memcpy(twa.w, t->tail_a, sizeof(twa.w));
+    memcpy(twb.w, t->tail_b, sizeof(twb.w));
+    const int ht = (ed.H == 5 && G == ROWS / 5) ? 5 : ((ed.H == 10 && G == ROWS / 10) ? 10 : 0);
+    auto feat = ht == 5 ? tc_features_kernel<5> : (ht == 10 ? tc_features_kernel<10> : tc_features_kernel<0>);
+
+    if ((rc = stamp(t, 0, "features", s))) return rc;
+    feat<<<(unsigned)ga.tiles, ROWS, 0, s>>>(env->p, env->state, env->time, env->human_v, p->action_dev, A, query_env, (int)NG, G,
+                                             env->theta, t->X, t->J, t->rew);
+    CN_LAUNCH_CHECK();
+    if ((rc = stamp(t, 1, "rows", s))) return rc;
+    if (net == CN_NET_LSTM_RL) {
+        // one sequence per (env, action) group over the humans in predict()'s order; h_n lands in the joint-state tiles
+        // (the feature kernel above left their self-state chunks and the rewards)
+        if ((rc = cn_grow(t->XL, t->cap_xl, gb.tiles * ed.H, X_TILE_BYTES))) return rc;
+        if ((rc = cn_grow(t->ord, t->cap_ord, (size_t)ed.E * ed.H, sizeof(int32_t)))) return rc;
+        lstm_order_kernel<<<(ed.E + 127) / 128, 128, 0, s>>>(env->p, env->state, query_env, t->ord);
         CN_LAUNCH_CHECK();
-        cn_trace_mark("rows", s);
-        if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[1], s));
-        if (p->d.net == CN_NET_LSTM_RL) {
-            // LSTM-RL: one sequence per (env, action) group over the humans in predict()'s order, then mlp(cat(self, h_n)) on the
-            // joint-state tiles (the feature kernel above left their self-state chunks and the rewards)
-            int ncl = t->num_sms / 2;
-            const int slots_l = (ntiles_b + 3) / 4;
-            if (ncl > slots_l) ncl = slots_l;
-            const int rnds = (ntiles_b + 4 * ncl - 1) / (4 * ncl);
-            const size_t ltiles = (size_t)rnds * 4 * ncl;
-            if (ltiles * ed.H > t->cap_xl) {
-                if (t->XL) cudaFree(t->XL);
-                t->XL = nullptr; t->cap_xl = 0;
-                CN_CUDA_CHECK(cudaMalloc((void **)&t->XL, ltiles * ed.H * X_TILE_BYTES));
-                t->cap_xl = ltiles * ed.H;
-            }
-            if ((size_t)ed.E * ed.H > t->cap_ord) {
-                if (t->ord) cudaFree(t->ord);
-                t->ord = nullptr; t->cap_ord = 0;
-                CN_CUDA_CHECK(cudaMalloc((void **)&t->ord, sizeof(int32_t) * (size_t)ed.E * ed.H));
-                t->cap_ord = (size_t)ed.E * ed.H;
-            }
-            lstm_order_kernel<<<(ed.E + 127) / 128, 128, 0, s>>>(env->p, env->state, query_env, t->ord);
-            CN_LAUNCH_CHECK();
-            tc_features_lstm_kernel<<<(unsigned)(ltiles * ed.H), ROWS, 0, s>>>(env->p, env->state, env->time, env->human_v, p->action_dev,
-                                                                            A, query_env, (int)NG, env->theta, t->ord, t->XL);
-            CN_LAUNCH_CHECK();
-            tc_lstm_pair_kernel<<<2 * ncl, kThreadsL, L_SMEM, s>>>(t->img_lstm, t->XL, t->J, ed.H, rnds);
-            CN_LAUNCH_CHECK();
-            TailW twb;
-            memcpy(twb.w, t->tail_b, sizeof(twb.w));
-            cn_trace_mark("mlp3", s);
-            if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[2], s));
-            tc_mlp3_pair_kernel<0><<<2 * ncl, kThreadsM3, M_SMEM, s>>>(env->p, env->state, t->img_pair_b, t->J, t->rew, A, (int)NG,
-                                                                      p->cfg.gamma, gamma_bar, p->cfg.v_pref, p->values, rnds, twb,
-                                                                      nullptr);
-            CN_LAUNCH_CHECK();
-            cn_trace_mark("argmax", s);
-            if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[3], s));
-            rc = cn_lookahead_argmax(p, env, epsilon, s, !pipelined);
-            if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[4], s));
+        tc_features_lstm_kernel<<<(unsigned)(gb.tiles * ed.H), ROWS, 0, s>>>(env->p, env->state, env->time, env->human_v, p->action_dev,
+                                                                           A, query_env, (int)NG, env->theta, t->ord, t->XL);
+        CN_LAUNCH_CHECK();
+        tc_lstm_pair_kernel<<<2 * gb.clusters, kThreadsL, L_SMEM, s>>>(t->img_lstm, t->XL, t->J, ed.H, gb.rounds);
+        CN_LAUNCH_CHECK();
+    } else if (net == CN_NET_CADRL) {
+        if ((rc = cn_grow(t->rowv, t->cap_rowv, ga.tiles * ROWS, sizeof(float)))) return rc;
+        if ((rc = cn_launch(tc_mlp3_pair_kernel<1>, 2 * ga.clusters, kThreadsM3, M_SMEM, s, false, env->p, env->state, t->img_pair_b,
+                            t->X, t->rew, A, (int)NG, p->cfg.gamma, gamma_bar, p->cfg.v_pref, p->values, ga.rounds, twb, t->rowv)))
             return rc;
-        }
-        if (p->d.net == CN_NET_CADRL) {
-            // CADRL: the whole network runs on the X tiles, one value per row, then the minimum over each group's humans
-            if (xtiles * ROWS > t->cap_rowv) {
-                if (t->rowv) cudaFree(t->rowv);
-                t->rowv = nullptr; t->cap_rowv = 0;
-                CN_CUDA_CHECK(cudaMalloc((void **)&t->rowv, sizeof(float) * xtiles * ROWS));
-                t->cap_rowv = xtiles * ROWS;
-            }
-            TailW twb;
-            memcpy(twb.w, t->tail_b, sizeof(twb.w));
-            tc_mlp3_pair_kernel<1><<<2 * nclusters, kThreadsM3, M_SMEM, s>>>(env->p, env->state, t->img_pair_b, t->X, t->rew, A, (int)NG,
-                                                                            p->cfg.gamma, gamma_bar, p->cfg.v_pref, p->values, rounds,
-                                                                            twb, t->rowv);
-            CN_LAUNCH_CHECK();
-            if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[2], s));
-            cadrl_min_kernel<<<(unsigned)((NG + 255) / 256), 256, 0, s>>>(env->p, env->state, t->rowv, t->rew, A, (int)NG, G, ed.H,
-                                                                          p->cfg.gamma, gamma_bar, p->cfg.v_pref, p->values);
-            CN_LAUNCH_CHECK();
-            cn_trace_mark("argmax", s);
-            if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[3], s));
-            rc = cn_lookahead_argmax(p, env, epsilon, s, !pipelined);
-            if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[4], s));
-            return rc;
-        }
+    } else {
         if (om) {
             // occupancy maps of the NEXT human states (multi_human_rl.py:47-49), folded into one row bias of mlp1.0 per human
             const size_t items = (size_t)ed.E * ed.H;
-            if (items > t->cap_om) {
-                if (t->omP) cudaFree(t->omP);
-                t->omP = nullptr; t->cap_om = 0;
-                CN_CUDA_CHECK(cudaMalloc((void **)&t->omP, sizeof(float) * items * N_H1));
-                t->cap_om = items;
-            }
+            if ((rc = cn_grow(t->omP, t->cap_om, items, sizeof(float) * N_H1))) return rc;
             tc_om_bias_kernel<<<(unsigned)((items + kOmItems - 1) / kOmItems), N_H1, 0, s>>>(env->p, p->d, p->w.m1[0], env->state,
                                                                                           env->human_v, query_env, t->omP);
             CN_LAUNCH_CHECK();
         }
-        if (om || pipelined) {          // om: the bias kernel sits between the feature kernel and this one -> plain launch
-            kern<<<2 * nclusters, kThreadsPair, Q_SMEM, s>>>(env->p, t->img_pair, t->X, t->J, (int)NG, G, rounds, tw, t->dbg, t->omP, A);
-        } else {
-            // programmatic dependent launch: the CTAs' prologue runs under the feature kernel's tail (pdl_wait() in the kernel)
-            cudaLaunchConfig_t lc = {};
-            lc.gridDim = dim3(2 * nclusters); lc.blockDim = dim3(kThreadsPair); lc.dynamicSmemBytes = Q_SMEM; lc.stream = s;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            at[0].val.programmaticStreamSerializationAllowed = 1;
-            lc.attrs = at; lc.numAttrs = 1;
-            CN_CUDA_CHECK(cudaLaunchKernelEx(&lc, kern, env->p, (const uint8_t *)t->img_pair, (const uint8_t *)t->X, t->J, (int)NG, G,
-                                             rounds, tw, t->dbg, (const float *)t->omP, A));
-        }
-        CN_LAUNCH_CHECK();
+        auto rows = om ? (ht == 5 ? tc_rows_pair_kernel<5, true> : (ht == 10 ? tc_rows_pair_kernel<10, true> : tc_rows_pair_kernel<0, true>))
+                       : (ht == 5 ? tc_rows_pair_kernel<5, false> : (ht == 10 ? tc_rows_pair_kernel<10, false> : tc_rows_pair_kernel<0, false>));
+        // PDL: the CTAs' prologue runs under the feature kernel's tail (pdl_wait() in the kernel); with om the bias kernel
+        // sits between the two -> plain launch
+        if ((rc = cn_launch(rows, 2 * ga.clusters, kThreadsPair, Q_SMEM, s, !om && !pipelined, env->p, t->img_pair, t->X, t->J, (int)NG,
+                            G, ga.rounds, twa, t->dbg, t->omP, A)))
+            return rc;
     }
-    if (tail && tail != s) {
-        // pipelined host steps: the rest of this shard's step runs on a HIGH-priority stream, so that when this row kernel
-        // exits its mlp3 is placed before the other shard's (already queued, lower-priority) row kernel takes every SM
+    if (pipelined) {
+        // pipelined host steps: the rest of this shard's step runs on a HIGH-priority stream, so that when the middle stage
+        // exits the scoring kernel is placed before the other shard's (already queued, lower-priority) row kernel takes every SM
         CN_CUDA_CHECK(cudaEventRecord(env->ev_rows, s));
         CN_CUDA_CHECK(cudaStreamWaitEvent(tail, env->ev_rows, 0));
         s = tail;
     }
-    {
-        int nclusters = t->num_sms / 2;
-        const int slots_needed = (ntiles_b + 3) / 4;
-        if (nclusters > slots_needed) nclusters = slots_needed;
-        const int rounds = (ntiles_b + 4 * nclusters - 1) / (4 * nclusters);
-        TailW tw;
-        memcpy(tw.w, t->tail_b, sizeof(tw.w));
-        cn_trace_mark("mlp3", s);
-        if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[2], s));
-        if (tail && tail != s) {       // (already on another stream than the row kernel: plain launch behind the event)
-            tc_mlp3_pair_kernel<0><<<2 * nclusters, kThreadsM3, M_SMEM, s>>>(env->p, env->state, t->img_pair_b, t->J, t->rew, A, (int)NG,
-                                                                            p->cfg.gamma, gamma_bar, p->cfg.v_pref, p->values, rounds, tw,
-                                                                            nullptr);
-        } else {
-            cudaLaunchConfig_t lc = {};
-            lc.gridDim = dim3(2 * nclusters); lc.blockDim = dim3(kThreadsM3); lc.dynamicSmemBytes = M_SMEM; lc.stream = s;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            at[0].val.programmaticStreamSerializationAllowed = 1;
-            lc.attrs = at; lc.numAttrs = 1;
-            CN_CUDA_CHECK(cudaLaunchKernelEx(&lc, tc_mlp3_pair_kernel<0>, env->p, (const double *)env->state, (const uint8_t *)t->img_pair_b,
-                                             (const uint8_t *)t->J, (const double *)t->rew, A, (int)NG, (double)p->cfg.gamma, gamma_bar,
-                                             (double)p->cfg.v_pref, p->values, rounds, tw, (float *)nullptr));
-        }
+    if ((rc = stamp(t, 2, "mlp3", s))) return rc;
+    if (net == CN_NET_CADRL) {
+        cadrl_min_kernel<<<(unsigned)((NG + 255) / 256), 256, 0, s>>>(env->p, env->state, t->rowv, t->rew, A, (int)NG, G, ed.H,
+                                                                      p->cfg.gamma, gamma_bar, p->cfg.v_pref, p->values);
         CN_LAUNCH_CHECK();
+    } else if ((rc = cn_launch(tc_mlp3_pair_kernel<0>, 2 * gb.clusters, kThreadsM3, M_SMEM, s, net != CN_NET_LSTM_RL, env->p,
+                                 env->state, t->img_pair_b, t->J, t->rew, A, (int)NG, p->cfg.gamma, gamma_bar, p->cfg.v_pref,
+                                 p->values, gb.rounds, twb, nullptr))) {
+        return rc;
     }
-    cn_trace_mark("argmax", s);
-    if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[3], s));
-    rc = cn_lookahead_argmax(p, env, epsilon, s, !pipelined);
-    if (t->ktime_on) CN_CUDA_CHECK(cudaEventRecord(t->kev[4], s));
-    return rc;
+    if ((rc = stamp(t, 3, "argmax", s))) return rc;
+    if ((rc = cn_lookahead_argmax(p, env, epsilon, s, !pipelined))) return rc;
+    return stamp(t, 4, nullptr, s);
 }
 
 static int selftest_impl(int32_t N, int32_t K, const float *a_host, const float *b_host, float *d_host, int device, int mode)

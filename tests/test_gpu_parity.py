@@ -526,17 +526,25 @@ def test_packed_host_step_matches_device_step(mcn, oracle_mod, weights0):
     env_a.close(); env_b.close(); pol.close()
 
 
-@pytest.mark.parametrize("shards,graphs", [(2, False), (4, True), (2, True)])
-def test_pipelined_host_rollout_matches_device_step(mcn, oracle_mod, weights0, shards, graphs):
+@pytest.mark.parametrize("net,shards,graphs", [("sarl", 2, False), ("sarl", 4, True), ("sarl", 2, True), ("cadrl", 2, True),
+                                               ("lstm", 2, True), ("om_sarl", 2, True)])
+def test_pipelined_host_rollout_matches_device_step(mcn, oracle_mod, weights0, units_nets, units_om, net, shards, graphs):
     """PipelinedHostRollout (env shards on their own streams, cn_rollout_step_host_packed_async: the copies of one
     shard overlap the kernels of another) returns bit for bit what the single device-resident handle computes,
-    including the episodes that finish and are re-seeded on the device (global env ids key the Philox streams)."""
+    including the episodes that finish and are re-seeded on the device (global env ids key the Philox streams).
+    Every tensor-core network: each hands its scoring stage and argmax over to the shard's tail stream."""
     E, H = 256, 5
+    if net == "sarl":
+        cfg, w = {}, weights0
+    elif net == "om_sarl":
+        cfg, w = _om_kw("sarl"), units_om["om_sarl_weights"]
+    else:
+        cfg, w = _net_kw(net), units_nets[net + "_weights"]
     env = mcn.BatchedCrowdSim(E, H, auto_reset=1, seed=3)
-    pol = mcn.BatchedSARL(precision="f16_tc"); pol.load_weights(weights0)
+    pol = mcn.BatchedSARL(precision="f16_tc", **cfg); pol.load_weights(w)
     env.reset_device()
     a0, t0 = env.get_state()
-    pipe = mcn.PipelinedHostRollout(E, H, weights0, shards=shards, precision="f16_tc", auto_reset=1, seed=3,
+    pipe = mcn.PipelinedHostRollout(E, H, w, shards=shards, precision="f16_tc", auto_reset=1, seed=3, policy_cfg=cfg,
                                     use_graphs=graphs)                    # graphs: one captured launch per shard and step
     pipe.reset_device()
     b = [x for x in pipe.bufs]
@@ -555,7 +563,7 @@ def test_pipelined_host_rollout_matches_device_step(mcn, oracle_mod, weights0, s
     assert sum(e.stats()["episodes"] for e in pipe.envs) == st["episodes"]
     pipe.close()
     # the device-resident form of the same sharding (cn_rollout_step_sharded: no copies, no host sync between steps)
-    dev = mcn.PipelinedHostRollout(E, H, weights0, shards=shards, precision="f16_tc", auto_reset=1, seed=3)
+    dev = mcn.PipelinedHostRollout(E, H, w, shards=shards, precision="f16_tc", auto_reset=1, seed=3, policy_cfg=cfg)
     dev.reset_device()
     for step in range(110):
         dev.step_device()
@@ -607,15 +615,17 @@ def test_golden_trajectories_kinematics(mcn, weights0, name, precision):
     env.close(); pol.close()
 
 
-def _net_policy(mcn, tag, **kw):
-    """BatchedSARL configured as the reference's CADRL / LSTM-RL ([cadrl], [lstm_rl] of policy.config)."""
-    kw = {k: v for k, v in kw.items() if v is not None}
-    precision = kw.pop("precision", "f32")
+def _net_kw(tag):
+    """BatchedSARL arguments of the reference's CADRL / LSTM-RL ([cadrl], [lstm_rl] of policy.config)."""
     if tag == "cadrl":
-        return mcn.BatchedSARL(precision=precision, network="cadrl", mlp3_dims=[150, 100, 100, 1], **kw)
+        return dict(network="cadrl", mlp3_dims=[150, 100, 100, 1])
     m1 = [150, 100, 100, 50] if tag == "lstm2" else [0, 0, 0, 0]
-    return mcn.BatchedSARL(precision=precision, network="lstm_rl", mlp3_dims=[150, 100, 100, 1], lstm_hidden=50,
-                           lstm_mlp1_dims=m1, **kw)
+    return dict(network="lstm_rl", mlp3_dims=[150, 100, 100, 1], lstm_hidden=50, lstm_mlp1_dims=m1)
+
+
+def _net_policy(mcn, tag, **kw):
+    kw = {k: v for k, v in kw.items() if v is not None}
+    return mcn.BatchedSARL(precision=kw.pop("precision", "f32"), **_net_kw(tag), **kw)
 
 
 @pytest.mark.parametrize("tag", ["cadrl", "lstm", "lstm2"])
@@ -714,11 +724,15 @@ def test_lstm_last_state_is_sorted(mcn, oracle_mod, units_nets):
     env.close(); pol.close()
 
 
-def _om_policy(mcn, policy, precision="f32"):
-    kw = dict(precision=precision, input_dim=61, with_om=1, cell_num=4, cell_size=1.0, om_channel_size=3)
+def _om_kw(policy):
+    kw = dict(input_dim=61, with_om=1, cell_num=4, cell_size=1.0, om_channel_size=3)
     if policy == "sarl":
-        return mcn.BatchedSARL(**kw)
-    return mcn.BatchedSARL(network="lstm_rl", mlp3_dims=[150, 100, 100, 1], lstm_hidden=50, **kw)
+        return kw
+    return dict(network="lstm_rl", mlp3_dims=[150, 100, 100, 1], lstm_hidden=50, **kw)
+
+
+def _om_policy(mcn, policy, precision="f32"):
+    return mcn.BatchedSARL(precision=precision, **_om_kw(policy))
 
 
 @pytest.mark.parametrize("H", [2, 5, 10])
