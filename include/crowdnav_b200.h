@@ -117,6 +117,10 @@ typedef struct {
     int32_t cell_num;            /* [om] cell_num = 4 (<= 8) */
     double cell_size;            /* [om] cell_size = 1 */
     int32_t om_channel_size;     /* [om] om_channel_size = 3 (1, 2 or 3) */
+    /* [sarl] with_global_state = false: attention.0 reads mlp1_out only (sarl.py:40-47), so its weight is
+     * [attn_dims[0]][mlp1_dims[1]] instead of [attn_dims[0]][2 * mlp1_dims[1]]; 0 = the reference default.  SARL only (with or
+     * without occupancy maps, both precisions); CN_EINVAL for CADRL and LSTM-RL. */
+    int32_t without_global_state;
 } cn_sarl_cfg;
 
 /* Episode statistics accumulated on the device by cn_env_step(update=1); the counters
@@ -218,7 +222,9 @@ int cn_policy_create(const cn_sarl_cfg *cfg, int device, cn_policy **out);
 int cn_policy_destroy(cn_policy *p);
 int64_t cn_policy_param_count(const cn_sarl_cfg *cfg);
 /* model.load_state_dict (test.py:59): flat fp32 parameters in state-dict order
- * mlp1.{0,2} mlp2.{0,2} attention.{0,2,4} mlp3.{0,2,4,6}, each .weight ([out][in] row-major) then .bias. */
+ * mlp1.{0,2} mlp2.{0,2} attention.{0,2,4} mlp3.{0,2,4,6}, each .weight ([out][in] row-major) then .bias.  attention.0.weight
+ * is [attn_dims[0]][2 * mlp1_dims[1]] ([mlp1_out | group mean] columns), or [attn_dims[0]][mlp1_dims[1]] with
+ * without_global_state. */
 int cn_policy_load_weights(cn_policy *p, const float *flat_host, int64_t n, void *stream);
 /* CADRL.build_action_space (cadrl.py:82-102), holonomic; out: A x 2 doubles; returns A via *n_actions. */
 int cn_policy_action_table(cn_policy *p, double *out_xy_host, int32_t *n_actions);
@@ -355,7 +361,8 @@ int cn_world_predict(cn_world *w, cn_env *env, void *stream);
 /* ---- value-network training step on the device (crowd_nav/utils/trainer.py:36-82) ------------------------------------
  * One optimisation step of the reference Trainer -- zero_grad, model(inputs), MSELoss, backward, SGD(momentum).step -- as
  * two kernels on ONE flat fp32 parameter block in torch state-dict order (the block cn_policy_load_weights takes; the
- * torch model's parameters may be views of it).  SARL value network without occupancy maps.
+ * torch model's parameters may be views of it).  SARL value network without occupancy maps, with or without the global
+ * state (cn_sarl_cfg.without_global_state).
  * cn_trainer_step: states_dev batch x human_num x input_dim fp32, targets_dev batch fp32 (device pointers).
  *   grad_out_dev == NULL : w_dev is updated in place (buf = momentum * buf + grad; w -= lr * buf), loss_dev (optional)
  *                          receives the batch MSE.

@@ -55,7 +55,8 @@ class SarlCfg(C.Structure):
                 ("speed_samples", C.c_int32), ("rotation_samples", C.c_int32), ("gamma", C.c_double),
                 ("v_pref", C.c_double), ("precision", C.c_int32), ("kinematics", C.c_int32),
                 ("network", C.c_int32), ("lstm_hidden", C.c_int32), ("lstm_mlp1_dims", C.c_int32 * 4),
-                ("with_om", C.c_int32), ("cell_num", C.c_int32), ("cell_size", C.c_double), ("om_channel_size", C.c_int32)]
+                ("with_om", C.c_int32), ("cell_num", C.c_int32), ("cell_size", C.c_double), ("om_channel_size", C.c_int32),
+                ("without_global_state", C.c_int32)]
 
 
 class RolloutRecord(C.Structure):

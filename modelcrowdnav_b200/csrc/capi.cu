@@ -52,6 +52,7 @@ static SarlDims dims_of(const cn_sarl_cfg *c, int om_dim)
     for (int i = 0; i < 4; ++i) d.lm1[i] = c->network == CN_NET_LSTM_RL ? c->lstm_mlp1_dims[i] : 0;
     d.lstm_in = d.lm1[0] > 0 ? d.lm1[3] : d.in;
     d.om_dim = om_dim; d.cell_num = c->cell_num; d.om_ch = c->om_channel_size; d.cell_size = c->cell_size;
+    d.no_gs = c->network == CN_NET_SARL && c->without_global_state ? 1 : 0;
     return d;
 }
 
@@ -72,7 +73,7 @@ std::vector<LayerSpec> cn_layers(const SarlDims &d, SarlWeightsDev &w)
     } else {                                              // mlp1.* mlp2.* attention.* mlp3.*
         chain(2, d.m1, w.m1);
         chain(2, d.m2, w.m2);
-        in = 2 * d.m1[1];
+        in = d.no_gs ? d.m1[1] : 2 * d.m1[1];           // attention.0 on [mlp1_out | mean] or mlp1_out (sarl.py:40-47)
         chain(3, d.at, w.at);
         in = d.m2[1] + d.self_dim;
         chain(4, d.m3, w.m3);
@@ -556,6 +557,9 @@ int cn_policy_create(const cn_sarl_cfg *cfg, int device, cn_policy **out)
     if (cfg->attn_dims[2] != 1 || cfg->mlp3_dims[3] != 1) { cn_set_error("attention and mlp3 must end in 1 unit"); return CN_EINVAL; }
     if (cfg->network != CN_NET_SARL && cfg->network != CN_NET_CADRL && cfg->network != CN_NET_LSTM_RL) {
         cn_set_error("unknown value network %d", cfg->network); return CN_EINVAL;
+    }
+    if (cfg->without_global_state && cfg->network != CN_NET_SARL) {
+        cn_set_error("without_global_state is a [sarl] option; CADRL and LSTM-RL have no global state"); return CN_EINVAL;
     }
     if (cfg->network == CN_NET_LSTM_RL) {
         if (cfg->lstm_hidden < 1 || cfg->lstm_hidden > 64) { cn_set_error("1 <= lstm_hidden <= 64 required"); return CN_EINVAL; }

@@ -94,6 +94,7 @@ struct SarlDims {
     int om_dim;     // occupancy-map floats per row (0 = with_om off), cell_num^2 * om_ch
     int cell_num, om_ch;
     double cell_size;
+    int no_gs;      // SARL without the global state: attention.0 reads mlp1_out only (in = m1[1])
 };
 
 // build_occupancy_maps for ONE human (multi_human_rl.py:109-163): grid of cell_num x cell_num cells of cell_size metres

@@ -111,13 +111,14 @@ __device__ void sarl_forward_smem(const SarlWeightsDev &W, const SarlDims &d, co
     __syncthreads();
     layer(W.m1[1], 0, d.m1[0], T0, pl.wT0, 1, M1, pl.wM1, rows, false, true, true);  // mlp1.2 + ReLU (last_relu)
     __syncthreads();
-    // global state = mean over humans (sarl.py:42); self_state = x[:, 0, :6] (sarl.py:36)
-    for (int i = threadIdx.x; i < ng * G1; i += blockDim.x) {
-        const int g = i / G1, k = i - g * G1;
-        float s = 0.0f;
-        for (int h = 0; h < H; ++h) s += M1[(size_t)(g * H + h) * pl.wM1 + k];
-        G[(size_t)g * pl.wM1 + k] = s / (float)H;
-    }
+    // global state = mean over humans (sarl.py:42), unless with_global_state = false; self_state = x[:, 0, :6] (sarl.py:36)
+    if (!d.no_gs)
+        for (int i = threadIdx.x; i < ng * G1; i += blockDim.x) {
+            const int g = i / G1, k = i - g * G1;
+            float s = 0.0f;
+            for (int h = 0; h < H; ++h) s += M1[(size_t)(g * H + h) * pl.wM1 + k];
+            G[(size_t)g * pl.wM1 + k] = s / (float)H;
+        }
     for (int i = threadIdx.x; i < ng * d.self_dim; i += blockDim.x) {
         const int g = i / d.self_dim, k = i - g * d.self_dim;
         J[(size_t)g * pl.wJ + k] = X[(size_t)(g * H) * pl.wX + k];
@@ -126,10 +127,15 @@ __device__ void sarl_forward_smem(const SarlWeightsDev &W, const SarlDims &d, co
     __syncthreads();
     layer(W.m2[1], 0, d.m2[0], T0, pl.wT0, 1, F, pl.wF, rows, false, true, false);   // mlp2.2
     __syncthreads();
-    // attention.0 on cat([mlp1_out, global]) (sarl.py:45): two partial products
-    layer(W.at[0], 0, G1, M1, pl.wM1, 1, T0, pl.wT0, rows, false, false, false);
-    __syncthreads();
-    layer(W.at[0], G1, G1, G, pl.wM1, H, T0, pl.wT0, rows, true, true, true);
+    if (d.no_gs) {
+        // attention.0 on mlp1_out alone (sarl.py:47)
+        layer(W.at[0], 0, G1, M1, pl.wM1, 1, T0, pl.wT0, rows, false, true, true);
+    } else {
+        // attention.0 on cat([mlp1_out, global]) (sarl.py:45): two partial products
+        layer(W.at[0], 0, G1, M1, pl.wM1, 1, T0, pl.wT0, rows, false, false, false);
+        __syncthreads();
+        layer(W.at[0], G1, G1, G, pl.wM1, H, T0, pl.wT0, rows, true, true, true);
+    }
     __syncthreads();
     layer(W.at[1], 0, d.at[0], T0, pl.wT0, 1, M1, pl.wM1, rows, false, true, true);  // attention.2 + ReLU
     __syncthreads();

@@ -6,7 +6,8 @@
 //  tc_features_kernel   rows = (env, action, human): propagate + reward + rotate -> X tiles (13 features, split hi+lo
 //       fp16 so layer 1 sees ~22-bit inputs), lookahead rewards, self-state chunks of the joint state J
 //  tc_rows_pair_kernel  per 128-row tile, all on chip:
-//       mlp1.0 -> mlp1.2 -> {mlp2.0 -> mlp2.2 ; attention.0 on [mlp1_out | group mean] -> attention.2}
+//       mlp1.0 -> mlp1.2 -> {mlp2.0 -> mlp2.2 ; attention.0 on [mlp1_out | group mean] (or on mlp1_out alone without the
+//       global state) -> attention.2}
 //       attention.4 (fp32 dot) -> masked softmax over the humans of a group -> weighted feature
 //       -> joint state J (fp16, 160 B per (env, action)) to HBM, already in UMMA operand order
 //  tc_mlp3_pair_kernel  rows = (env, action).  mlp3.0 -> .2 -> .4 on tensor cores, .6 as an fp32 dot,
@@ -106,6 +107,14 @@ __device__ __forceinline__ void split_hl(float x, float &hi, float &lo)
 #include "tc_rows_pair.cuh"
 #include "tc_mlp3_pair.cuh"
 #include "tc_lstm_pair.cuh"
+
+// tc_rows_pair_kernel<HT, OM, GS> as kRowsKernels[!GS][OM][HT = 0, 5, 10]
+using RowsKernel = decltype(&tc_rows_pair_kernel<0, false, true>);
+constexpr RowsKernel kRowsKernels[2][2][3] = {
+    {{tc_rows_pair_kernel<0, false, true>, tc_rows_pair_kernel<5, false, true>, tc_rows_pair_kernel<10, false, true>},
+     {tc_rows_pair_kernel<0, true, true>, tc_rows_pair_kernel<5, true, true>, tc_rows_pair_kernel<10, true, true>}},
+    {{tc_rows_pair_kernel<0, false, false>, tc_rows_pair_kernel<5, false, false>, tc_rows_pair_kernel<10, false, false>},
+     {tc_rows_pair_kernel<0, true, false>, tc_rows_pair_kernel<5, true, false>, tc_rows_pair_kernel<10, true, false>}}};
 
 // =====================================================================================================
 // self-test kernel: D[128 x N] = A[128 x K] * B[N x K]^T
@@ -225,8 +234,9 @@ void fill_tail(const HostLinear &L, float *tail)
 }
 
 // The row network (mlp1, mlp2, attention: L[0..6]) as the two half images of tc_rows_pair_kernel (CTA `rank` holds output
-// rows [rank N/2, (rank+1) N/2) of every layer); attention.4 goes to `tail`.
-std::vector<uint8_t> rows_image(const HostLinear *L, float *tail)
+// rows [rank N/2, (rank+1) N/2) of every layer); attention.4 goes to `tail`.  gs = false: attention.0 has only the 100
+// mlp1_out columns (sarl.py:40-47) and the group-mean half H_WB stays empty (tc_rows_pair_kernel<.., .., false> never reads it).
+std::vector<uint8_t> rows_image(const HostLinear *L, bool gs, float *tail)
 {
     std::vector<uint8_t> a(IMG_A_BYTES, 0);
     // mlp1.0: K = [x_hi(13) 1 1 0 | x_lo(13) 0 0 0]; bias at k = 13,14; ones -> n = 150,151
@@ -236,7 +246,7 @@ std::vector<uint8_t> rows_image(const HostLinear *L, float *tail)
     fill_layer(a, OFF_W3, N_M1, L[2], 0, 100, 0, 100, 100);          // mlp2.0
     fill_layer(a, OFF_W4, N_F, L[3], 0, 100, 0, 100, -1);            // mlp2.2 (no ones needed downstream)
     fill_layer(a, OFF_WA1, N_M1, L[4], 0, 100, 0, 100, 100);         // attention.0, mlp1_out half
-    fill_layer(a, OFF_WA1, N_M1, L[4], 100, 100, N_M1, -1, -1);      //              group-mean half
+    if (gs) fill_layer(a, OFF_WA1, N_M1, L[4], 100, 100, N_M1, -1, -1);   //          group-mean half
     fill_layer(a, OFF_WA2, N_M1, L[5], 0, 100, 0, 100, -1);          // attention.2
     fill_tail(L[6], tail);
     std::vector<uint8_t> hp(2 * IMG_H_BYTES, 0);
@@ -246,7 +256,7 @@ std::vector<uint8_t> rows_image(const HostLinear *L, float *tail)
         split_rows(h + H_W2, a.data() + OFF_W2, N_M1, N_H1, rank);
         // stage 2 is ONE N = 224 UMMA: rank 0's half = attention.0 (mlp1_out half of K) -> D [0,112), rank 1's = mlp2.0 -> [112,224)
         memcpy(h + H_W3A, rank == 0 ? a.data() + OFF_WA1 : a.data() + OFF_W3, bytes_of(N_M1, N_M1));
-        split_rows(h + H_WB, a.data() + OFF_WA1 + bytes_of(N_M1, N_M1), N_M1, N_M1, rank);   // group-mean half of K
+        if (gs) split_rows(h + H_WB, a.data() + OFF_WA1 + bytes_of(N_M1, N_M1), N_M1, N_M1, rank);   // group-mean half of K
         split_rows(h + H_W4, a.data() + OFF_W4, N_F, N_M1, rank);
         split_rows(h + H_WA2, a.data() + OFF_WA2, N_M1, N_M1, rank);
         memcpy(h + H_TAIL, tail, TAIL_BYTES);      // copied to shared memory by the kernel, which reads the TailW parameter
@@ -440,12 +450,9 @@ int cn_tc_init(cn_policy *p)
     cudaDeviceProp prop;
     CN_CUDA_CHECK(cudaGetDeviceProperties(&prop, p->device));
     t->num_sms = prop.multiProcessorCount;
-    CN_CUDA_CHECK(cudaFuncSetAttribute(tc_rows_pair_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
-    CN_CUDA_CHECK(cudaFuncSetAttribute(tc_rows_pair_kernel<5, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
-    CN_CUDA_CHECK(cudaFuncSetAttribute(tc_rows_pair_kernel<10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
-    CN_CUDA_CHECK(cudaFuncSetAttribute(tc_rows_pair_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
-    CN_CUDA_CHECK(cudaFuncSetAttribute(tc_rows_pair_kernel<5, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
-    CN_CUDA_CHECK(cudaFuncSetAttribute(tc_rows_pair_kernel<10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
+    for (const auto &by_om : kRowsKernels)
+        for (const auto &by_ht : by_om)
+            for (RowsKernel k : by_ht) CN_CUDA_CHECK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Q_SMEM));
     CN_CUDA_CHECK(cudaFuncSetAttribute(tc_mlp3_pair_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)M_SMEM));
     CN_CUDA_CHECK(cudaFuncSetAttribute(tc_mlp3_pair_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)M_SMEM));
     CN_CUDA_CHECK(cudaFuncSetAttribute(tc_lstm_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L_SMEM));
@@ -494,7 +501,7 @@ int cn_tc_load_weights(cn_policy *p, const float *flat, cudaStream_t s)
     std::vector<uint8_t> hp, hl;
     CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair_b, hb.data(), hb.size(), cudaMemcpyHostToDevice, s));
     if (d.net == CN_NET_SARL) {
-        hp = rows_image(L.data(), t->tail_a);
+        hp = rows_image(L.data(), !d.no_gs, t->tail_a);
         CN_CUDA_CHECK(cudaMemcpyAsync(t->img_pair, hp.data(), hp.size(), cudaMemcpyHostToDevice, s));
     } else if (d.net == CN_NET_LSTM_RL) {
         hl = lstm_image(lstm);
@@ -568,8 +575,7 @@ int cn_lookahead_tc(cn_policy *p, cn_env *env, int query_env, double epsilon, cu
                                                                                           env->human_v, query_env, t->omP);
             CN_LAUNCH_CHECK();
         }
-        auto rows = om ? (ht == 5 ? tc_rows_pair_kernel<5, true> : (ht == 10 ? tc_rows_pair_kernel<10, true> : tc_rows_pair_kernel<0, true>))
-                       : (ht == 5 ? tc_rows_pair_kernel<5, false> : (ht == 10 ? tc_rows_pair_kernel<10, false> : tc_rows_pair_kernel<0, false>));
+        const RowsKernel rows = kRowsKernels[p->d.no_gs ? 1 : 0][om ? 1 : 0][ht == 5 ? 1 : (ht == 10 ? 2 : 0)];
         // PDL: the CTAs' prologue runs under the feature kernel's tail (pdl_wait() in the kernel); with om the bias kernel
         // sits between the two -> plain launch
         if ((rc = cn_launch(rows, 2 * ga.clusters, kThreadsPair, Q_SMEM, s, !om && !pipelined, env->p, t->img_pair, t->X, t->J, (int)NG,

@@ -25,6 +25,14 @@
 //          humans of the group in shared memory -> joint state J (fp16) -> HBM
 // The next tile's propagate / rotate features, clearances and rewards are computed under stages 2-3.
 //
+// GS = false ([sarl] with_global_state = false, sarl.py:40-47: attention.0 reads mlp1_out only) drops the group mean and
+// stage 3, so a tile has FOUR stages and one cross-CTA hand-over less; the shared-memory and TMEM maps are the same:
+//   stage  UMMA                                                A operand        D          epilogue
+//   0, 1   as above
+//   2      [attn.0 | mlp2.0]     K=112  N=224, own commit      mlp1_out (R2)    [0,224)    ReLU -> Ha1 fp16 IN PLACE in TMEM [0,56), H3 (R1)
+//   3      attn.2 ; mlp2.2       as stage 4 above                                          as stage 4 above
+// The number of completions per tile stays four (stage 2 commits itself instead of riding on stage 3's commit).
+//
 // Reference: crowd_nav/policy/sarl.py:28-65 (value network), cadrl.py:104-129,217-252 (propagate, rotate),
 // multi_human_rl.py:65-88 / crowd_sim.py:344-403 (lookahead reward).
 
@@ -44,7 +52,7 @@ constexpr int T_F = T_A2 + N_M1;           // mlp2.2 accumulator (the pairwise f
 constexpr uint32_t H_W1 = 0;                                        //  80 x 32
 constexpr uint32_t H_W2 = H_W1 + bytes_of(N_H1 / 2, K_X);           //  56 x 160
 constexpr uint32_t H_W3A = H_W2 + bytes_of(N_M1 / 2, N_H1);         // 112 x 112  (rank 0: attention.0 first half, rank 1: mlp2.0)
-constexpr uint32_t H_WB = H_W3A + bytes_of(N_M1, N_M1);             //  56 x 112  attention.0, group-mean half
+constexpr uint32_t H_WB = H_W3A + bytes_of(N_M1, N_M1);             //  56 x 112  attention.0, group-mean half (GS only)
 constexpr uint32_t H_W4 = H_WB + bytes_of(N_M1 / 2, N_M1);          //  32 x 112
 constexpr uint32_t H_WA2 = H_W4 + bytes_of(N_F / 2, N_M1);          //  56 x 112
 constexpr uint32_t H_TAIL = H_WA2 + bytes_of(N_M1 / 2, N_M1);       // fp32: attention.4 weight[100], bias
@@ -277,7 +285,8 @@ __device__ __forceinline__ void ctx_barrier(int ctx)
 // HT = compile-time human count (5, 10: the benchmark configurations) or 0 = run-time H
 // OM = occupancy maps (multi_human_rl.py:109-163): the map of a human does not depend on the robot's action, so its product
 // with mlp1.0's map columns is one fp32 row bias per (env, human) (omP, from tc_om_bias_kernel), added in the E0 epilogue
-template <int HT, bool OM>
+// GS = the global state: attention.0 on [mlp1_out | group mean] (five stages per tile), or on mlp1_out alone (four stages)
+template <int HT, bool OM, bool GS>
 // __maxnreg__(88), not __launch_bounds__ (the two exclude each other): see cn_small_block() in cn_common.cuh -- 88 registers
 // leave room for one <= 72-register warp of another shard's small kernels in every SM sub-partition; no measurable cost here.
 __global__ void __cluster_dims__(2, 1, 1) __maxnreg__(88)
@@ -335,7 +344,8 @@ tc_rows_pair_kernel(EnvParams p,
         if (rank == 0 && lane == 0) {
             const uint32_t sW1 = smem_u32(smem + H_W1), sW2 = smem_u32(smem + H_W2), sW3A = smem_u32(smem + H_W3A);
             const uint32_t sWB = smem_u32(smem + H_WB), sW4 = smem_u32(smem + H_W4), sWA2 = smem_u32(smem + H_WA2);
-            const int total = 5 * rounds;
+            constexpr int NS = GS ? 5 : 4;                  // UMMA stages per tile
+            const int total = NS * rounds;
             int stage0 = 0, stage1 = 0;
             uint32_t ph0 = 0, ph1 = 0, phm0 = 0, phm1 = 0, phx0 = 0, phx1 = 0;
             uint32_t idle_polls = 0;
@@ -344,23 +354,23 @@ tc_rows_pair_kernel(EnvParams p,
                 for (int c = 0; c < 2; ++c) {
                     int &stage = c ? stage1 : stage0;
                     if (stage >= total) continue;
-                    const int s = stage % 5;
-                    uint32_t &ph = (s == 3) ? (c ? phm1 : phm0) : (c ? ph1 : ph0);
-                    if (!mbar_test_wait_cluster((s == 3) ? (c ? reqm1 : reqm0) : (c ? req1 : req0), ph)) continue;
+                    const int s = stage % NS;
+                    uint32_t &ph = (GS && s == 3) ? (c ? phm1 : phm0) : (c ? ph1 : ph0);
+                    if (!mbar_test_wait_cluster((GS && s == 3) ? (c ? reqm1 : reqm0) : (c ? req1 : req0), ph)) continue;
                     if (s == 0) {                                   // stage 0 also needs the TMA-landed X of both CTAs
                         uint32_t &phx = c ? phx1 : phx0;
                         if (!mbar_test_wait_cluster(c ? xfull1 : xfull0, phx)) continue;
                         phx ^= 1;
                     }
                     ph ^= 1;
-                    const bool probe_round = stage / 5 == 3;
+                    const bool probe_round = stage / NS == 3;
                     QPROBE(2 + c, 2 * s);
                     fence_after_sync();
                     const uint32_t tm = tmem + (uint32_t)c * PAIR_CTX_COLS;
                     const uint32_t sR1 = smem_u32(smem + Q_CTX0 + (uint32_t)c * Q_CTX_BYTES), sR2 = sR1 + Q_R1_BYTES;
                     const uint32_t done = c ? done1 : done0;
 #ifdef CN_ABLATE_MMA
-                    if (s != 2) commit_2(done, 3);
+                    if (!GS || s != 2) commit_2(done, 3);
                     if (1) {
                     } else if (s == 0) {
 #else
@@ -374,8 +384,9 @@ tc_rows_pair_kernel(EnvParams p,
                         mma_steps_2_ts(tm + T_D1, tm + T_H1B, sW2, N_H1 / 32, N_H1 / 16, N_M1, true);
                         commit_2(done, 3);
                     } else if (s == 2) {
-                        mma_layer_2(tm, sR2, ROWS, sW3A, N_M1, N_S2, false);          // completion rides on stage 3's commit
-                    } else if (s == 3) {
+                        mma_layer_2(tm, sR2, ROWS, sW3A, N_M1, N_S2, false);          // GS: completion rides on stage 3's commit
+                        if constexpr (!GS) commit_2(done, 3);
+                    } else if (GS && s == 3) {
                         mma_layer_2(tm, sR1, ROWS, sWB, N_M1, N_M1, true);             // attention.0 accumulator = [0,112)
                         commit_2(done, 3);
                     } else {
@@ -483,81 +494,84 @@ tc_rows_pair_kernel(EnvParams p,
             else epilogue_to_smem<true>(tl, T_D1 + 64, 48, R2, row, 8);
 #endif
             PAIR_SIGNAL(); QPROBE(ctx, 4);                                         // stage 2 may start
-            QPROBE(ctx, 12);
-            // ---- group mean of mlp1_out over the humans of a group (sarl.py:42), replicated on the group's rows -> R1 ----
-            ctx_barrier(ctx);
-            QPROBE(ctx, 13);
+            if constexpr (GS) {
+                QPROBE(ctx, 12);
+                // ---- group mean of mlp1_out over the humans of a group (sarl.py:42), replicated on the group's rows -> R1 ----
+                ctx_barrier(ctx);
+                QPROBE(ctx, 13);
 #ifdef CN_ABLATE_EPI
-            if (0) {
+                if (0) {
 #else
-            if (!HT && mean_split >= 2) {
+                if (!HT && mean_split >= 2) {
 #endif
-                const int P = mean_split, nitems = G * (N_M1 / 8);
-                const int it = t256 / P, seg = t256 & (P - 1);
-                const bool on = it < nitems;
-                const int c = on ? it / G : 0, gl = on ? it - c * G : 0;
-                const int n = on ? (H - seg + P - 1) / P : 0;                    // rows seg, seg + P, ... of the group
-                float acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-                sum_f16x8_rows(R2 + chunk_off(ROWS, gl * H + seg, c), n, 16u * P, acc);
-                for (int off = 1; off < P; off <<= 1)                                // whole warps take part (it may be off)
+                    const int P = mean_split, nitems = G * (N_M1 / 8);
+                    const int it = t256 / P, seg = t256 & (P - 1);
+                    const bool on = it < nitems;
+                    const int c = on ? it / G : 0, gl = on ? it - c * G : 0;
+                    const int n = on ? (H - seg + P - 1) / P : 0;                    // rows seg, seg + P, ... of the group
+                    float acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+                    sum_f16x8_rows(R2 + chunk_off(ROWS, gl * H + seg, c), n, 16u * P, acc);
+                    for (int off = 1; off < P; off <<= 1)                                // whole warps take part (it may be off)
 #pragma unroll
-                    for (int k = 0; k < 8; ++k) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], off);
-                const uint4 o = make_uint4(h2(acc[0] * invH, acc[1] * invH), h2(acc[2] * invH, acc[3] * invH),
-                                           h2(acc[4] * invH, acc[5] * invH), h2(acc[6] * invH, acc[7] * invH));
-                for (int h = seg; h < H && on; h += P)                               // replicate on the same rows
-                    *reinterpret_cast<uint4 *>(R1 + chunk_off(ROWS, gl * H + h, c)) = o;
-            } else
+                        for (int k = 0; k < 8; ++k) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], off);
+                    const uint4 o = make_uint4(h2(acc[0] * invH, acc[1] * invH), h2(acc[2] * invH, acc[3] * invH),
+                                               h2(acc[4] * invH, acc[5] * invH), h2(acc[6] * invH, acc[7] * invH));
+                    for (int h = seg; h < H && on; h += P)                               // replicate on the same rows
+                        *reinterpret_cast<uint4 *>(R1 + chunk_off(ROWS, gl * H + h, c)) = o;
+                } else
 #pragma unroll
-            for (int i = 0; i < kMeanIters; ++i) {
+                for (int i = 0; i < kMeanIters; ++i) {
 #ifdef CN_ABLATE_EPI
-                break;
+                    break;
 #endif
-                if (mean_off[i] < 0) continue;
-                const uint8_t *src = R2 + mean_off[i];
-                uint4 v[HT ? HT : 1];
-                __half2 acc[4];
-                if (HT) {
+                    if (mean_off[i] < 0) continue;
+                    const uint8_t *src = R2 + mean_off[i];
+                    uint4 v[HT ? HT : 1];
+                    __half2 acc[4];
+                    if (HT) {
 #pragma unroll
-                    for (int h = 0; h < HT; ++h) v[h] = *reinterpret_cast<const uint4 *>(src + h * 16);
-                    const __half2 *h0 = reinterpret_cast<const __half2 *>(&v[0]);
-                    acc[0] = h0[0]; acc[1] = h0[1]; acc[2] = h0[2]; acc[3] = h0[3];
+                        for (int h = 0; h < HT; ++h) v[h] = *reinterpret_cast<const uint4 *>(src + h * 16);
+                        const __half2 *h0 = reinterpret_cast<const __half2 *>(&v[0]);
+                        acc[0] = h0[0]; acc[1] = h0[1]; acc[2] = h0[2]; acc[3] = h0[3];
 #pragma unroll
-                    for (int h = 1; h < HT; ++h) {
-                        const __half2 *hv = reinterpret_cast<const __half2 *>(&v[h]);
+                        for (int h = 1; h < HT; ++h) {
+                            const __half2 *hv = reinterpret_cast<const __half2 *>(&v[h]);
 #pragma unroll
-                        for (int k = 0; k < 4; ++k) acc[k] = __hadd2(acc[k], hv[k]);
+                            for (int k = 0; k < 4; ++k) acc[k] = __hadd2(acc[k], hv[k]);
+                        }
+                    } else {
+                        v[0] = *reinterpret_cast<const uint4 *>(src);
+                        const __half2 *h0 = reinterpret_cast<const __half2 *>(&v[0]);
+                        acc[0] = h0[0]; acc[1] = h0[1]; acc[2] = h0[2]; acc[3] = h0[3];
+                        for (int h = 1; h < H; ++h) {
+                            const uint4 u = *reinterpret_cast<const uint4 *>(src + h * 16);
+                            const __half2 *hv = reinterpret_cast<const __half2 *>(&u);
+#pragma unroll
+                            for (int k = 0; k < 4; ++k) acc[k] = __hadd2(acc[k], hv[k]);
+                        }
                     }
-                } else {
-                    v[0] = *reinterpret_cast<const uint4 *>(src);
-                    const __half2 *h0 = reinterpret_cast<const __half2 *>(&v[0]);
-                    acc[0] = h0[0]; acc[1] = h0[1]; acc[2] = h0[2]; acc[3] = h0[3];
-                    for (int h = 1; h < H; ++h) {
-                        const uint4 u = *reinterpret_cast<const uint4 *>(src + h * 16);
-                        const __half2 *hv = reinterpret_cast<const __half2 *>(&u);
+                    uint4 o;
+                    {
+                        const float2 f0 = __half22float2(acc[0]), f1 = __half22float2(acc[1]);
+                        const float2 f2 = __half22float2(acc[2]), f3 = __half22float2(acc[3]);
+                        o.x = h2(f0.x * invH, f0.y * invH); o.y = h2(f1.x * invH, f1.y * invH);
+                        o.z = h2(f2.x * invH, f2.y * invH); o.w = h2(f3.x * invH, f3.y * invH);
+                    }
+                    uint8_t *dst = R1 + mean_off[i];
+                    if (HT) {
 #pragma unroll
-                        for (int k = 0; k < 4; ++k) acc[k] = __hadd2(acc[k], hv[k]);
+                        for (int h = 0; h < HT; ++h) *reinterpret_cast<uint4 *>(dst + h * 16) = o;
+                    } else {
+                        for (int h = 0; h < H; ++h) *reinterpret_cast<uint4 *>(dst + h * 16) = o;
                     }
                 }
-                uint4 o;
-                {
-                    const float2 f0 = __half22float2(acc[0]), f1 = __half22float2(acc[1]);
-                    const float2 f2 = __half22float2(acc[2]), f3 = __half22float2(acc[3]);
-                    o.x = h2(f0.x * invH, f0.y * invH); o.y = h2(f1.x * invH, f1.y * invH);
-                    o.z = h2(f2.x * invH, f2.y * invH); o.w = h2(f3.x * invH, f3.y * invH);
-                }
-                uint8_t *dst = R1 + mean_off[i];
-                if (HT) {
-#pragma unroll
-                    for (int h = 0; h < HT; ++h) *reinterpret_cast<uint4 *>(dst + h * 16) = o;
-                } else {
-                    for (int h = 0; h < H; ++h) *reinterpret_cast<uint4 *>(dst + h * 16) = o;
-                }
+                QPROBE(ctx, 14);
+                PAIR_SIGNAL_TO(reqm_leader); QPROBE(ctx, 5);
+                if (dbg && blockIdx.x < 2 && rnd == 3 && ctx == 0 && lane == 0) dbg[192 + blockIdx.x * 8 + hf * 4 + q] = clock64();                           // stage 3 may start
             }
-            QPROBE(ctx, 14);
-            PAIR_SIGNAL_TO(reqm_leader); QPROBE(ctx, 5);
-            if (dbg && blockIdx.x < 2 && rnd == 3 && ctx == 0 && lane == 0) dbg[192 + blockIdx.x * 8 + hf * 4 + q] = clock64();                           // stage 3 may start
             QPROBE(ctx, 6);
-            // ---- E3: H3 = relu(acc[0,112)) -> R1 (hf 0) ; Ha1 = relu(acc[112,224)) -> R2 (hf 1) ----
+            // ---- E3: Ha1 = relu(acc[0,112)) fp16 in place in TMEM (hf 0) ; H3 = relu(acc[112,224)) -> R1 (hf 1) ----
+            // (GS: after stage 3, whose commit covers stage 2; otherwise after stage 2's own commit)
             PAIR_WAIT(); QPROBE(ctx, 7);
 #ifndef CN_ABLATE_EPI
             if (hf == 0) compact_to_tmem<true, true>(tl, 0, N_M1, 0, 1.0f);         // Ha1: fp16 pairs in place, [0,56)

@@ -17,7 +17,8 @@
 //
 // Parameter layout = the torch state-dict order of ValueNetwork (mlp1.0, mlp1.2, mlp2.0, mlp2.2, attention.0, .2, .4,
 // mlp3.0, .2, .4, .6; weight [out][in] then bias), the same flat block cn_policy_load_weights takes, so the torch model's
-// parameters can be VIEWS of the block this trainer updates.
+// parameters can be VIEWS of the block this trainer updates.  Without the global state ([sarl] with_global_state = false,
+// sarl.py:40-47) attention.0 reads e_i itself: no [e | mean] input is built and its gradient has no mean term.
 #include "cn_common.cuh"
 #include "dense_f32.cuh"
 
@@ -42,6 +43,7 @@ struct TDims {
     TLayer L[kLayers];
     int n_params, t_size, a_size;
     int in, self_dim;
+    int no_gs;                 // without the global state: attention.0's input is e (L[4].in = E1), not [e | mean]
     int wbuf_floats;           // size of one staging buffer = the largest block
 };
 
@@ -76,7 +78,7 @@ __host__ __device__ inline Plan make_plan(const TDims &d, int H, int ns)
     p.e = o; o += R * p.ld_e;
     p.f1 = o; o += R * p.ld_f1;
     p.f = o; o += R * p.ld_f;
-    p.u = o; o += R * p.ld_u;             // attention input [e_i | mean]
+    p.u = o; o += R * p.ld_u;             // attention input [e_i | mean] (unused without the global state)
     p.t1 = o; o += R * p.ld_t;
     p.t2 = o; o += R * p.ld_t;
     p.sc = o; o += pad4(R);
@@ -188,20 +190,23 @@ trainer_fwd_bwd_kernel(TDims d, const float *__restrict__ Wt, const float *__res
     FWD(0, xs, p.ld_x, R, a1, p.ld_a1, true); end_op();                        // mlp1.0 + ReLU
     FWD(1, a1, p.ld_a1, R, e, p.ld_e, true); end_op();                         // mlp1.2 + ReLU (last_relu)
     FWD(2, e, p.ld_e, R, f1, p.ld_f1, true);                                   // mlp2.0 + ReLU
-    // attention input u = [e_i | mean over the sample's humans]
-    for (int idx = tid; idx < ns * E1; idx += kThreads) {
-        const int s = idx / E1, k = idx - s * E1;
-        float m = 0.0f;
-        for (int h = 0; h < H; ++h) m += e[(size_t)(s * H + h) * p.ld_e + k];
-        m /= (float)H;
-        for (int h = 0; h < H; ++h) {
-            u[(size_t)(s * H + h) * p.ld_u + k] = e[(size_t)(s * H + h) * p.ld_e + k];
-            u[(size_t)(s * H + h) * p.ld_u + E1 + k] = m;
+    // attention input u = [e_i | mean over the sample's humans]; without the global state attention.0 reads e itself
+    const float *att_in = d.no_gs ? e : u;
+    const int ld_att = d.no_gs ? p.ld_e : p.ld_u;
+    if (!d.no_gs)
+        for (int idx = tid; idx < ns * E1; idx += kThreads) {
+            const int s = idx / E1, k = idx - s * E1;
+            float m = 0.0f;
+            for (int h = 0; h < H; ++h) m += e[(size_t)(s * H + h) * p.ld_e + k];
+            m /= (float)H;
+            for (int h = 0; h < H; ++h) {
+                u[(size_t)(s * H + h) * p.ld_u + k] = e[(size_t)(s * H + h) * p.ld_e + k];
+                u[(size_t)(s * H + h) * p.ld_u + E1 + k] = m;
+            }
         }
-    }
     end_op();
     FWD(3, f1, p.ld_f1, R, f, p.ld_f, false); end_op();                        // mlp2.2
-    FWD(4, u, p.ld_u, R, t1, p.ld_t, true); end_op();                          // attention.0 + ReLU
+    FWD(4, att_in, ld_att, R, t1, p.ld_t, true); end_op();                     // attention.0 + ReLU
     FWD(5, t1, p.ld_t, R, t2, p.ld_t, true); end_op();                         // attention.2 + ReLU
     FWD(6, t2, p.ld_t, R, sc, 1, false); end_op();                             // attention.4 -> score
     if (tid < ns) {                                                            // masked softmax (sarl.py:52-53)
@@ -289,19 +294,24 @@ trainer_fwd_bwd_kernel(TDims d, const float *__restrict__ Wt, const float *__res
     weight_grad_call(dt2, p.ld_t, t1, p.ld_t, R, L[5].out, L[5].in, G + L[5].w_off, G + L[5].b_off);
     float *dt1 = t2;                                                // t2 is dead once its mask and attention.4's gradient are taken
     BWD(5, dt2, p.ld_t, R, dt1, p.ld_t, false, t1, p.ld_t); end_op();
-    // attention.0 on u = [e | mean]
-    weight_grad_call(dt1, p.ld_t, u, p.ld_u, R, L[4].out, L[4].in, G + L[4].w_off, G + L[4].b_off);
-    float *du = d1;                                                 // [R][ld_u]  (dt2 is dead)
-    BWD(4, dt1, p.ld_t, R, du, p.ld_u, false, nullptr, 0); end_op();
-    // de_i = du_i[:E1] + (1/H) sum_k du_k[E1:]  + mlp2.0's path (df1 W_20)
+    // attention.0 on u = [e | mean] (or on e)
+    weight_grad_call(dt1, p.ld_t, att_in, ld_att, R, L[4].out, L[4].in, G + L[4].w_off, G + L[4].b_off);
     float *de = t1;                                                 // t1 is dead; rows of ld_t floats
-    for (int idx = tid; idx < ns * E1; idx += kThreads) {
-        const int s = idx / E1, k = idx - s * E1;
-        float m = 0.0f;
-        for (int h = 0; h < H; ++h) m += du[(size_t)(s * H + h) * p.ld_u + E1 + k];
-        m /= (float)H;
-        for (int h = 0; h < H; ++h) de[(size_t)(s * H + h) * p.ld_t + k] = du[(size_t)(s * H + h) * p.ld_u + k] + m;
+    if (d.no_gs) {
+        BWD(4, dt1, p.ld_t, R, de, p.ld_t, false, nullptr, 0); end_op();      // de_i = du_i
+    } else {
+        float *du = d1;                                             // [R][ld_u]  (dt2 is dead)
+        BWD(4, dt1, p.ld_t, R, du, p.ld_u, false, nullptr, 0); end_op();
+        // de_i = du_i[:E1] + (1/H) sum_k du_k[E1:]
+        for (int idx = tid; idx < ns * E1; idx += kThreads) {
+            const int s = idx / E1, k = idx - s * E1;
+            float m = 0.0f;
+            for (int h = 0; h < H; ++h) m += du[(size_t)(s * H + h) * p.ld_u + E1 + k];
+            m /= (float)H;
+            for (int h = 0; h < H; ++h) de[(size_t)(s * H + h) * p.ld_t + k] = du[(size_t)(s * H + h) * p.ld_u + k] + m;
+        }
     }
+    // + mlp2.0's path (df1 W_20)
     BWD(2, df1, p.ld_f1, R, de, p.ld_t, true, e, p.ld_e); end_op();            // += df1 * W_mlp2.0   (begin_op's barrier publishes de)
     // mlp1.2
     weight_grad_call(de, p.ld_t, a1, p.ld_a1, R, L[1].out, L[1].in, G + L[1].w_off, G + L[1].b_off);
@@ -380,7 +390,8 @@ int cn_trainer_create(const cn_sarl_cfg *cfg, int device, int32_t max_batch, int
 {
     if (!cfg || !out) { cn_set_error("null argument"); return CN_EINVAL; }
     if (cfg->network != CN_NET_SARL || cfg->with_om) {
-        cn_set_error("the fused trainer covers the SARL value network without occupancy maps; use torch autograd for the others");
+        cn_set_error("the fused trainer covers the SARL value network without occupancy maps (with or without the global state); "
+                     "use torch autograd for the others");
         return CN_EUNSUPPORTED;
     }
     if (max_batch < 1 || max_humans < 1 || max_humans > kMaxH) { cn_set_error("1 <= max_humans <= %d, max_batch >= 1", kMaxH); return CN_EINVAL; }
@@ -392,7 +403,8 @@ int cn_trainer_create(const cn_sarl_cfg *cfg, int device, int32_t max_batch, int
     memset(t, 0, sizeof(*t));
     t->device = device; t->max_batch = max_batch; t->max_humans = max_humans;
     TDims &d = t->d;
-    const int ins[kLayers] = {cfg->input_dim, cfg->mlp1_dims[0], cfg->mlp1_dims[1], cfg->mlp2_dims[0], 2 * cfg->mlp1_dims[1],
+    const int att_in = cfg->without_global_state ? cfg->mlp1_dims[1] : 2 * cfg->mlp1_dims[1];
+    const int ins[kLayers] = {cfg->input_dim, cfg->mlp1_dims[0], cfg->mlp1_dims[1], cfg->mlp2_dims[0], att_in,
                               cfg->attn_dims[0], cfg->attn_dims[1], cfg->mlp2_dims[1] + cfg->self_state_dim, cfg->mlp3_dims[0],
                               cfg->mlp3_dims[1], cfg->mlp3_dims[2]};
     const int outs[kLayers] = {cfg->mlp1_dims[0], cfg->mlp1_dims[1], cfg->mlp2_dims[0], cfg->mlp2_dims[1], cfg->attn_dims[0],
@@ -409,7 +421,7 @@ int cn_trainer_create(const cn_sarl_cfg *cfg, int device, int32_t max_batch, int
         if (blk > wbuf) wbuf = blk;
     }
     d.n_params = off; d.t_size = toff; d.a_size = aoff; d.wbuf_floats = wbuf;
-    d.in = cfg->input_dim; d.self_dim = cfg->self_state_dim;
+    d.in = cfg->input_dim; d.self_dim = cfg->self_state_dim; d.no_gs = cfg->without_global_state ? 1 : 0;
     if (outs[6] != 1 || outs[10] != 1) { delete t; cn_set_error("attention and mlp3 must end in 1 unit"); return CN_EINVAL; }
     std::vector<int32_t> tmap(d.n_params), amap(d.n_params, -1);
     for (int i = 0; i < kLayers; ++i) {

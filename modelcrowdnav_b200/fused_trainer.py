@@ -117,4 +117,5 @@ def _layer_dims(model):
         return [m.out_features for m in seq if isinstance(m, torch.nn.Linear)]
     first = [m for m in model.mlp1 if isinstance(m, torch.nn.Linear)][0]
     return dict(input_dim=first.in_features, self_state_dim=model.self_state_dim, mlp1_dims=widths(model.mlp1),
-                mlp2_dims=widths(model.mlp2), attn_dims=widths(model.attention), mlp3_dims=widths(model.mlp3))
+                mlp2_dims=widths(model.mlp2), attn_dims=widths(model.attention), mlp3_dims=widths(model.mlp3),
+                without_global_state=int(not model.with_global_state))

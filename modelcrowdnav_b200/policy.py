@@ -245,10 +245,10 @@ class SARL(Policy):
         attention_dims = [int(x) for x in config.get("sarl", "attention_dims").split(", ")]
         self.with_om = config.getboolean("sarl", "with_om")
         with_global_state = config.getboolean("sarl", "with_global_state")
-        if not with_global_state:
-            raise NotImplementedError("with_global_state = false is not supported by the CUDA lookahead")
         self._dims = dict(mlp1_dims=mlp1_dims, mlp2_dims=mlp2_dims, attn_dims=attention_dims, mlp3_dims=mlp3_dims)
         self._net_kwargs = dict(self._dims, **self._om_kwargs())
+        if not with_global_state:
+            self._net_kwargs["without_global_state"] = 1
         self.model = make_value_network(self.input_dim(), self.self_state_dim, mlp1_dims, mlp2_dims, mlp3_dims,
                                         attention_dims, with_global_state)
         self.multiagent_training = config.getboolean("sarl", "multiagent_training")
