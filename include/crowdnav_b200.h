@@ -360,9 +360,19 @@ int cn_world_predict(cn_world *w, cn_env *env, void *stream);
 
 /* ---- value-network training step on the device (crowd_nav/utils/trainer.py:36-82) ------------------------------------
  * One optimisation step of the reference Trainer -- zero_grad, model(inputs), MSELoss, backward, SGD(momentum).step -- as
- * two kernels on ONE flat fp32 parameter block in torch state-dict order (the block cn_policy_load_weights takes; the
- * torch model's parameters may be views of it).  SARL value network without occupancy maps, with or without the global
- * state (cn_sarl_cfg.without_global_state).
+ * two kernels on ONE flat fp32 parameter block in torch state-dict order (the block cn_policy_load_weights takes, the same
+ * layer list; cn_trainer_param_count = cn_policy_param_count of the config; the torch model's parameters may be views of
+ * it).  Networks covered (cn_sarl_cfg.network):
+ *   CN_NET_SARL      SARL with or without the global state (without_global_state); with_om = 1: OM-SARL, mlp1.0 reads
+ *                    input_dim = 13 + cell_num^2 * om_channel_size columns (CN_EINVAL when input_dim disagrees).
+ *   CN_NET_CADRL     value_network = mlp(13 -> mlp3_dims) on single-human states (cadrl.py:209): max_humans and human_num
+ *                    must be 1 (CN_EINVAL otherwise); the batch is batch x input_dim.
+ *   CN_NET_LSTM_RL   ValueNetwork1 (lstm_mlp1_dims[0] == 0): nn.LSTM(input_dim -> lstm_hidden) over the human_num rows in the
+ *                    given order, then mlp(self_state_dim + lstm_hidden -> mlp3_dims) on [state[:, 0, :self_state_dim] | h_n];
+ *                    ValueNetwork2 (lstm_mlp1_dims[0] > 0): a per-row mlp1 in front of the LSTM.  With or without maps.
+ *                    Layout [mlp1.*] mlp.* lstm.weight_ih_l0, weight_hh_l0, bias_ih_l0, bias_hh_l0 (gates i, f, g, o).
+ * Limits: 1 <= max_humans <= 16 (SARL: CN_EINVAL above; CADRL and LSTM-RL: CN_EUNSUPPORTED); shapes whose activations and
+ * largest weight block (LSTM-RL: weight_hh, 4 lstm_hidden^2 floats) do not fit one CTA's shared memory: CN_EUNSUPPORTED.
  * cn_trainer_step: states_dev batch x human_num x input_dim fp32, targets_dev batch fp32 (device pointers).
  *   grad_out_dev == NULL : w_dev is updated in place (buf = momentum * buf + grad; w -= lr * buf), loss_dev (optional)
  *                          receives the batch MSE.

@@ -40,7 +40,7 @@ void cn_trace_mark(const char *name, cudaStream_t s)
 
 // ---- network shapes and state-dict layer lists ---------------------------------------------------
 // The network shape of a configuration (om_dim = 0 without occupancy maps)
-static SarlDims dims_of(const cn_sarl_cfg *c, int om_dim)
+SarlDims cn_dims_of(const cn_sarl_cfg *c, int om_dim)
 {
     SarlDims d;
     memset(&d, 0, sizeof(d));
@@ -495,7 +495,7 @@ int64_t cn_policy_param_count(const cn_sarl_cfg *c)
     if (!c) return 0;
     SarlWeightsDev w;        // only the destinations of the layer list, never written here
     int64_t n = 0;
-    for (const LayerSpec &l : cn_layers(dims_of(c, 0), w)) n += (int64_t)cn_layer_floats(l);
+    for (const LayerSpec &l : cn_layers(cn_dims_of(c, 0), w)) n += (int64_t)cn_layer_floats(l);
     return n;
 }
 
@@ -579,7 +579,7 @@ int cn_policy_create(const cn_sarl_cfg *cfg, int device, cn_policy **out)
     cn_policy *p = new cn_policy();
     memset(p, 0, sizeof(*p));
     p->device = device; p->cfg = *cfg;
-    p->d = dims_of(cfg, om_dim);
+    p->d = cn_dims_of(cfg, om_dim);
     SarlDims &d = p->d;
     d.A = build_action_table(cfg, p->action_host);
     p->n_params = cn_policy_param_count(cfg);

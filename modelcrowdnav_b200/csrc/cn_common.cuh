@@ -167,6 +167,7 @@ struct LayerSpec {
     int in, out;
     LinearDev *dst, *dst_hh;
 };
+SarlDims cn_dims_of(const cn_sarl_cfg *c, int om_dim);                   // the network shape of a configuration (capi.cu)
 std::vector<LayerSpec> cn_layers(const SarlDims &d, SarlWeightsDev &w);   // state-dict order of d.net (capi.cu)
 inline size_t cn_layer_floats(const LayerSpec &l)
 {

@@ -84,6 +84,21 @@ __device__ __forceinline__ void dense_t(const float *__restrict__ X, int ldx, in
     }
 }
 
+// Weight staging (the fused trainers): cp.async copies of a 16-byte aligned block of n floats (n a multiple of 4) from
+// global into shared memory, issued by the whole CTA as one commit group; cp_async_wait<N> leaves N groups in flight.
+__device__ __forceinline__ void cp_async16(float *dst_smem, const float *src)
+{
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" :: "n"(N) : "memory"); }
+__device__ __forceinline__ void stage_async(float *dst, const float *src, int n)
+{
+#pragma unroll 4
+    for (int i = threadIdx.x * 4; i < n; i += kThreads * 4) cp_async16(dst + i, src + i);
+    cp_async_commit();
+}
+
 __device__ __forceinline__ void dense(const float *__restrict__ X, int ldx, int R, int K, const float *__restrict__ Wt,
                                       const float *__restrict__ b, int O, float *__restrict__ Y, int ldy, bool relu, bool accumulate)
 {

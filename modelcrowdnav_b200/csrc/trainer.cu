@@ -1,26 +1,31 @@
-// trainer.cu -- one optimisation step of the SARL value network on the device (CN_NET_SARL, FP32):
+// trainer.cu -- one optimisation step of a value network on the device (FP32):
 //   MSE( ValueNetwork(states), targets ) -> backward -> [gradient all-reduce by the caller] -> SGD with momentum.
 // Replaces the ~150 kernel launches (+ one host sync) of the torch autograd step the reference runs per batch
 // (crowd_nav/utils/trainer.py:61-82: zero_grad, model(inputs), MSELoss, backward, SGD(momentum 0.9).step, loss.item())
 // with TWO kernels:
-//   trainer_fwd_bwd_kernel   one CTA per kSPC samples of the batch: the whole forward (sarl.py:28-65) and backward of those
-//                            samples with every activation in shared memory.  The 21 weight blocks a step walks through
-//                            (11 forward layers, 10 backward-data products) are STAGED: while layer i computes from one
-//                            shared-memory buffer, cp.async brings layer i + 1's block (<= 80 kB, L2-resident) into the
-//                            other -- streamed straight from L2 the dependent loads of a 256-thread CTA were all latency
-//                            (226 us per step in the ncu launch list, profiles/r02l_train_launches_summary.txt);
-//                            per-CTA partial weight gradients -> gpart[cta][n_params]
+//   trainer_fwd_bwd_kernel   SARL / OM-SARL (CN_NET_SARL): one CTA per kSPC samples of the batch: the whole forward
+//                            (sarl.py:28-65) and backward of those samples with every activation in shared memory.  The 21
+//                            weight blocks a step walks through (11 forward layers, 10 backward-data products) are STAGED:
+//                            while layer i computes from one shared-memory buffer, cp.async brings layer i + 1's block
+//                            (<= 80 kB, L2-resident) into the other -- streamed straight from L2 the dependent loads of a
+//                            256-thread CTA were all latency (226 us per step in the ncu launch list,
+//                            profiles/r02l_train_launches_summary.txt); per-CTA partial weight gradients -> gpart[cta][n_params]
+//   trainer_nets_fwd_bwd_kernel   the same for CADRL and LSTM-RL (ValueNetwork1 / 2, with or without maps): trainer_nets.cu
 //   trainer_reduce_kernel    fixed-order sum of the partials (deterministic) -> gradient; with grad_out == NULL it also
 //                            applies SGD momentum in place and refreshes the transposed weight copy the forward reads
 //   trainer_apply_kernel     the SGD half alone, for the data-parallel form (gradient -> NCCL all-reduce -> apply)
-// FP32 FMA bound: ~3 x 62 k MAC per (sample, human) row; 100 x 5 rows = 0.1 GFLOP per step.
+// SARL is FP32 FMA bound: ~3 x 62 k MAC per (sample, human) row; 100 x 5 rows = 0.1 GFLOP per step.
 //
-// Parameter layout = the torch state-dict order of ValueNetwork (mlp1.0, mlp1.2, mlp2.0, mlp2.2, attention.0, .2, .4,
-// mlp3.0, .2, .4, .6; weight [out][in] then bias), the same flat block cn_policy_load_weights takes, so the torch model's
-// parameters can be VIEWS of the block this trainer updates.  Without the global state ([sarl] with_global_state = false,
-// sarl.py:40-47) attention.0 reads e_i itself: no [e | mean] input is built and its gradient has no mean term.
+// Parameter layout = the torch state-dict order of the value network, the same flat block cn_policy_load_weights takes,
+// derived from the same layer list (cn_layers), so the torch model's parameters can be VIEWS of the block this trainer
+// updates.  SARL: mlp1.0, mlp1.2, mlp2.0, mlp2.2, attention.0, .2, .4, mlp3.0, .2, .4, .6 (weight [out][in] then bias);
+// with occupancy maps mlp1.0 reads 13 + cell_num^2 * om_channel_size columns.  Without the global state ([sarl]
+// with_global_state = false, sarl.py:40-47) attention.0 reads e_i itself: no [e | mean] input is built and its gradient has
+// no mean term.  CADRL: value_network.{0,2,4,6}.  LSTM-RL: [mlp1.*] mlp.* lstm.weight_ih_l0, weight_hh_l0, bias_ih_l0,
+// bias_hh_l0.
 #include "cn_common.cuh"
 #include "dense_f32.cuh"
+#include "trainer_nets.cuh"
 
 #include <math.h>
 #include <string.h>
@@ -34,11 +39,6 @@ constexpr int kSPC = 1;           // samples per CTA: 100 CTAs for the reference
 constexpr int kMaxH = 16;         // humans per sample supported by the shared-memory plan
 constexpr int kLayers = 11;
 
-// w_off / b_off: the flat master block (torch state-dict order).  t_off: this layer's block in the transposed copy Wt --
-// [in][out] followed by the bias, both padded to 4 floats, 16-byte aligned (one cp.async target).  a_off: its block in the
-// aligned copy Wa of the ORIGINAL [out][in] layout (what the backward-data products read).
-struct TLayer { int in, out; int w_off, b_off, t_off, a_off; };
-
 struct TDims {
     TLayer L[kLayers];
     int n_params, t_size, a_size;
@@ -46,13 +46,6 @@ struct TDims {
     int no_gs;                 // without the global state: attention.0's input is e (L[4].in = E1), not [e | mean]
     int wbuf_floats;           // size of one staging buffer = the largest block
 };
-
-__device__ __forceinline__ void cp_async16(float *dst_smem, const float *src)
-{
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" :: "n"(N) : "memory"); }
 
 // shared-memory plan (floats); every row stride is a multiple of 4 floats
 struct Plan {
@@ -112,12 +105,7 @@ __device__ __noinline__ void weight_grad_call(const float *dY, int ldy, const fl
 {
     weight_grad(dY, ldy, Xin, ldx, R, O, K, gW, gb);
 }
-__device__ __noinline__ void stage_block(float *dst, const float *src, int n)
-{
-#pragma unroll 4
-    for (int i = threadIdx.x * 4; i < n; i += kThreads * 4) cp_async16(dst + i, src + i);
-    cp_async_commit();
-}
+__device__ __noinline__ void stage_block(float *dst, const float *src, int n) { stage_async(dst, src, n); }
 
 __global__ void __launch_bounds__(kThreads, 1)
 trainer_fwd_bwd_kernel(TDims d, const float *__restrict__ Wt, const float *__restrict__ Wa, const float *__restrict__ X,
@@ -377,84 +365,176 @@ __global__ void trainer_transpose_kernel(int n_params, const float *__restrict__
 
 struct cn_trainer {
     int device;
+    int net;                                      // CN_NET_*: SARL runs trainer_fwd_bwd_kernel on d, the others trainer_nets.cu on nd
     TDims d;
+    NetDims nd;
+    int n_params;
     int max_batch, max_humans;
     float *Wt, *Wa, *mom, *gpart, *loss_part;     // transposed / aligned weight copies, momentum, per-CTA partials
     int32_t *tmap, *amap;                         // flat parameter index -> index in Wt / Wa (-1: not in Wa)
     int nparts_cap;
 };
 
+// The weight matrices of the flat block in state-dict order, from the layer list the lookahead loads (cn_layers): a Linear
+// is one TLayer, the LSTM block two (weight_ih with bias_ih, weight_hh with bias_hh).  Fills w_off / b_off / t_off / a_off;
+// returns the parameter count, *wbuf = the largest staged block.
+static int trainer_layers(const cn_sarl_cfg *cfg, std::vector<TLayer> &L, int *t_size, int *a_size, int *wbuf)
+{
+    SarlWeightsDev w;        // only the destinations of the layer list, never written here
+    int off = 0;
+    for (const LayerSpec &l : cn_layers(cn_dims_of(cfg, 0), w)) {
+        if (!l.dst_hh) {
+            L.push_back({l.in, l.out, off, off + l.in * l.out, 0, 0});
+        } else {                                          // weight_ih_l0, weight_hh_l0, bias_ih_l0, bias_hh_l0
+            const int hid = l.out / 4, whh = off + l.out * l.in, bih = whh + l.out * hid;
+            L.push_back({l.in, l.out, off, bih, 0, 0});
+            L.push_back({hid, l.out, whh, bih + l.out, 0, 0});
+        }
+        off += (int)cn_layer_floats(l);
+    }
+    int toff = 0, aoff = 0;
+    *wbuf = 0;
+    for (TLayer &l : L) {
+        l.t_off = toff; toff += pad4(l.in * l.out) + pad4(l.out);      // [in][out] | bias, 16-byte aligned blocks
+        l.a_off = aoff; aoff += pad4(l.in * l.out);                    // [out][in]
+        const int blk = pad4(l.in * l.out) + pad4(l.out);
+        if (blk > *wbuf) *wbuf = blk;
+    }
+    *t_size = toff; *a_size = aoff;
+    return off;
+}
+
+// CADRL / LSTM-RL: the layers and the order in which trainer_nets_fwd_bwd_kernel stages their blocks
+static void trainer_net_dims(const cn_sarl_cfg *cfg, const std::vector<TLayer> &L, NetDims &nd)
+{
+    nd.net = cfg->network;
+    nd.n_layers = (int)L.size();
+    for (int i = 0; i < nd.n_layers; ++i) nd.L[i] = L[i];
+    nd.in = cfg->input_dim; nd.self_dim = cfg->self_state_dim;
+    const bool lstm = cfg->network == CN_NET_LSTM_RL;
+    nd.vn2 = lstm && cfg->lstm_mlp1_dims[0] > 0;
+    nd.lstm_h = lstm ? cfg->lstm_hidden : 0;
+    nd.lstm_in = nd.vn2 ? cfg->lstm_mlp1_dims[3] : cfg->input_dim;
+    nd.mlp0 = nd.vn2 ? 4 : 0;
+    nd.ih = nd.mlp0 + 4; nd.hh = nd.mlp0 + 5;
+    int n = 0;
+    auto push = [&](int layer, int bwd) { nd.op_layer[n] = (int8_t)layer; nd.op_bwd[n] = (int8_t)bwd; ++n; };
+    if (lstm) {
+        if (nd.vn2) for (int i = 0; i < 4; ++i) push(i, 0);                 // mlp1
+        push(nd.ih, 0); push(nd.hh, 0);                                        // x W_ih^T, then W_hh^T for the recurrence
+    }
+    for (int i = 0; i < 4; ++i) push(nd.mlp0 + i, 0);                          // the value mlp
+    for (int i = 3; i >= (lstm ? 0 : 1); --i) push(nd.mlp0 + i, 1);            // its backward-data products (LSTM-RL: down to h_H)
+    if (lstm) {
+        push(nd.hh, 1);                                                        // BPTT
+        if (nd.vn2) { push(nd.ih, 1); for (int i = 3; i >= 1; --i) push(i, 1); }   // dx_t, then mlp1
+    }
+    nd.n_ops = n;
+}
+
 extern "C" {
 
 int cn_trainer_create(const cn_sarl_cfg *cfg, int device, int32_t max_batch, int32_t max_humans, cn_trainer **out)
 {
     if (!cfg || !out) { cn_set_error("null argument"); return CN_EINVAL; }
-    if (cfg->network != CN_NET_SARL || cfg->with_om) {
-        cn_set_error("the fused trainer covers the SARL value network without occupancy maps (with or without the global state); "
-                     "use torch autograd for the others");
-        return CN_EUNSUPPORTED;
+    const int net = cfg->network;
+    if (net != CN_NET_SARL && net != CN_NET_CADRL && net != CN_NET_LSTM_RL) { cn_set_error("unknown value network %d", net); return CN_EINVAL; }
+    if (cfg->without_global_state && net != CN_NET_SARL) {
+        cn_set_error("without_global_state is a [sarl] option; CADRL and LSTM-RL have no global state"); return CN_EINVAL;
     }
-    if (max_batch < 1 || max_humans < 1 || max_humans > kMaxH) { cn_set_error("1 <= max_humans <= %d, max_batch >= 1", kMaxH); return CN_EINVAL; }
+    if (cfg->with_om) {
+        if (net == CN_NET_CADRL) { cn_set_error("CADRL has no occupancy maps (cadrl.py:60-62)"); return CN_EINVAL; }
+        if (cfg->cell_num < 1 || cfg->cell_num > 8 || cfg->om_channel_size < 1 || cfg->om_channel_size > 3) {
+            cn_set_error("with_om needs 1 <= cell_num <= 8 and om_channel_size in {1, 2, 3}"); return CN_EINVAL;
+        }
+        const int om_in = 13 + cfg->cell_num * cfg->cell_num * cfg->om_channel_size;
+        if (cfg->input_dim != om_in) {
+            cn_set_error("with_om: input_dim %d must be 13 + cell_num^2 * om_channel_size = %d", cfg->input_dim, om_in); return CN_EINVAL;
+        }
+    }
+    if (max_batch < 1 || max_humans < 1 || (net == CN_NET_SARL && max_humans > kMaxH)) {
+        cn_set_error("1 <= max_humans <= %d, max_batch >= 1", kMaxH); return CN_EINVAL;
+    }
+    if (net == CN_NET_CADRL && max_humans != 1) {
+        cn_set_error("CADRL trains on single-human states (cadrl.py:209): max_humans must be 1"); return CN_EINVAL;
+    }
+    if (max_humans > kMaxH) {
+        cn_set_error("fused trainer: at most %d humans per sample (max_humans %d)", kMaxH, max_humans); return CN_EUNSUPPORTED;
+    }
+    if (net == CN_NET_LSTM_RL && cfg->lstm_hidden < 1) { cn_set_error("lstm_hidden >= 1 required"); return CN_EINVAL; }
+    if (net == CN_NET_LSTM_RL && (cfg->self_state_dim < 1 || cfg->self_state_dim > cfg->input_dim)) {
+        cn_set_error("1 <= self_state_dim <= input_dim required (the self state is the first columns of row 0)"); return CN_EINVAL;
+    }
+    std::vector<TLayer> L;
+    int t_size = 0, a_size = 0, wbuf = 0;
+    const int n_params = trainer_layers(cfg, L, &t_size, &a_size, &wbuf);
+    for (const TLayer &l : L)
+        if (l.in < 1 || l.out < 1) { cn_set_error("layer widths must be >= 1"); return CN_EINVAL; }
+    NetDims nd;
+    memset(&nd, 0, sizeof(nd));
+    size_t smem = 0;
+    int spc = kSPC;
+    if (net == CN_NET_SARL) {
+        if (cfg->attn_dims[2] != 1 || cfg->mlp3_dims[3] != 1) { cn_set_error("attention and mlp3 must end in 1 unit"); return CN_EINVAL; }
+    } else {
+        if (cfg->mlp3_dims[3] != 1) { cn_set_error("the value mlp must end in 1 unit"); return CN_EINVAL; }
+        trainer_net_dims(cfg, L, nd);
+        nd.n_params = n_params; nd.t_size = t_size; nd.a_size = a_size; nd.wbuf_floats = wbuf;
+        smem = trainer_nets_smem(nd, max_humans, 1);
+        spc = trainer_nets_spc(nd);
+    }
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) { cudaGetLastError(); cn_set_error("no CUDA device available; no CPU fallback"); return CN_ECUDA; }
     if (device < 0 || device >= n) { cn_set_error("device %d out of range", device); return CN_EINVAL; }
     CN_CUDA_CHECK(cudaSetDevice(device));
     cn_trainer *t = new cn_trainer();
     memset(t, 0, sizeof(*t));
-    t->device = device; t->max_batch = max_batch; t->max_humans = max_humans;
+    t->device = device; t->net = net; t->max_batch = max_batch; t->max_humans = max_humans;
+    t->n_params = n_params;
+    t->nd = nd;
     TDims &d = t->d;
-    const int att_in = cfg->without_global_state ? cfg->mlp1_dims[1] : 2 * cfg->mlp1_dims[1];
-    const int ins[kLayers] = {cfg->input_dim, cfg->mlp1_dims[0], cfg->mlp1_dims[1], cfg->mlp2_dims[0], att_in,
-                              cfg->attn_dims[0], cfg->attn_dims[1], cfg->mlp2_dims[1] + cfg->self_state_dim, cfg->mlp3_dims[0],
-                              cfg->mlp3_dims[1], cfg->mlp3_dims[2]};
-    const int outs[kLayers] = {cfg->mlp1_dims[0], cfg->mlp1_dims[1], cfg->mlp2_dims[0], cfg->mlp2_dims[1], cfg->attn_dims[0],
-                               cfg->attn_dims[1], cfg->attn_dims[2], cfg->mlp3_dims[0], cfg->mlp3_dims[1], cfg->mlp3_dims[2],
-                               cfg->mlp3_dims[3]};
-    int off = 0, toff = 0, aoff = 0, wbuf = 0;
-    for (int i = 0; i < kLayers; ++i) {
-        d.L[i].in = ins[i]; d.L[i].out = outs[i];
-        d.L[i].w_off = off; off += ins[i] * outs[i];
-        d.L[i].b_off = off; off += outs[i];
-        d.L[i].t_off = toff; toff += pad4(ins[i] * outs[i]) + pad4(outs[i]);      // [in][out] | bias, 16-byte aligned blocks
-        d.L[i].a_off = aoff; aoff += pad4(ins[i] * outs[i]);                      // [out][in]
-        const int blk = pad4(ins[i] * outs[i]) + pad4(outs[i]);
-        if (blk > wbuf) wbuf = blk;
+    if (net == CN_NET_SARL) {
+        for (int i = 0; i < kLayers; ++i) d.L[i] = L[i];
+        d.n_params = n_params; d.t_size = t_size; d.a_size = a_size; d.wbuf_floats = wbuf;
+        d.in = cfg->input_dim; d.self_dim = cfg->self_state_dim; d.no_gs = cfg->without_global_state ? 1 : 0;
+        smem = sizeof(float) * ((size_t)pad4(make_plan(d, max_humans, kSPC).total) + wbuf);
     }
-    d.n_params = off; d.t_size = toff; d.a_size = aoff; d.wbuf_floats = wbuf;
-    d.in = cfg->input_dim; d.self_dim = cfg->self_state_dim; d.no_gs = cfg->without_global_state ? 1 : 0;
-    if (outs[6] != 1 || outs[10] != 1) { delete t; cn_set_error("attention and mlp3 must end in 1 unit"); return CN_EINVAL; }
-    std::vector<int32_t> tmap(d.n_params), amap(d.n_params, -1);
-    for (int i = 0; i < kLayers; ++i) {
-        for (int o = 0; o < outs[i]; ++o)
-            for (int k = 0; k < ins[i]; ++k) {
-                tmap[d.L[i].w_off + o * ins[i] + k] = d.L[i].t_off + k * outs[i] + o;
-                amap[d.L[i].w_off + o * ins[i] + k] = d.L[i].a_off + o * ins[i] + k;
+    std::vector<int32_t> tmap(n_params), amap(n_params, -1);
+    for (const TLayer &l : L) {
+        for (int o = 0; o < l.out; ++o)
+            for (int k = 0; k < l.in; ++k) {
+                tmap[l.w_off + o * l.in + k] = l.t_off + k * l.out + o;
+                amap[l.w_off + o * l.in + k] = l.a_off + o * l.in + k;
             }
-        for (int o = 0; o < outs[i]; ++o) tmap[d.L[i].b_off + o] = d.L[i].t_off + pad4(ins[i] * outs[i]) + o;
+        for (int o = 0; o < l.out; ++o) tmap[l.b_off + o] = l.t_off + pad4(l.in * l.out) + o;
     }
-    t->nparts_cap = (max_batch + kSPC - 1) / kSPC;
-    const Plan pl = make_plan(d, max_humans, kSPC);
-    if (sizeof(float) * ((size_t)pad4(pl.total) + wbuf) > 232448) {
-        delete t; cn_set_error("fused trainer: %d humans per sample do not fit the shared-memory plan", max_humans); return CN_EUNSUPPORTED;
+    t->nparts_cap = (max_batch + spc - 1) / spc;
+    if (smem > 232448) {
+        delete t;
+        cn_set_error("fused trainer: %d humans per sample%s do not fit the shared-memory plan", max_humans,
+                     net == CN_NET_LSTM_RL ? " at this lstm_hidden / layer widths" : "");
+        return CN_EUNSUPPORTED;
     }
-    if (cudaMalloc((void **)&t->Wt, sizeof(float) * d.t_size) != cudaSuccess ||
-        cudaMalloc((void **)&t->Wa, sizeof(float) * d.a_size) != cudaSuccess ||
-        cudaMalloc((void **)&t->mom, sizeof(float) * d.n_params) != cudaSuccess ||
-        cudaMalloc((void **)&t->gpart, sizeof(float) * (size_t)d.n_params * t->nparts_cap) != cudaSuccess ||
+    if (cudaMalloc((void **)&t->Wt, sizeof(float) * t_size) != cudaSuccess ||
+        cudaMalloc((void **)&t->Wa, sizeof(float) * a_size) != cudaSuccess ||
+        cudaMalloc((void **)&t->mom, sizeof(float) * n_params) != cudaSuccess ||
+        cudaMalloc((void **)&t->gpart, sizeof(float) * (size_t)n_params * t->nparts_cap) != cudaSuccess ||
         cudaMalloc((void **)&t->loss_part, sizeof(float) * t->nparts_cap) != cudaSuccess ||
-        cudaMalloc((void **)&t->tmap, sizeof(int32_t) * d.n_params) != cudaSuccess ||
-        cudaMalloc((void **)&t->amap, sizeof(int32_t) * d.n_params) != cudaSuccess) {
+        cudaMalloc((void **)&t->tmap, sizeof(int32_t) * n_params) != cudaSuccess ||
+        cudaMalloc((void **)&t->amap, sizeof(int32_t) * n_params) != cudaSuccess) {
         cn_set_error("cudaMalloc failed in cn_trainer_create");
         cn_trainer_destroy(t);
         return CN_ENOMEM;
     }
     // (the padding floats of the blocks are read by cp.async, hence the memsets)
-    cudaError_t ce = cudaMemset(t->Wt, 0, sizeof(float) * d.t_size);
-    if (ce == cudaSuccess) ce = cudaMemset(t->Wa, 0, sizeof(float) * d.a_size);
-    if (ce == cudaSuccess) ce = cudaMemset(t->mom, 0, sizeof(float) * d.n_params);
-    if (ce == cudaSuccess) ce = cudaMemcpy(t->tmap, tmap.data(), sizeof(int32_t) * d.n_params, cudaMemcpyHostToDevice);
-    if (ce == cudaSuccess) ce = cudaMemcpy(t->amap, amap.data(), sizeof(int32_t) * d.n_params, cudaMemcpyHostToDevice);
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(trainer_fwd_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+    cudaError_t ce = cudaMemset(t->Wt, 0, sizeof(float) * t_size);
+    if (ce == cudaSuccess) ce = cudaMemset(t->Wa, 0, sizeof(float) * a_size);
+    if (ce == cudaSuccess) ce = cudaMemset(t->mom, 0, sizeof(float) * n_params);
+    if (ce == cudaSuccess) ce = cudaMemcpy(t->tmap, tmap.data(), sizeof(int32_t) * n_params, cudaMemcpyHostToDevice);
+    if (ce == cudaSuccess) ce = cudaMemcpy(t->amap, amap.data(), sizeof(int32_t) * n_params, cudaMemcpyHostToDevice);
+    if (ce == cudaSuccess)
+        ce = net == CN_NET_SARL ? cudaFuncSetAttribute(trainer_fwd_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448)
+                                : trainer_nets_configure();
     if (ce != cudaSuccess) {
         cn_set_error("cn_trainer_create: %s", cudaGetErrorString(ce));
         cn_trainer_destroy(t);
@@ -474,14 +554,14 @@ int cn_trainer_destroy(cn_trainer *t)
     return CN_OK;
 }
 
-int64_t cn_trainer_param_count(const cn_trainer *t) { return t ? t->d.n_params : 0; }
+int64_t cn_trainer_param_count(const cn_trainer *t) { return t ? t->n_params : 0; }
 
 int cn_trainer_sync_weights(cn_trainer *t, const float *w_dev, int zero_momentum, void *stream)
 {
     if (!t || !w_dev) { cn_set_error("null argument"); return CN_EINVAL; }
     CN_CUDA_CHECK(cudaSetDevice(t->device));
     cudaStream_t s = (cudaStream_t)stream;
-    const int n = t->d.n_params;
+    const int n = t->n_params;
     trainer_transpose_kernel<<<(n + 255) / 256, 256, 0, s>>>(n, w_dev, t->Wt, t->Wa, t->tmap, t->amap);
     CN_LAUNCH_CHECK();
     if (zero_momentum) CN_CUDA_CHECK(cudaMemsetAsync(t->mom, 0, sizeof(float) * n, s));
@@ -493,22 +573,31 @@ static int trainer_step_impl(cn_trainer *t, float *w_dev, const float *states_de
                              float *grad_out_dev, float *loss_dev, int loss_accumulate, void *stream)
 {
     if (!t || !w_dev || !states_dev || !targets_dev) { cn_set_error("null argument"); return CN_EINVAL; }
+    if (t->net == CN_NET_CADRL && human_num != 1) {
+        cn_set_error("CADRL trains on single-human states (cadrl.py:209): human_num must be 1, got %d", human_num); return CN_EINVAL;
+    }
     if (batch < 1 || batch > t->max_batch || human_num < 1 || human_num > t->max_humans) {
         cn_set_error("batch %d / human_num %d outside the trainer's capacity (%d, %d)", batch, human_num, t->max_batch, t->max_humans);
         return CN_EINVAL;
     }
     CN_CUDA_CHECK(cudaSetDevice(t->device));
     cudaStream_t s = (cudaStream_t)stream;
-    const int nparts = (batch + kSPC - 1) / kSPC;
-    const Plan pl = make_plan(t->d, human_num, kSPC);
-    // two staging buffers (the next weight block is copied while the current layer computes) when they fit, else one
-    const size_t act = (size_t)pad4(pl.total);
-    const int nbuf = sizeof(float) * (act + 2 * (size_t)t->d.wbuf_floats) <= 232448 ? 2 : 1;
-    const size_t smem = sizeof(float) * (act + (size_t)nbuf * t->d.wbuf_floats);
-    trainer_fwd_bwd_kernel<<<nparts, kThreads, smem, s>>>(t->d, t->Wt, t->Wa, states_dev, targets_dev, index_dev, batch, human_num,
-                                                         nbuf, t->gpart, t->loss_part);
-    CN_LAUNCH_CHECK();
-    const int n = t->d.n_params;
+    int nparts = (batch + kSPC - 1) / kSPC;
+    if (t->net == CN_NET_SARL) {
+        const Plan pl = make_plan(t->d, human_num, kSPC);
+        // two staging buffers (the next weight block is copied while the current layer computes) when they fit, else one
+        const size_t act = (size_t)pad4(pl.total);
+        const int nbuf = sizeof(float) * (act + 2 * (size_t)t->d.wbuf_floats) <= 232448 ? 2 : 1;
+        const size_t smem = sizeof(float) * (act + (size_t)nbuf * t->d.wbuf_floats);
+        trainer_fwd_bwd_kernel<<<nparts, kThreads, smem, s>>>(t->d, t->Wt, t->Wa, states_dev, targets_dev, index_dev, batch,
+                                                             human_num, nbuf, t->gpart, t->loss_part);
+        CN_LAUNCH_CHECK();
+    } else {
+        const int rc = trainer_nets_launch(t->nd, t->Wt, t->Wa, states_dev, targets_dev, index_dev, batch, human_num, t->gpart,
+                                           t->loss_part, &nparts, s);
+        if (rc != CN_OK) return rc;
+    }
+    const int n = t->n_params;
     trainer_reduce_kernel<<<(n + 255) / 256, 256, 0, s>>>(n, nparts, t->gpart, t->loss_part, batch, grad_out_dev, w_dev, t->Wt, t->Wa,
                                                          t->mom, t->tmap, t->amap, lr, momentum, loss_dev, loss_accumulate);
     CN_LAUNCH_CHECK();
@@ -535,7 +624,7 @@ int cn_trainer_apply(cn_trainer *t, float *w_dev, const float *grad_dev, float g
 {
     if (!t || !w_dev || !grad_dev) { cn_set_error("null argument"); return CN_EINVAL; }
     CN_CUDA_CHECK(cudaSetDevice(t->device));
-    const int n = t->d.n_params;
+    const int n = t->n_params;
     trainer_apply_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(n, grad_dev, grad_scale, w_dev, t->Wt, t->Wa, t->mom, t->tmap,
                                                                           t->amap, lr, momentum);
     CN_LAUNCH_CHECK();

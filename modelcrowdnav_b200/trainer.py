@@ -3,9 +3,10 @@
 Batches are drawn directly from the device-resident replay tensors instead of a DataLoader over Python tuples.
 Three execution forms of the same optimisation step (MSE -> backward -> [gradient all-reduce] -> SGD momentum):
 
-* ``fused``  (CUDA, SARL value network): the hand-written forward / backward kernel + SGD kernel of the C ABI
-  (``cn_trainer_*``, csrc/trainer.cu) working on ONE flat fp32 parameter block that the torch model's parameters are
-  views of; the gradient all-reduce (NCCL, one 386 kB bucket) sits between the two kernels.
+* ``fused``  (CUDA; SARL and OM-SARL with or without the global state, CADRL, LSTM-RL ValueNetwork1 / 2 with or without
+  occupancy maps): the hand-written forward / backward kernel + SGD kernel of the C ABI (``cn_trainer_*``,
+  csrc/trainer.cu, csrc/trainer_nets.cu) working on ONE flat fp32 parameter block that the torch model's parameters are
+  views of; the gradient all-reduce (NCCL, one bucket: 386 kB for SARL) sits between the two kernels.
 * ``graph``  (CUDA, any network): torch autograd captured once per batch shape into a CUDA graph and replayed.
 * ``eager``  (CPU / gloo tests, odd batch sizes): plain torch autograd.
 
@@ -70,9 +71,9 @@ class Trainer(object):
         logging.info("Current learning rate: %f", learning_rate)
         self.lr = float(learning_rate)
         if self.mode == "fused":
-            from .fused_trainer import FusedSarlTrainer
+            from .fused_trainer import FusedTrainer
             if self._fused is None:
-                self._fused = FusedSarlTrainer(self.model, self.device, momentum=self.momentum)
+                self._fused = FusedTrainer(self.model, self.device, momentum=self.momentum)
             self._fused.lr = self.lr
             self.optimizer = self._fused          # "Learning rate is not set!" check below
             return
@@ -211,9 +212,13 @@ class Trainer(object):
 
     def _fused_indexed_ok(self):
         m = self.memory
-        return (self.mode == "fused" and getattr(m, "states", None) is not None and m.states.is_cuda and m.states.dim() == 3
-                and m.states.dtype == torch.float32 and m.values.dtype == torch.float32 and m.states.is_contiguous()
-                and m.values.is_contiguous() and m.states.shape[1] <= self._fused.max_humans)
+        if self.mode != "fused" or getattr(m, "states", None) is None:
+            return False
+        # (capacity, H, D) replay tensors; CADRL's single-human states are (capacity, D)
+        shape_ok = m.states.dim() == 2 if self._fused.single_human else (
+            m.states.dim() == 3 and m.states.shape[1] <= self._fused.max_humans)
+        return (shape_ok and m.states.is_cuda and m.states.dtype == torch.float32 and m.values.dtype == torch.float32
+                and m.states.is_contiguous() and m.values.is_contiguous())
 
     def _after(self):
         if self._fused is not None:
