@@ -105,7 +105,10 @@ typedef struct {
      * false only, see multi_human_rl.py:37-42), nn.LSTM(13 or lstm_mlp1_dims[3] -> lstm_hidden) over the rows, mlp3_dims =
      * [lstm_rl] mlp2_dims on cat(self_state, h_n); lstm_mlp1_dims[0] > 0 selects ValueNetwork2 (with_interaction_module).
      * Both run on either precision: CN_PREC_F16_TC takes the reference's default shapes (CADRL mlp_dims 150,100,100,1; LSTM-RL
-     * without interaction module / occupancy maps, lstm_hidden 50, mlp2_dims 150,100,100,1), CN_PREC_F32 any shape. */
+     * without interaction module / occupancy maps, lstm_hidden 50, mlp2_dims 150,100,100,1), CN_PREC_F32 any shape whose
+     * activations for one action (one sample in cn_policy_forward) fit a CTA's shared memory: H rows of every layer width,
+     * so all-256 SARL layers with 8 x 8 x 3 maps at 64 humans return CN_EUNSUPPORTED from the lookahead and the forward.
+     * Narrower plans take fewer actions per CTA instead. */
     int32_t network;             /* CN_NET_* */
     int32_t lstm_hidden;         /* [lstm_rl] global_state_dim = 50 */
     int32_t lstm_mlp1_dims[4];   /* [lstm_rl] mlp1_dims = 150,100,100,50; {0} = ValueNetwork1 */

@@ -196,6 +196,8 @@ def default_sarl_cfg(**kw):
             raise AttributeError("cn_sarl_cfg has no field %r" % k)
         if isinstance(v, (list, tuple)):
             arr = getattr(cfg, k)
+            if len(v) != len(arr):
+                raise ValueError("cn_sarl_cfg.%s holds %d values, got %d" % (k, len(arr), len(v)))
             for i, x in enumerate(v):
                 arr[i] = x
         else:

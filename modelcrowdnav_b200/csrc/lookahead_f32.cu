@@ -448,25 +448,29 @@ __global__ void transform_kernel(EnvParams p, SarlDims nd, const double *__restr
     s[9] = ag(F_PX, h + 1); s[10] = ag(F_PY, h + 1); s[11] = ag(F_VX, h + 1); s[12] = ag(F_VY, h + 1);
     s[13] = ag(F_R, h + 1);
     cn_rotate(s, o, p.kinematics);
-    int pos = h;
-    if (sort_humans) {
-        const double rx = st[st_idx(d, F_PX, 0, e)], ry = st[st_idx(d, F_PY, 0, e)];
-        const double dh = norm2d(st[st_idx(d, F_PX, h + 1, e)] - rx, st[st_idx(d, F_PY, h + 1, e)] - ry);
-        pos = 0;
-        for (int k = 0; k < d.H; ++k) {
-            if (k == h) continue;
-            const double dk = norm2d(st[st_idx(d, F_PX, k + 1, e)] - rx, st[st_idx(d, F_PY, k + 1, e)] - ry);
-            pos += (dk > dh || (dk == dh && k < h)) ? 1 : 0;
-        }
-    }
+    const double rx = st[st_idx(d, F_PX, 0, e)], ry = st[st_idx(d, F_PY, 0, e)];
+    auto dist = [&](int k) { return norm2d(st[st_idx(d, F_PX, k + 1, e)] - rx, st[st_idx(d, F_PY, k + 1, e)] - ry); };
+    auto rank = [&](int k) {                 // position of human k in the sorted order
+        if (!sort_humans) return k;
+        const double dh = dist(k);
+        int r = 0;
+        for (int j = 0; j < d.H; ++j)
+            if (j != k) { const double dj = dist(j); r += (dj > dh || (dj == dh && j < k)) ? 1 : 0; }
+        return r;
+    };
+    const int pos = rank(h);
     const int D = 13 + nd.om_dim;
     float *row = out + ((size_t)e * d.H + pos) * D;
     for (int k = 0; k < 13; ++k) row[k] = o[k];
-    // with_om (multi_human_rl.py:98-101): map of the CURRENT human states around this human.  The others are visited in env
-    // order; for a sorted last_state the reference visits them in sorted order, which only permutes a float64 sum.
-    if (nd.om_dim > 0)
-        occupancy_map_row(nd, d.H, h, [&](int j, int f) { return st[st_idx(d, f == 0 ? F_PX : f == 1 ? F_PY : f == 2 ? F_VX : F_VY, j + 1, e)]; },
-                          row + 13);
+    // with_om (multi_human_rl.py:98-101): map of the CURRENT human states around this human, the others visited in the order
+    // of the human list the reference builds it from -- sorted for a sorted last_state (lstm_rl.py:99-105).  The order of the
+    // float64 velocity sums can change a mean's float32 rounding.
+    if (nd.om_dim > 0) {
+        int ord[CN_MAX_HUMANS];
+        for (int k = 0; k < d.H; ++k) ord[rank(k)] = k;
+        occupancy_map_row(nd, d.H, pos, [&](int j, int f) {
+            return st[st_idx(d, f == 0 ? F_PX : f == 1 ? F_PY : f == 2 ? F_VX : F_VY, ord[j] + 1, e)]; }, row + 13);
+    }
 }
 
 // ValueNetwork.forward on a device batch (B x H x 13 -> B); grid = chunks of CA items
@@ -489,13 +493,11 @@ forward_kernel(SarlWeightsDev W, SarlDims d, F32Plan pl, const float *__restrict
     for (int i = threadIdx.x; i < nb; i += blockDim.x) out[b0 + i] = Vv[i];
 }
 
-F32Plan make_plan(const SarlDims &d, int H, int A, int A1)
+F32Plan plan_for(const SarlDims &d, int H, int A, int A1, int CA)
 {
     F32Plan pl;
     pl.H = H; pl.A = A;
-    pl.CA = kRowsCap / H;
-    if (pl.CA < 1) pl.CA = 1;
-    if (pl.CA > A) pl.CA = A;
+    pl.CA = CA;
     const int rows = pl.CA * H;
     auto mx = [](int a, int b) { return a > b ? a : b; };
     pl.wX = d.in <= 16 ? 16 : pad4(d.in);          // 13 rotated features (+ occupancy map)
@@ -524,6 +526,18 @@ F32Plan make_plan(const SarlDims &d, int H, int A, int A1)
     pl.oOrd = o; o += pad4(H);                      // LSTM-RL: humans in network order
     pl.oOm = o; o += pad4(H * d.om_dim);            // with_om: one map per human
     pl.total_floats = o;
+    return pl;
+}
+
+// kRowsCap rows per CTA (CA actions or samples of H rows each); layers too wide for that many rows in shared memory get
+// fewer actions per CTA, down to one.  A plan that still does not fit is refused by the caller.
+F32Plan make_plan(const SarlDims &d, int H, int A, int A1)
+{
+    int ca = kRowsCap / H;
+    if (ca < 1) ca = 1;
+    if (ca > A) ca = A;
+    F32Plan pl = plan_for(d, H, A, A1, ca);
+    while (ca > 1 && sizeof(float) * (size_t)pl.total_floats > kMaxDynSmem) pl = plan_for(d, H, A, A1, --ca);
     return pl;
 }
 

@@ -191,6 +191,12 @@ def make_value_network(input_dim, self_state_dim, mlp1_dims, mlp2_dims, mlp3_dim
     return ValueNetwork()
 
 
+# [sarl] keys of the layer widths and how many layers each has (sarl.py:28-35); the last attention and mlp3 layer has 1 unit
+SARL_DIM_LENGTHS = dict(mlp1_dims=2, mlp2_dims=2, attention_dims=3, mlp3_dims=4)
+# the only widths the tensor-core lookahead is specialised for (lookahead_tc.cu, cn_tc_init)
+SARL_TC_DIMS = dict(mlp1_dims=[150, 100], mlp2_dims=[100, 50], attn_dims=[100, 100, 1], mlp3_dims=[150, 100, 100, 1])
+
+
 class SARL(Policy):
     """SARL with the MultiHumanRL lookahead on the GPU (sarl.py:68-89, multi_human_rl.py:11-104)."""
 
@@ -239,14 +245,21 @@ class SARL(Policy):
         self.set_common_parameters(config)
         if self.kinematics not in KIN_CODE:
             raise NotImplementedError("kinematics must be holonomic, unicycle or None (the fork's literal behaviour)")
-        mlp1_dims = [int(x) for x in config.get("sarl", "mlp1_dims").split(", ")]
-        mlp2_dims = [int(x) for x in config.get("sarl", "mlp2_dims").split(", ")]
-        mlp3_dims = [int(x) for x in config.get("sarl", "mlp3_dims").split(", ")]
-        attention_dims = [int(x) for x in config.get("sarl", "attention_dims").split(", ")]
+        dims = {}
+        for key, n in SARL_DIM_LENGTHS.items():
+            dims[key] = [int(x) for x in config.get("sarl", key).split(", ")]
+            if len(dims[key]) != n:
+                raise ValueError("[sarl] %s needs %d layer widths, got %d" % (key, n, len(dims[key])))
+        for key in ("attention_dims", "mlp3_dims"):
+            if dims[key][-1] != 1:
+                raise ValueError("[sarl] %s must end in 1 unit" % key)
+        mlp1_dims, mlp2_dims, mlp3_dims, attention_dims = (dims[k] for k in ("mlp1_dims", "mlp2_dims", "mlp3_dims",
+                                                                              "attention_dims"))
         self.with_om = config.getboolean("sarl", "with_om")
         with_global_state = config.getboolean("sarl", "with_global_state")
         self._dims = dict(mlp1_dims=mlp1_dims, mlp2_dims=mlp2_dims, attn_dims=attention_dims, mlp3_dims=mlp3_dims)
         self._net_kwargs = dict(self._dims, **self._om_kwargs())
+        self.precision = "f16_tc" if self._tc_shape() else "f32"
         if not with_global_state:
             self._net_kwargs["without_global_state"] = 1
         self.model = make_value_network(self.input_dim(), self.self_state_dim, mlp1_dims, mlp2_dims, mlp3_dims,
@@ -368,6 +381,11 @@ class SARL(Policy):
         """multi_human_rl.py:106-107"""
         return self.joint_state_dim + (self.cell_num ** 2 * self.om_channel_size if self.with_om else 0)
 
+    def _tc_shape(self):
+        """Whether cn_tc_init runs this SARL on the tensor cores: the default [sarl] widths, with or without the global state
+        and with any [om] setting.  Every other shape runs on the FP32 kernels."""
+        return self._dims == SARL_TC_DIMS and self.self_state_dim == 6
+
     def _om_kwargs(self):
         """cn_sarl_cfg fields of the occupancy maps.  OM-SARL keeps the tensor-core lookahead (the map enters mlp1.0 as a row
         bias per human, tc_om_bias_kernel); OM-LSTM-RL is FP32 like LSTM-RL itself."""
@@ -396,7 +414,7 @@ def make_cadrl_network(input_dim, mlp_dims):
 
 def make_lstm_network(input_dim, self_state_dim, mlp1_dims, mlp_dims, lstm_hidden_dim):
     """torch ValueNetwork1 (mlp1_dims None) / ValueNetwork2 of LSTM-RL with the reference's parameter names and
-    registration order (lstm_rl.py:9-66); the initial LSTM state follows the input's device."""
+    registration order (lstm_rl.py:9-66); the initial LSTM state follows the input's device and dtype."""
     import torch
     import torch.nn as nn
 
@@ -416,8 +434,8 @@ def make_lstm_network(input_dim, self_state_dim, mlp1_dims, mlp_dims, lstm_hidde
             seq = state
             if mlp1_dims:
                 seq = self.mlp1(state.reshape((-1, size[2]))).reshape((size[0], size[1], -1))
-            h0 = torch.zeros(1, size[0], self.lstm_hidden_dim, device=state.device)
-            c0 = torch.zeros(1, size[0], self.lstm_hidden_dim, device=state.device)
+            h0 = torch.zeros(1, size[0], self.lstm_hidden_dim, device=state.device, dtype=state.dtype)
+            c0 = torch.zeros(1, size[0], self.lstm_hidden_dim, device=state.device, dtype=state.dtype)
             _, (hn, _) = self.lstm(seq, (h0, c0))
             return self.mlp(torch.cat([self_state, hn.squeeze(0)], dim=1))
 

@@ -65,8 +65,8 @@ class TrainingLoop(object):
         torch.manual_seed(seed)
         self.policy = policy = mcn.policy_factory[policy_name]()
         policy.configure(policy_config)
-        if policy_name == "sarl" and not policy.with_om:
-            policy.precision = precision          # CADRL, LSTM-RL and occupancy maps run on the FP32 path
+        if policy.precision == "f16_tc":
+            policy.precision = precision          # configure() chose FP32 for the shapes the tensor cores do not run
         policy.set_device(device)
         self.env = env = mcn.CrowdSim()
         env.configure(env_config)
