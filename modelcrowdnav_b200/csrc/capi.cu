@@ -81,6 +81,44 @@ std::vector<LayerSpec> cn_layers(const SarlDims &d, SarlWeightsDev &w)
     return L;
 }
 
+// ---- checks shared by the entry points (declared in cn_common.cuh) ---------------------------------
+int use_device(int device)
+{
+    int n = 0;
+    cudaError_t e = cudaGetDeviceCount(&n);
+    if (e != cudaSuccess || n == 0) {
+        cudaGetLastError();
+        cn_set_error("no CUDA device available (%s); libcrowdnav_b200 has no CPU fallback",
+                     e != cudaSuccess ? cudaGetErrorString(e) : "device count 0");
+        return CN_ECUDA;
+    }
+    if (device < 0 || device >= n) { cn_set_error("device %d out of range (0..%d)", device, n - 1); return CN_EINVAL; }
+    CN_CUDA_CHECK(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    CN_CUDA_CHECK(cudaGetDeviceProperties(&prop, device));
+    if (prop.major != 10) {
+        cn_set_error("device %d is sm_%d%d; this library is built for sm_100a only", device, prop.major, prop.minor);
+        return CN_ECUDA;
+    }
+    return CN_OK;
+}
+
+int cn_check_net_cfg(const cn_sarl_cfg *cfg)
+{
+    const int net = cfg->network;
+    if (net != CN_NET_SARL && net != CN_NET_CADRL && net != CN_NET_LSTM_RL) { cn_set_error("unknown value network %d", net); return CN_EINVAL; }
+    if (cfg->without_global_state && net != CN_NET_SARL) {
+        cn_set_error("without_global_state is a [sarl] option; CADRL and LSTM-RL have no global state"); return CN_EINVAL;
+    }
+    if (cfg->with_om) {
+        if (net == CN_NET_CADRL) { cn_set_error("CADRL has no occupancy maps (cadrl.py:60-62)"); return CN_EINVAL; }
+        if (cfg->cell_num < 1 || cfg->cell_num > 8 || cfg->om_channel_size < 1 || cfg->om_channel_size > 3 || !(cfg->cell_size > 0)) {
+            cn_set_error("with_om needs 1 <= cell_num <= 8, om_channel_size in {1, 2, 3} and cell_size > 0"); return CN_EINVAL;
+        }
+    }
+    return CN_OK;
+}
+
 extern "C" {
 
 /* Developer diagnostic: on = 1 starts recording a timeline of the library's stream operations (one CUDA event per mark),
@@ -148,27 +186,6 @@ void cn_sarl_cfg_default(cn_sarl_cfg *c)
     c->kinematics = CN_KIN_HOLONOMIC;
     c->network = CN_NET_SARL; c->lstm_hidden = 50;      // [lstm_rl] global_state_dim; lstm_mlp1_dims = {0}: ValueNetwork1
     c->with_om = 0; c->cell_num = 4; c->cell_size = 1.0; c->om_channel_size = 3;   // [om]
-}
-
-static int use_device(int device)
-{
-    int n = 0;
-    cudaError_t e = cudaGetDeviceCount(&n);
-    if (e != cudaSuccess || n == 0) {
-        cudaGetLastError();
-        cn_set_error("no CUDA device available (%s); libcrowdnav_b200 has no CPU fallback",
-                     e != cudaSuccess ? cudaGetErrorString(e) : "device count 0");
-        return CN_ECUDA;
-    }
-    if (device < 0 || device >= n) { cn_set_error("device %d out of range (0..%d)", device, n - 1); return CN_EINVAL; }
-    CN_CUDA_CHECK(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    CN_CUDA_CHECK(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) {
-        cn_set_error("device %d is sm_%d%d; this library is built for sm_100a only", device, prop.major, prop.minor);
-        return CN_ECUDA;
-    }
-    return CN_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -539,12 +556,9 @@ int cn_policy_create(const cn_sarl_cfg *cfg, int device, cn_policy **out)
     if (!cfg || !out) { cn_set_error("null argument"); return CN_EINVAL; }
     const int A = cfg->speed_samples * cfg->rotation_samples + 1;
     int om_dim = 0;
+    int rc = cn_check_net_cfg(cfg);
+    if (rc) return rc;
     if (cfg->with_om) {
-        if (cfg->cell_num < 1 || cfg->cell_num > 8 || cfg->om_channel_size < 1 || cfg->om_channel_size > 3 || !(cfg->cell_size > 0)) {
-            cn_set_error("with_om needs 1 <= cell_num <= 8, om_channel_size in {1, 2, 3} and cell_size > 0");
-            return CN_EINVAL;
-        }
-        if (cfg->network == CN_NET_CADRL) { cn_set_error("CADRL has no occupancy maps (cadrl.py:60-62)"); return CN_EINVAL; }
         if (cfg->precision != CN_PREC_F32 && cfg->network != CN_NET_SARL) {
             cn_set_error("occupancy maps on the tensor-core path are built for SARL only; use CN_PREC_F32"); return CN_EUNSUPPORTED;
         }
@@ -555,12 +569,6 @@ int cn_policy_create(const cn_sarl_cfg *cfg, int device, cn_policy **out)
         return CN_EUNSUPPORTED;
     }
     if (cfg->attn_dims[2] != 1 || cfg->mlp3_dims[3] != 1) { cn_set_error("attention and mlp3 must end in 1 unit"); return CN_EINVAL; }
-    if (cfg->network != CN_NET_SARL && cfg->network != CN_NET_CADRL && cfg->network != CN_NET_LSTM_RL) {
-        cn_set_error("unknown value network %d", cfg->network); return CN_EINVAL;
-    }
-    if (cfg->without_global_state && cfg->network != CN_NET_SARL) {
-        cn_set_error("without_global_state is a [sarl] option; CADRL and LSTM-RL have no global state"); return CN_EINVAL;
-    }
     if (cfg->network == CN_NET_LSTM_RL) {
         if (cfg->lstm_hidden < 1 || cfg->lstm_hidden > 64) { cn_set_error("1 <= lstm_hidden <= 64 required"); return CN_EINVAL; }
         if (cfg->lstm_mlp1_dims[0] > 0)
@@ -572,8 +580,7 @@ int cn_policy_create(const cn_sarl_cfg *cfg, int device, cn_policy **out)
                         cfg->attn_dims[1], cfg->mlp3_dims[0], cfg->mlp3_dims[1], cfg->mlp3_dims[2]};
     for (int v : dims) if (v < 1 || v > 256) { cn_set_error("layer widths must be in [1, 256]"); return CN_EINVAL; }
     if (cfg->precision != CN_PREC_F32 && cfg->precision != CN_PREC_F16_TC) { cn_set_error("unknown precision"); return CN_EINVAL; }
-    int rc = use_device(device);
-    if (rc) return rc;
+    if ((rc = use_device(device))) return rc;
     if ((rc = cn_f32_configure_device())) return rc;
 
     cn_policy *p = new cn_policy();

@@ -324,6 +324,12 @@ __device__ __forceinline__ void cn_effective_velocity(int kinematics, double the
 __host__ __device__ __forceinline__ double norm2d(double a, double b) { return sqrt(fma(b, b, a * a)); }
 
 // ---- module entry points (each .cu) -----------------------------------------------------------
+// Makes `device` current after checking that it exists and is an sm_100 part: CN_ECUDA (no device, or another architecture)
+// or CN_EINVAL (out of range) with a message otherwise (capi.cu).
+int use_device(int device);
+// The checks every entry point that takes a network configuration makes with CN_EINVAL: a known network, the global-state
+// switch on SARL only, and occupancy maps of a valid shape on a network that has them (capi.cu).
+int cn_check_net_cfg(const cn_sarl_cfg *cfg);
 int cn_launch_orca(cn_env *env, cudaStream_t s);
 int cn_launch_robot_orca(cn_env *env, double safety_space, cudaStream_t s);
 int cn_launch_step(cn_env *env, const double *action_xy_dev, int update, cudaStream_t s, int fuse_reset = 0);

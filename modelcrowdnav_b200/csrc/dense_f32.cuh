@@ -1,5 +1,5 @@
 // dense_f32.cuh -- FP32 CUDA-core building blocks of the small dense layers that run OUTSIDE the tensor-core lookahead
-// (the fused trainer, trainer.cu, and the world models, world_model.cu): activations in shared memory, weights streamed
+// (the fused trainer, trainer_nets.cu, and the world models, world_model.cu): activations in shared memory, weights streamed
 // from L2 as a transposed [in][out] block, one CTA of kThreads threads.
 #pragma once
 #include <stdint.h>
@@ -19,7 +19,7 @@ template <bool W_IN_SMEM>
 __device__ __forceinline__ float ldw(const float *p) { return W_IN_SMEM ? *p : __ldg(p); }
 
 // gate: optional ReLU-backward mask applied to the result (see the epilogue).
-// W_IN_SMEM: the weight block (and bias) was staged into shared memory (trainer.cu prefetches the next layer's block with
+// W_IN_SMEM: the weight block (and bias) was staged into shared memory (trainer_nets.cu prefetches the next op's block with
 // cp.async while this one computes); otherwise it is streamed from L2.
 template <bool W_IN_SMEM>
 __device__ __forceinline__ void dense_t(const float *__restrict__ X, int ldx, int R, int K, const float *__restrict__ Wt,

@@ -611,9 +611,8 @@ static int selftest_impl(int32_t N, int32_t K, const float *a_host, const float 
         cn_set_error("N in [16,256] step 16, K in [16,256] step 16 (K <= 128 for the MN-major variant)");
         return CN_EINVAL;
     }
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) { cudaGetLastError(); cn_set_error("no CUDA device available; no CPU fallback"); return CN_ECUDA; }
-    CN_CUDA_CHECK(cudaSetDevice(device));
+    const int rc = use_device(device);
+    if (rc) return rc;
     std::vector<uint8_t> ai(bytes_of(ROWS, K), 0), bi(bmn ? bytes_of(ROWS, N) : bytes_of(N, K), 0);
     for (int r = 0; r < ROWS; ++r) for (int k = 0; k < K; ++k) put(ai, 0, ROWS, r, k, a_host[(size_t)r * K + k]);
     for (int r = 0; r < N; ++r)
@@ -662,9 +661,8 @@ extern "C" int cn_selftest_umma_pair(int32_t N, int32_t K, const float *a_host, 
         cn_set_error("N in [32,256] step 16, K in [16,256] step 16, reps >= 1");
         return CN_EINVAL;
     }
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) { cudaGetLastError(); cn_set_error("no CUDA device available; no CPU fallback"); return CN_ECUDA; }
-    CN_CUDA_CHECK(cudaSetDevice(device));
+    const int rc = use_device(device);
+    if (rc) return rc;
     const size_t a_bytes = bytes_of(ROWS, K), b_bytes = bytes_of(N / 2, K);
     std::vector<uint8_t> ai(2 * a_bytes, 0), bi(2 * b_bytes, 0);
     for (int r = 0; r < 2 * ROWS; ++r)

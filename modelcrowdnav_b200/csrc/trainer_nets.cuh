@@ -1,5 +1,6 @@
 // trainer_nets.cuh -- what trainer.cu (the cn_trainer_* entry points, SGD / reduce kernels) and trainer_nets.cu (the forward
-// + backward kernel of CADRL and LSTM-RL) share: one parameter layer of the flat block and the network description.
+// + backward kernels of every value network) share: one parameter layer of the flat block, the network description and the
+// host interface of the forward + backward step.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -10,10 +11,11 @@
 // backward-data products read).  LSTM-RL's nn.LSTM is two such layers, weight_ih / bias_ih and weight_hh / bias_hh.
 struct TLayer { int in, out; int w_off, b_off, t_off, a_off; };
 
-constexpr int kNetMaxLayers = 10;     // LSTM-RL ValueNetwork2: mlp1 (4) + mlp (4) + weight_ih + weight_hh
+constexpr int kNetMaxLayers = 11;     // SARL: mlp1 (2) + mlp2 (2) + attention (3) + mlp3 (4)
 constexpr int kNetMaxOps = 2 * kNetMaxLayers;
 
-// CADRL (net = CN_NET_CADRL): L[0..3] = value_network.{0,2,4,6}, one row per sample.
+// SARL / OM-SARL (net = CN_NET_SARL): L[0..10] = mlp1.{0,2}, mlp2.{0,2}, attention.{0,2,4}, mlp3.{0,2,4,6}.
+// CADRL (CN_NET_CADRL): L[0..3] = value_network.{0,2,4,6}, one row per sample.
 // LSTM-RL (CN_NET_LSTM_RL): [L[0..3] = mlp1.{0,2,4,6} (ValueNetwork2)], then mlp.{0,2,4,6}, weight_ih, weight_hh.
 // ops: the weight blocks in the order the kernel stages them, op_layer[k] = layer, op_bwd[k] = 1 for a backward-data
 // product (block from Wa, no bias) and 0 for a forward layer (block from Wt, bias behind the weights).
@@ -22,6 +24,7 @@ struct NetDims {
     TLayer L[kNetMaxLayers];
     int n_params, t_size, a_size;
     int in, self_dim;
+    int no_gs;                 // SARL without the global state: attention.0's input is e (L[4].in = L[1].out), not [e | mean]
     int vn2;                   // LSTM-RL with the per-row mlp1 in front of the LSTM
     int lstm_h, lstm_in;
     int mlp0;                  // first layer of the value mlp (0 for CADRL and ValueNetwork1, 4 for ValueNetwork2)
@@ -31,13 +34,16 @@ struct NetDims {
     int wbuf_floats;           // size of one staging buffer = the largest block
 };
 
-// Samples per CTA of the network (several CADRL rows share one CTA; one LSTM sequence per CTA).
-int trainer_nets_spc(const NetDims &d);
+// 227 kB: the opt-in dynamic shared memory of one CTA on sm_100
+constexpr size_t kTrainerMaxSmem = 232448;
+
+// Samples per CTA of the network (one SARL or LSTM-RL sample per CTA, several CADRL rows).
+int trainer_spc(const NetDims &d);
 // Shared memory of one CTA: activations for `H` humans and nbuf staging buffers (bytes).
-size_t trainer_nets_smem(const NetDims &d, int H, int nbuf);
-// The kernel's shared-memory limit (call after cudaSetDevice).
-cudaError_t trainer_nets_configure();
-// Forward + backward of `batch` samples -> per-CTA partial gradients gpart[cta][n_params] and squared errors loss_part[cta];
-// *nparts = CTAs launched.  Same arguments as trainer_fwd_bwd_kernel.
-int trainer_nets_launch(const NetDims &d, const float *Wt, const float *Wa, const float *X, const float *target,
-                        const int64_t *index, int batch, int H, float *gpart, float *loss_part, int *nparts, cudaStream_t s);
+size_t trainer_smem(const NetDims &d, int H, int nbuf);
+// The network's kernel may use kTrainerMaxSmem (call after cudaSetDevice).
+cudaError_t trainer_configure(const NetDims &d);
+// Forward + backward of `batch` samples (item index[s] of X / target, or sample s itself when index is NULL) -> per-CTA
+// partial gradients gpart[cta][n_params] and squared errors loss_part[cta]; *nparts = CTAs launched.
+int trainer_launch(const NetDims &d, const float *Wt, const float *Wa, const float *X, const float *target,
+                   const int64_t *index, int batch, int H, float *gpart, float *loss_part, int *nparts, cudaStream_t s);

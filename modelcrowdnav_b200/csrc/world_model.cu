@@ -185,10 +185,8 @@ int cn_world_create(int32_t kind, int32_t human_num, int device, cn_world **out)
     if (!out) { cn_set_error("null argument"); return CN_EINVAL; }
     if (kind != CN_WORLD_ATTENTION && kind != CN_WORLD_MLP) { cn_set_error("unknown world model kind %d", kind); return CN_EINVAL; }
     if (kind == CN_WORLD_MLP && (human_num < 1 || human_num > CN_MAX_HUMANS)) { cn_set_error("MlpWorld needs its human count"); return CN_EINVAL; }
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) { cudaGetLastError(); cn_set_error("no CUDA device available; no CPU fallback"); return CN_ECUDA; }
-    if (device < 0 || device >= n) { cn_set_error("device %d out of range", device); return CN_EINVAL; }
-    CN_CUDA_CHECK(cudaSetDevice(device));
+    const int rc = use_device(device);
+    if (rc) return rc;
     cn_world *w = new cn_world();
     memset(w, 0, sizeof(*w));
     w->device = device;

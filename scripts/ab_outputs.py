@@ -2,7 +2,9 @@
 """Bit-for-bit comparison of what library builds compute: for a fixed seeded matrix of networks, precisions and shapes,
 20 auto-reset rollout steps (state, reward, done, info, and the number of kernel launches of every step), then one lookahead
 (values, action_idx).  Covers the networks bench.py --dump-outputs does not (OM-SARL, CADRL, LSTM-RL) and the pipelined
-host rollout.  Each library runs in its own subprocess (ctypes cannot unload).
+host rollout.  Then the fused trainer of every value network, from seeded weights and a seeded replay memory: the flat
+weights and the loss sum after 20 cn_trainer_step_indexed steps, and the gradient of one grad_out step.  Each library runs
+in its own subprocess (ctypes cannot unload).
 Usage: python scripts/ab_outputs.py [--envs 1024] lib_a.so lib_b.so ...   (exit status 1 when any output differs)"""
 import argparse
 import os
@@ -16,6 +18,60 @@ STEPS = 20
 OM = dict(input_dim=61, with_om=1, cell_num=4, cell_size=1.0, om_channel_size=3)
 NETS = {"sarl": {}, "om_sarl": OM, "cadrl": dict(network="cadrl", mlp3_dims=[150, 100, 100, 1]),
         "lstm": dict(network="lstm_rl", mlp3_dims=[150, 100, 100, 1], lstm_hidden=50)}
+
+
+TRAIN_STEPS = 20
+TRAIN_NETS = ("sarl", "sarl_no_gs", "om_sarl", "cadrl", "lstm_rl", "lstm_rl_vn2", "om_lstm_rl")
+
+
+def train_model(name):
+    from modelcrowdnav_b200.policy import make_cadrl_network, make_lstm_network, make_value_network
+    d = 61 if name.startswith("om_") else 13
+    m3 = [150, 100, 100, 1]
+    if name == "cadrl":
+        return make_cadrl_network(d, m3)
+    if name.endswith("sarl") or name == "sarl_no_gs":
+        return make_value_network(d, 6, [150, 100], [100, 50], m3, [100, 100, 1], with_global_state=name != "sarl_no_gs")
+    return make_lstm_network(d, 6, [150, 100, 100, 50] if name.endswith("vn2") else None, m3, 50)
+
+
+def trainer_rows(res):
+    """flat weights and loss sum after TRAIN_STEPS indexed steps, and one step's gradient, of every value network"""
+    import ctypes as C
+    import torch
+    from modelcrowdnav_b200._capi import check
+    from modelcrowdnav_b200.fused_trainer import FusedTrainer
+    dev = torch.device("cuda:0")
+    for seed, name in enumerate(TRAIN_NETS):
+        g = torch.Generator().manual_seed(1000 + seed)
+        H, d = 5, 61 if name.startswith("om_") else 13
+        states = torch.rand((600, d) if name == "cadrl" else (600, H, d), generator=g) * 4 - 2
+        states[..., 2] = 0.0
+        if d > 13:
+            states[..., 13::3] = (states[..., 13::3] > 0).float()
+        states, values = states.to(dev), (torch.rand((600, 1), generator=g) - 0.25).to(dev)
+        idx = torch.randint(600, (TRAIN_STEPS, 100), generator=g).to(dev)
+        fts = []
+        for _ in range(2):
+            torch.manual_seed(seed)
+            ft = FusedTrainer(train_model(name).to(dev), dev)
+            ft.lr = 0.01
+            fts.append(ft)
+        loss = torch.zeros((), device=dev)
+        for i in range(TRAIN_STEPS):
+            fts[0].step_indexed(states, values, idx[i], loss)
+        f = fts[1]
+        f.sync_from_model()
+        x, y = states[idx[0]].contiguous(), values[idx[0]].reshape(-1).contiguous()
+        check(f.lib.cn_trainer_step(f.handle, C.c_void_p(f.flat.data_ptr()), C.c_void_p(x.data_ptr()), C.c_void_p(y.data_ptr()),
+                                    100, 1 if name == "cadrl" else H, f.lr, f.momentum, C.c_void_p(f.grad.data_ptr()), None,
+                                    f._stream()))
+        torch.cuda.synchronize()
+        res["train_%s/weights" % name] = fts[0].flat.cpu().numpy()
+        res["train_%s/loss_sum" % name] = loss.cpu().numpy()
+        res["train_%s/grad" % name] = f.grad.cpu().numpy()
+        for ft in fts:
+            ft.close()
 
 
 def matrix():
@@ -68,6 +124,7 @@ def child(lib, E, path):
         res[name + "/" + k] = v
     res[name + "/launches"] = np.array(launches)
     pipe.close()
+    trainer_rows(res)
     np.savez(path, **res)
 
 
@@ -100,8 +157,9 @@ def main():
                    if k not in got or ref[k].dtype != got[k].dtype or ref[k].shape != got[k].shape
                    or ref[k].tobytes() != got[k].tobytes()]
             same &= not bad
-            print("  %-28s %-22s launches/step %s" % (c, "bit-identical" if not bad else "DIFFERS: " + ",".join(bad),
-                                                    " ".join(str(n) for n in got[c + "/launches"][:3]) + " ..."))
+            launches = got.get(c + "/launches")
+            print("  %-28s %-22s %s" % (c, "bit-identical" if not bad else "DIFFERS: " + ",".join(bad), "" if launches is None
+                                        else "launches/step " + " ".join(str(n) for n in launches[:3]) + " ..."))
     print("all bit-identical" if same else "OUTPUTS DIFFER")
     return 0 if same else 1
 

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Per-step time of the fused trainer against the CUDA-graph replay of torch autograd: wall clock vs CUDA events over N
 back-to-back steps (cn_trainer_step_indexed / graph replay) on a synthetic replay memory (batch 100 x 5 humans; CADRL: one
-human per sample).  Usage: python scripts/trainer_timing.py [network] [steps], network one of sarl (default), om_sarl,
-cadrl, lstm_rl, lstm_rl_vn2; lines for a network other than sarl start with its name."""
+human per sample).  Usage: python scripts/trainer_timing.py [--lib libcrowdnav_b200.so] [network] [steps], network one of
+sarl (default), om_sarl, cadrl, lstm_rl, lstm_rl_vn2; lines for a network other than sarl start with its name.  --lib
+times another build of the library (e.g. the parent commit's, for an A/B comparison)."""
 import os
 import sys
 import time
@@ -21,6 +22,9 @@ NETS = {"sarl": lambda: make_value_network(13, 6, [150, 100], [100, 50], [150, 1
         "lstm_rl": lambda: make_lstm_network(13, 6, None, [150, 100, 100, 1], 50),
         "lstm_rl_vn2": lambda: make_lstm_network(13, 6, [150, 100, 100, 50], [150, 100, 100, 1], 50)}
 args = sys.argv[1:]
+if args[:1] == ["--lib"]:
+    mcn._capi.LIB_PATH = os.path.abspath(args[1])
+    args = args[2:]
 net = args.pop(0) if args and not args[0].isdigit() else "sarl"
 if net not in NETS:
     sys.exit("network must be one of %s" % ", ".join(NETS))

@@ -235,6 +235,7 @@ def test_refusals(dev):
     assert create(5, input_dim=13, **om) == _capi.CN_EINVAL                       # with_om and input_dim disagree
     assert create(5, input_dim=60, **om, **lstm) == _capi.CN_EINVAL
     assert create(1, input_dim=61, **om, **cadrl) == _capi.CN_EINVAL               # CADRL has no maps
+    assert create(5, input_dim=61, cell_size=0.0, **om) == _capi.CN_EINVAL        # the map cells need a positive size
     # a CADRL step with more than one human per sample
     h = C.c_void_p()
     _capi.check(lib.cn_trainer_create(C.byref(_capi.default_sarl_cfg(**cadrl)), 0, 128, 1, C.byref(h)))
