@@ -477,11 +477,16 @@ def test_tc_matches_f32_odd_shapes(mcn, weights0, E, H, speeds, rots):
 
 
 @pytest.mark.parametrize("net", ["cadrl", "lstm", "om_sarl"])
-@pytest.mark.parametrize("E,H,query_env", [(1000, 4, 0), (777, 6, 1), (130, 13, 0), (3000, 5, 0)])
+@pytest.mark.parametrize("E,H,query_env", [(1000, 4, 0), (777, 6, 1), (130, 13, 0), (3000, 5, 0),
+                                           # the ends of the human range and the G = 64, 3, 2 layouts of the X tiles, with
+                                           # >= 3 rounds of J tiles per CTA-pair slot (LSTM-RL: 3 x H recurrent stages)
+                                           (1, 1, 0), (1200, 1, 1), (1000, 2, 1), (1000, 33, 0), (1100, 43, 1), (1500, 64, 0)])
 def test_tc_other_networks_match_f32_at_size(mcn, units_nets, units_om, net, E, H, query_env):
     """The tensor-core forms of CADRL (tc_mlp3_pair_kernel<1>), LSTM-RL (tc_lstm_pair_kernel: several rounds per slot, every
     step count) and OM-SARL (tc_om_bias_kernel + the row kernel's bias epilogue) against their FP32 kernels (themselves pinned
-    to the reference's episodes) on sizes that divide nothing, over evolving device-generated states."""
+    to the reference's episodes) on sizes that divide nothing, over evolving device-generated states.  On 148 SMs a round is
+    296 tiles: at 1200 x 1, 1000 x 2, 1000 x 33, 1100 x 43 and 1500 x 64 the LSTM's 760, 633, 633, 697 and 950 J tiles take 3 to
+    4 rounds, so every slot resets h_0 and c_0 between tiles and wraps its mbarrier phases."""
     env = mcn.BatchedCrowdSim(E, H, auto_reset=1, seed=11, sim_rule=1)
     if net == "om_sarl":
         p32, p16 = _om_policy(mcn, "sarl", "f32"), _om_policy(mcn, "sarl", "f16_tc")
