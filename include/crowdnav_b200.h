@@ -217,6 +217,12 @@ int cn_env_read_stats(cn_env *env, cn_stats *out, int reset, void *stream);
  * NULL), asynchronously on `stream`: a roll-out that fills the replay memory records its per-step rewards and done flags
  * this way instead of reading them back (explorer.py:62-69,87-89).  A frozen env reports reward 0, done 1. */
 int cn_env_copy_outputs(cn_env *env, double *reward_dev, uint8_t *done_dev, uint8_t *info_dev, void *stream);
+/* Training pairs of a world model (ModelCrowdSim's sim_world), device -> device on `stream`: x_dev (E x H x 4 fp32) = every
+ * human's CURRENT (px, py, vx, vy), cast to fp32 exactly as cn_world_predict reads it; y_dev (E x H x 2 fp32) = the cached
+ * velocities of this step (cn_env_orca, or cn_world_predict); valid_dev (optional, E bytes) = 1 where the env is not frozen.
+ * Call between the ORCA solve and cn_env_step: (x, y) is then (state before step t, the velocity each human takes in step t).
+ * CN_EINVAL without a cached ORCA / world-model result. */
+int cn_env_copy_world_pairs(cn_env *env, float *x_dev, float *y_dev, uint8_t *valid_dev, void *stream);
 int64_t cn_env_episode_table_bytes(const cn_env *env);
 int cn_env_read_episode_table(cn_env *env, void *table_host, uint8_t *frozen_host, void *stream);
 
@@ -360,6 +366,46 @@ int cn_world_destroy(cn_world *w);
 int64_t cn_world_param_count(const cn_world *w);
 int cn_world_load_weights(cn_world *w, const float *flat_host, int64_t n, void *stream);
 int cn_world_predict(cn_world *w, cn_env *env, void *stream);
+/* cn_world_load_weights from a DEVICE block (the same flat layout), enqueued on `stream` with no host staging: a model being
+ * trained (cn_world_trainer_*) drives cn_world_predict without a weight copy through the host. */
+int cn_world_load_weights_device(cn_world *w, const float *flat_dev, int64_t n, void *stream);
+
+/* ---- training a world model on the device: MSELoss + backward + torch.optim.Adam -----------------------------------------
+ * One optimisation step of AttentionWorld / MlpWorld on ONE flat fp32 parameter block in the reference module's state-dict
+ * order (the block cn_world_load_weights takes: AttentionWorld 94,953 parameters, MlpWorld(H) 4H*128 + 128 + 8,256 + 780 +
+ * 24H + 2H): a forward + hand-written backward kernel, then a reduce + Adam kernel.  Data: x_dev batch x human_num x 4 fp32
+ * human states (px, py, vx, vy), y_dev batch x human_num x 2 fp32 velocities (cn_env_copy_world_pairs); sample i is item
+ * index_dev[i] (int64, device) of x_dev / y_dev, or item i when index_dev is NULL.  Loss: torch.nn.MSELoss() (mean over
+ * batch * human_num * 2 outputs).
+ * cn_world_trainer_create: kind CN_WORLD_ATTENTION (human_num = the most humans a sample may have) or CN_WORLD_MLP (built
+ *   for human_num humans).  drop_rate: MlpWorld's Dropout after the ReLUs of mlp.0 and mlp.3 in training mode, kept units
+ *   scaled by 1 / (1 - drop_rate); the mask of (batch position, layer, unit) is a Philox draw keyed by (seed, the step count
+ *   since the last optimizer reset).  AttentionWorld has no dropout (drop_rate must be 0).
+ * cn_world_trainer_sync_weights: call before the first step and whenever w_dev was changed by anyone else; reset_optimizer = 1
+ *   also zeroes Adam's moments and step count (a new optimiser).
+ * cn_world_trainer_step: grad_out_dev == NULL: Adam in place on w_dev (m = b1 m + (1-b1) g, v = b2 v + (1-b2) g^2,
+ *   w -= lr / (1 - b1^t) * m / (sqrt(v) / sqrt(1 - b2^t) + eps), t counted in the handle); grad_out_dev != NULL: only the
+ *   gradient (n_params fp32) -- the caller all-reduces it and calls cn_world_trainer_apply(grad, 1 / world).  loss_sum_dev
+ *   (optional) is ADDED the batch MSE.  mask_dev (optional, MlpWorld) receives the dropout masks, batch x (128 + 64) bytes in
+ *   the order of mlp.0's then mlp.3's units, 1 = kept.
+ * cn_world_trainer_eval: forward only, dropout off: ADDS the MSE of the n samples to *loss_sum_dev (validation loss).  Reads
+ *   the weights as of the last step / sync.
+ * Limits: CN_EINVAL for batch > max_batch, drop_rate outside [0, 1), an MlpWorld whose human count differs from the data's,
+ *   and a step before the first sync; CN_EUNSUPPORTED for a human count whose shared-memory plan does not fit one CTA
+ *   (AttentionWorld: more than 23 humans). */
+typedef struct cn_world_trainer cn_world_trainer;
+int cn_world_trainer_create(int32_t kind, int32_t human_num, int device, int32_t max_batch, float drop_rate,
+                            cn_world_trainer **out);
+int cn_world_trainer_destroy(cn_world_trainer *t);
+int64_t cn_world_trainer_param_count(const cn_world_trainer *t);
+int cn_world_trainer_sync_weights(cn_world_trainer *t, const float *w_dev, int reset_optimizer, void *stream);
+int cn_world_trainer_step(cn_world_trainer *t, float *w_dev, const float *x_dev, const float *y_dev, const int64_t *index_dev,
+                          int32_t batch, int32_t human_num, float lr, float beta1, float beta2, float eps, uint64_t seed,
+                          float *grad_out_dev, float *loss_sum_dev, uint8_t *mask_dev, void *stream);
+int cn_world_trainer_apply(cn_world_trainer *t, float *w_dev, const float *grad_dev, float grad_scale, float lr, float beta1,
+                           float beta2, float eps, void *stream);
+int cn_world_trainer_eval(cn_world_trainer *t, const float *x_dev, const float *y_dev, const int64_t *index_dev, int32_t n,
+                          int32_t human_num, float *loss_sum_dev, void *stream);
 
 /* ---- value-network training step on the device (crowd_nav/utils/trainer.py:36-82) ------------------------------------
  * One optimisation step of the reference Trainer -- zero_grad, model(inputs), MSELoss, backward, SGD(momentum).step -- as

@@ -22,10 +22,12 @@ EXPORTS = [
     "cn_last_error", "cn_version", "cn_device_count", "cn_env_cfg_default", "cn_sarl_cfg_default",
     "cn_env_create", "cn_env_destroy", "cn_env_set_state", "cn_env_get_state", "cn_env_set_theta", "cn_env_get_theta", "cn_env_reset", "cn_env_orca",
     "cn_env_robot_orca", "cn_env_step", "cn_env_get_views", "cn_env_read_outputs", "cn_env_read_human_actions",
-    "cn_env_read_next_obs", "cn_env_read_actions", "cn_env_set_actions", "cn_env_set_human_actions", "cn_env_read_stats", "cn_env_copy_outputs", "cn_env_episode_table_bytes", "cn_env_read_episode_table", "cn_policy_create", "cn_policy_destroy",
+    "cn_env_read_next_obs", "cn_env_read_actions", "cn_env_set_actions", "cn_env_set_human_actions", "cn_env_read_stats", "cn_env_copy_outputs", "cn_env_copy_world_pairs", "cn_env_episode_table_bytes", "cn_env_read_episode_table", "cn_policy_create", "cn_policy_destroy",
     "cn_policy_param_count", "cn_policy_load_weights", "cn_policy_action_table", "cn_policy_lookahead",
     "cn_policy_read", "cn_policy_bad_count", "cn_policy_transform", "cn_policy_last_state", "cn_policy_forward", "cn_rollout_step", "cn_rollout_step_sharded", "cn_rollout_episodes", "cn_rollout_step_host", "cn_rollout_step_host_packed", "cn_rollout_step_host_packed_async", "cn_stream_sync", "cn_host_step_bytes",
     "cn_scenes_generate", "cn_world_create", "cn_world_destroy", "cn_world_param_count", "cn_world_load_weights", "cn_world_predict",
+    "cn_world_load_weights_device", "cn_world_trainer_create", "cn_world_trainer_destroy", "cn_world_trainer_param_count",
+    "cn_world_trainer_sync_weights", "cn_world_trainer_step", "cn_world_trainer_apply", "cn_world_trainer_eval",
     "cn_trainer_create", "cn_trainer_destroy", "cn_trainer_param_count", "cn_trainer_sync_weights", "cn_trainer_step", "cn_trainer_step_indexed", "cn_trainer_apply",
     "cn_launch_count", "cn_debug_trace", "cn_debug_trace_dump", "cn_selftest_umma", "cn_selftest_umma_bmn", "cn_selftest_umma_ts", "cn_selftest_umma_pair", "cn_debug_tc_timing", "cn_debug_kernel_ms",
 ]
@@ -151,6 +153,17 @@ def load():
     L.cn_world_param_count.restype = i64
     L.cn_world_load_weights.argtypes = [vp, vp, i64, vp]
     L.cn_world_predict.argtypes = [vp, vp, vp]
+    L.cn_world_load_weights_device.argtypes = [vp, vp, i64, vp]
+    L.cn_env_copy_world_pairs.argtypes = [vp, vp, vp, vp, vp]
+    f32 = C.c_float
+    L.cn_world_trainer_create.argtypes = [i32, i32, C.c_int, i32, f32, C.POINTER(vp)]
+    L.cn_world_trainer_destroy.argtypes = [vp]
+    L.cn_world_trainer_param_count.argtypes = [vp]
+    L.cn_world_trainer_param_count.restype = i64
+    L.cn_world_trainer_sync_weights.argtypes = [vp, vp, C.c_int, vp]
+    L.cn_world_trainer_step.argtypes = [vp, vp, vp, vp, vp, i32, i32, f32, f32, f32, f32, C.c_uint64, vp, vp, vp, vp]
+    L.cn_world_trainer_apply.argtypes = [vp, vp, vp, f32, f32, f32, f32, f32, vp]
+    L.cn_world_trainer_eval.argtypes = [vp, vp, vp, vp, i32, i32, vp, vp]
     L.cn_trainer_create.argtypes = [C.POINTER(SarlCfg), C.c_int, i32, i32, C.POINTER(vp)]
     L.cn_trainer_destroy.argtypes = [vp]
     L.cn_trainer_param_count.argtypes = [vp]

@@ -489,6 +489,33 @@ int cn_env_copy_outputs(cn_env *env, double *reward_dev, uint8_t *done_dev, uint
     return CN_OK;
 }
 
+// one thread per (env, human): the world model's input (px, py, vx, vy) and target (the cached velocities), cast to fp32 as
+// attention_world_kernel / mlp_world_kernel cast the state they read
+static __global__ void copy_world_pairs_kernel(EnvDims d, const double *__restrict__ st, const double *__restrict__ human_v,
+                                               const uint8_t *__restrict__ frozen, float *__restrict__ x, float *__restrict__ y,
+                                               uint8_t *__restrict__ valid)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= d.E * d.H) return;
+    const int env = i / d.H, h = i - env * d.H;
+    const int fields[4] = {F_PX, F_PY, F_VX, F_VY};
+    for (int k = 0; k < 4; ++k) x[(size_t)i * 4 + k] = (float)st[st_idx(d, fields[k], h + 1, env)];
+    for (int c = 0; c < 2; ++c) y[(size_t)i * 2 + c] = (float)human_v[(size_t)(c * d.H + h) * d.E + env];
+    if (h == 0 && valid) valid[env] = frozen[env] ? 0 : 1;
+}
+
+int cn_env_copy_world_pairs(cn_env *env, float *x_dev, float *y_dev, uint8_t *valid_dev, void *stream)
+{
+    CN_ENV_ENTER(env);
+    if (!x_dev || !y_dev) { cn_set_error("null argument"); return CN_EINVAL; }
+    if (!env->orca_valid) { cn_set_error("no cached ORCA or world-model result; call cn_env_orca or cn_world_predict"); return CN_EINVAL; }
+    const EnvDims d = env->p.d;
+    const int n = d.E * d.H;
+    copy_world_pairs_kernel<<<(n + 255) / 256, 256, 0, s>>>(d, env->state, env->human_v, env->frozen, x_dev, y_dev, valid_dev);
+    CN_LAUNCH_CHECK();
+    return CN_OK;
+}
+
 int64_t cn_env_episode_table_bytes(const cn_env *env) { return env ? (int64_t)env->p.d.E * 8 * 11 : 0; }
 
 int cn_env_read_episode_table(cn_env *env, void *table_host, uint8_t *frozen_host, void *stream)

@@ -330,6 +330,9 @@ int use_device(int device);
 // The checks every entry point that takes a network configuration makes with CN_EINVAL: a known network, the global-state
 // switch on SARL only, and occupancy maps of a valid shape on a network that has them (capi.cu).
 int cn_check_net_cfg(const cn_sarl_cfg *cfg);
+// The Linear layers of a world model (CN_WORLD_*; MlpWorld built for human_num humans) in state-dict order: in / out widths,
+// returns their count (world_model.cu)
+int world_layer_dims(int kind, int human_num, int *ins, int *outs);
 int cn_launch_orca(cn_env *env, cudaStream_t s);
 int cn_launch_robot_orca(cn_env *env, double safety_space, cudaStream_t s);
 int cn_launch_step(cn_env *env, const double *action_xy_dev, int update, cudaStream_t s, int fuse_reset = 0);

@@ -89,9 +89,44 @@ struct cn_trainer {
     int nparts_cap;
 };
 
+void trainer_layout(NetDims &d)
+{
+    int toff = 0, aoff = 0;
+    d.wbuf_floats = 0;
+    for (int i = 0; i < d.n_layers; ++i) {
+        TLayer &l = d.L[i];
+        l.t_off = toff; toff += pad4(l.in * l.out) + pad4(l.out);      // [in][out] | bias, 16-byte aligned blocks
+        l.a_off = aoff; aoff += pad4(l.in * l.out);                    // [out][in]
+        const int blk = pad4(l.in * l.out) + pad4(l.out);
+        if (blk > d.wbuf_floats) d.wbuf_floats = blk;
+    }
+    d.t_size = toff; d.a_size = aoff;
+}
+
+void trainer_maps(const NetDims &d, int32_t *tmap, int32_t *amap)
+{
+    for (int i = 0; i < d.n_params; ++i) amap[i] = -1;
+    for (int i = 0; i < d.n_layers; ++i) {
+        const TLayer &l = d.L[i];
+        for (int o = 0; o < l.out; ++o)
+            for (int k = 0; k < l.in; ++k) {
+                tmap[l.w_off + o * l.in + k] = l.t_off + k * l.out + o;
+                amap[l.w_off + o * l.in + k] = l.a_off + o * l.in + k;
+            }
+        for (int o = 0; o < l.out; ++o) tmap[l.b_off + o] = l.t_off + pad4(l.in * l.out) + o;
+    }
+}
+
+int trainer_refresh(int n_params, const float *W, float *Wt, float *Wa, const int32_t *tmap, const int32_t *amap, cudaStream_t s)
+{
+    trainer_transpose_kernel<<<(n_params + 255) / 256, 256, 0, s>>>(n_params, W, Wt, Wa, tmap, amap);
+    CN_LAUNCH_CHECK();
+    return CN_OK;
+}
+
 // The weight matrices of the flat block in state-dict order, from the layer list the lookahead loads (cn_layers): a Linear
-// is one TLayer, the LSTM block two (weight_ih with bias_ih, weight_hh with bias_hh).  Fills d.L / n_layers (w_off / b_off /
-// t_off / a_off), the parameter count, the sizes of Wt and Wa, and wbuf_floats = the largest staged block.
+// is one TLayer, the LSTM block two (weight_ih with bias_ih, weight_hh with bias_hh).  Fills d.L / n_layers (w_off / b_off),
+// the parameter count, and through trainer_layout the Wt / Wa blocks and wbuf_floats = the largest staged block.
 static void trainer_layers(const cn_sarl_cfg *cfg, NetDims &d)
 {
     SarlWeightsDev w;        // only the destinations of the layer list, never written here
@@ -108,16 +143,7 @@ static void trainer_layers(const cn_sarl_cfg *cfg, NetDims &d)
     }
     d.n_layers = n;
     d.n_params = off;
-    int toff = 0, aoff = 0;
-    d.wbuf_floats = 0;
-    for (int i = 0; i < n; ++i) {
-        TLayer &l = d.L[i];
-        l.t_off = toff; toff += pad4(l.in * l.out) + pad4(l.out);      // [in][out] | bias, 16-byte aligned blocks
-        l.a_off = aoff; aoff += pad4(l.in * l.out);                    // [out][in]
-        const int blk = pad4(l.in * l.out) + pad4(l.out);
-        if (blk > d.wbuf_floats) d.wbuf_floats = blk;
-    }
-    d.t_size = toff; d.a_size = aoff;
+    trainer_layout(d);
 }
 
 // The rest of the network description (after trainer_layers) and the order in which its kernel stages the weight blocks
@@ -197,16 +223,8 @@ int cn_trainer_create(const cn_sarl_cfg *cfg, int device, int32_t max_batch, int
         return CN_EUNSUPPORTED;
     }
     const int n_params = d.n_params;
-    std::vector<int32_t> tmap(n_params), amap(n_params, -1);
-    for (int i = 0; i < d.n_layers; ++i) {
-        const TLayer &l = d.L[i];
-        for (int o = 0; o < l.out; ++o)
-            for (int k = 0; k < l.in; ++k) {
-                tmap[l.w_off + o * l.in + k] = l.t_off + k * l.out + o;
-                amap[l.w_off + o * l.in + k] = l.a_off + o * l.in + k;
-            }
-        for (int o = 0; o < l.out; ++o) tmap[l.b_off + o] = l.t_off + pad4(l.in * l.out) + o;
-    }
+    std::vector<int32_t> tmap(n_params), amap(n_params);
+    trainer_maps(d, tmap.data(), amap.data());
     cn_trainer *t = new cn_trainer();
     memset(t, 0, sizeof(*t));
     t->device = device; t->d = d; t->max_batch = max_batch; t->max_humans = max_humans;
@@ -257,8 +275,8 @@ int cn_trainer_sync_weights(cn_trainer *t, const float *w_dev, int zero_momentum
     CN_CUDA_CHECK(cudaSetDevice(t->device));
     cudaStream_t s = (cudaStream_t)stream;
     const int n = t->d.n_params;
-    trainer_transpose_kernel<<<(n + 255) / 256, 256, 0, s>>>(n, w_dev, t->Wt, t->Wa, t->tmap, t->amap);
-    CN_LAUNCH_CHECK();
+    const int rc = trainer_refresh(n, w_dev, t->Wt, t->Wa, t->tmap, t->amap, s);
+    if (rc) return rc;
     if (zero_momentum) CN_CUDA_CHECK(cudaMemsetAsync(t->mom, 0, sizeof(float) * n, s));
     return CN_OK;
 }

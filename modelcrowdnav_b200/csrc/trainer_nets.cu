@@ -492,24 +492,342 @@ trainer_nets_fwd_bwd_kernel(NetDims d, const float *__restrict__ Wt, const float
     st.finish();
 }
 
+// ---------------- the world models (crowd_nav/policy/world_model.py:20-106) ----------------
+// Loss of both: MSELoss(mean) over the batch x H x 2 predicted velocities.
+
+// AttentionWorld's shared-memory plan (floats) for the R = H rows of one sample; every row stride is a multiple of 4 floats
+struct WPlan {
+    int ld_x, ld_a1, ld_e, ld_f1, ld_f, ld_u, ld_t, ld_j, ld_g1, ld_g, ld_o;
+    int x, a1, e, f1, f, u, t1, t2, sc, wt, dc, j, g1, g2, g3, o, d0, d1, total;
+};
+
+__host__ __device__ inline WPlan make_wplan(const NetDims &d, int R)
+{
+    WPlan p;
+    p.ld_x = pad4(d.in); p.ld_a1 = pad4(d.L[0].out); p.ld_e = pad4(d.L[1].out); p.ld_f1 = pad4(d.L[2].out);
+    p.ld_f = pad4(d.L[3].out); p.ld_u = pad4(d.L[4].in);
+    p.ld_t = pad4(max(max(d.L[4].out, d.L[5].out), d.L[1].out));      // t1 / t2 rows also host de (mlp1's output gradient)
+    p.ld_j = pad4(d.L[7].in); p.ld_g1 = pad4(d.L[7].out); p.ld_g = pad4(max(d.L[8].out, d.L[9].out)); p.ld_o = pad4(d.L[10].out);
+    int o = 0;
+    p.x = o; o += R * p.ld_x;
+    p.a1 = o; o += R * p.ld_a1;
+    p.e = o; o += R * p.ld_e;
+    p.f1 = o; o += R * p.ld_f1;
+    p.f = o; o += R * p.ld_f;
+    p.u = o; o += R * p.ld_u;
+    p.t1 = o; o += R * p.ld_t;
+    p.t2 = o; o += R * p.ld_t;
+    p.sc = o; o += pad4(R);
+    p.wt = o; o += pad4(R);
+    p.dc = o; o += p.ld_f;
+    p.j = o; o += R * p.ld_j;
+    p.g1 = o; o += R * p.ld_g1;
+    p.g2 = o; o += R * p.ld_g;
+    p.g3 = o; o += R * p.ld_g;
+    p.o = o; o += R * p.ld_o;
+    // two gradient scratch buffers, each as wide as the widest gradient row they hold
+    const int wide = max(max(max(p.ld_u, p.ld_a1), max(p.ld_g1, p.ld_j)), max(max(p.ld_t, p.ld_g), max(p.ld_f, p.ld_o)));
+    p.d0 = o; o += R * wide;
+    p.d1 = o; o += R * wide;
+    p.total = o;
+    return p;
+}
+
+// AttentionWorld: one CTA per sample, its H rows through SARL's blocks -- mlp1, mlp2, attention on [e_i | mean e], the masked
+// softmax -- and then mlp3 on EVERY row, joint_i = [x_i | the sample's weighted feature] -> (vx, vy) of human i.  The op list
+// is SARL's (forward 0..10, backward-data 10, 9, 8, 7, 3, 6, 5, 4, 2, 1).  Backward differences from SARL: mlp3's gradients
+// run over R rows, d(feature) is the sum over the rows of the feature columns of d(joint_i), and the first d.in columns of
+// d(joint_i) (the input itself) are dropped.  fwd_only: the squared errors alone (the op list then ends after layer 10).
+__global__ void __launch_bounds__(kThreads, 1)
+world_attention_fwd_bwd_kernel(NetDims d, const float *__restrict__ Wt, const float *__restrict__ Wa, const float *__restrict__ X,
+                               const float *__restrict__ target, const int64_t *__restrict__ index, int B, int H, int nbuf,
+                               int fwd_only, float *__restrict__ gpart, float *__restrict__ loss_part)
+{
+    extern __shared__ __align__(16) float sm[];
+    const int R = H, tid = threadIdx.x;
+    const WPlan p = make_wplan(d, H);
+    float *xs = sm + p.x, *a1 = sm + p.a1, *e = sm + p.e, *f1 = sm + p.f1, *f = sm + p.f, *u = sm + p.u, *t1 = sm + p.t1,
+          *t2 = sm + p.t2, *sc = sm + p.sc, *wt = sm + p.wt, *dcv = sm + p.dc, *j = sm + p.j, *g1 = sm + p.g1, *g2 = sm + p.g2,
+          *g3 = sm + p.g3, *out = sm + p.o, *d0 = sm + p.d0, *d1 = sm + p.d1;
+    const int E1 = d.L[1].out, F = d.L[3].out, IN = d.in, O = d.L[10].out;
+    const size_t item = index ? (size_t)index[blockIdx.x] : (size_t)blockIdx.x;
+    Staging st(d, Wt, Wa, sm + pad4(p.total), nbuf);
+
+    // ---------------- forward (world_model.py:71-106), the arithmetic of attention_world_kernel ----------------
+    for (int idx = tid; idx < R * p.ld_x; idx += kThreads) {
+        const int r = idx / p.ld_x, k = idx - r * p.ld_x;
+        xs[idx] = k < IN ? X[(item * H + r) * IN + k] : 0.0f;
+    }
+    st.fwd(0, xs, p.ld_x, R, a1, p.ld_a1, true);                                // mlp1.0 + ReLU
+    st.fwd(1, a1, p.ld_a1, R, e, p.ld_e, true);                                 // mlp1.2 + ReLU
+    st.fwd(2, e, p.ld_e, R, f1, p.ld_f1, true, false);                          // mlp2.0 + ReLU
+    for (int k = tid; k < E1; k += kThreads) {                                  // u = [e_i | mean over the sample's humans]
+        float m = 0.0f;
+        for (int h = 0; h < H; ++h) m += e[(size_t)h * p.ld_e + k];
+        m /= (float)H;
+        for (int h = 0; h < H; ++h) {
+            u[(size_t)h * p.ld_u + k] = e[(size_t)h * p.ld_e + k];
+            u[(size_t)h * p.ld_u + E1 + k] = m;
+        }
+    }
+    st.end_op();
+    st.fwd(3, f1, p.ld_f1, R, f, p.ld_f, false);                                // mlp2.2
+    st.fwd(4, u, p.ld_u, R, t1, p.ld_t, true);                                  // attention.0 + ReLU
+    st.fwd(5, t1, p.ld_t, R, t2, p.ld_t, true);                                 // attention.2 + ReLU
+    st.fwd(6, t2, p.ld_t, R, sc, 1, false);                                     // attention.4 -> score
+    if (tid == 0) {                                                             // masked softmax (world_model.py:85-86)
+        float z = 0.0f;
+        for (int h = 0; h < H; ++h) {
+            const float s = sc[h];
+            const float ex = expf(s) * (s != 0.0f ? 1.0f : 0.0f);
+            wt[h] = ex; z += ex;
+        }
+        for (int h = 0; h < H; ++h) wt[h] /= z;
+    }
+    __syncthreads();
+    for (int idx = tid; idx < R * p.ld_j; idx += kThreads) {                    // joint_i = [x_i | weighted feature]
+        const int r = idx / p.ld_j, k = idx - r * p.ld_j;
+        float val = 0.0f;
+        if (k < IN) val = xs[(size_t)r * p.ld_x + k];
+        else if (k < IN + F)
+            for (int h = 0; h < H; ++h) val = fmaf(wt[h], f[(size_t)h * p.ld_f + k - IN], val);
+        j[idx] = val;
+    }
+    st.fwd(7, j, p.ld_j, R, g1, p.ld_g1, true);                                 // mlp3.0   (begin_op's barrier publishes j)
+    st.fwd(8, g1, p.ld_g1, R, g2, p.ld_g, true);                                // mlp3.2
+    st.fwd(9, g2, p.ld_g, R, g3, p.ld_g, true);                                 // mlp3.4
+    st.fwd(10, g3, p.ld_g, R, out, p.ld_o, false);                              // mlp3.6 -> (vx, vy)
+
+    // ---------------- loss and backward ----------------
+    // MSELoss(mean) over B x H x O outputs: dL/dout = 2 (out - y) / (B H O)
+    const float *y = target + item * H * O;
+    if (tid == 0) {
+        float ls = 0.0f;
+        for (int i = 0; i < R * O; ++i) { const float df = out[(size_t)(i / O) * p.ld_o + i % O] - y[i]; ls += df * df; }
+        loss_part[blockIdx.x] = ls;
+    }
+    if (fwd_only) { st.finish(); return; }
+    float *G = gpart + (size_t)blockIdx.x * d.n_params;
+    const float norm = 2.0f / (float)((int64_t)B * H * O);
+    float *dout = d0;                                               // [R][ld_o]
+    for (int i = tid; i < R * O; i += kThreads) {
+        const size_t at = (size_t)(i / O) * p.ld_o + i % O;
+        dout[at] = norm * (out[at] - y[i]);
+    }
+    __syncthreads();
+    // mlp3 over every row
+    wgrad(d, G, 10, dout, p.ld_o, g3, p.ld_g, R);
+    float *dg3 = d1;
+    st.bwd(10, dout, p.ld_o, R, dg3, p.ld_g, g3, p.ld_g);
+    wgrad(d, G, 9, dg3, p.ld_g, g2, p.ld_g, R);
+    float *dg2 = d0;                                                // dout is dead
+    st.bwd(9, dg3, p.ld_g, R, dg2, p.ld_g, g2, p.ld_g);
+    wgrad(d, G, 8, dg2, p.ld_g, g1, p.ld_g1, R);
+    float *dg1 = d1;                                                // dg3 is dead
+    st.bwd(8, dg2, p.ld_g, R, dg1, p.ld_g1, g1, p.ld_g1);
+    wgrad(d, G, 7, dg1, p.ld_g1, j, p.ld_j, R);
+    float *dj = d0;                                                 // [R][ld_j]; x_i's columns have no parameters upstream
+    st.bwd(7, dg1, p.ld_g1, R, dj, p.ld_j, nullptr, 0);
+    // d(feature) = sum over the rows of d(joint_i)[IN:]
+    for (int k = tid; k < F; k += kThreads) {
+        float s = 0.0f;
+        for (int r = 0; r < R; ++r) s += dj[(size_t)r * p.ld_j + IN + k];
+        dcv[k] = s;
+    }
+    __syncthreads();
+    // weighted feature c = sum_i w_i f_i :  df_i = w_i dc,  dw_i = dc . f_i ;  softmax: ds_i = w_i (dw_i - sum_k w_k dw_k)
+    float *df = d1;                                                 // [R][ld_f]  (dg1 is dead)
+    float *dsc = sc;                                                // scores are dead after the softmax: reuse for ds
+    if (tid < R) {
+        float dw = 0.0f;
+        for (int k = 0; k < F; ++k) dw = fmaf(dcv[k], f[(size_t)tid * p.ld_f + k], dw);
+        dsc[tid] = dw;
+    }
+    for (int idx = tid; idx < R * F; idx += kThreads) {
+        const int r = idx / F, k = idx - r * F;
+        df[(size_t)r * p.ld_f + k] = wt[r] * dcv[k];
+    }
+    __syncthreads();
+    if (tid == 0) {
+        float dot = 0.0f;
+        for (int h = 0; h < H; ++h) dot = fmaf(wt[h], dsc[h], dot);
+        for (int h = 0; h < H; ++h) dsc[h] = wt[h] * (dsc[h] - dot);
+    }
+    __syncthreads();
+    // from here on SARL's backward with one sample: mlp2.2 (no ReLU after it) and attention.4
+    wgrad(d, G, 3, df, p.ld_f, f1, p.ld_f1, R);
+    wgrad(d, G, 6, dsc, 1, t2, p.ld_t, R);
+    float *df1 = d0;                                                // [R][ld_f1]  (dj is dead)
+    st.bwd(3, df, p.ld_f, R, df1, p.ld_f1, f1, p.ld_f1);
+    wgrad(d, G, 2, df1, p.ld_f1, e, p.ld_e, R);
+    float *dt2 = d1;                                                // [R][ld_t]  (df is dead)
+    st.bwd(6, dsc, 1, R, dt2, p.ld_t, t2, p.ld_t);
+    wgrad(d, G, 5, dt2, p.ld_t, t1, p.ld_t, R);
+    float *dt1 = t2;                                                // t2 is dead
+    st.bwd(5, dt2, p.ld_t, R, dt1, p.ld_t, t1, p.ld_t);
+    wgrad(d, G, 4, dt1, p.ld_t, u, p.ld_u, R);
+    float *de = t1, *du = d1;                                       // t1 is dead; du: dt2 is dead
+    st.bwd(4, dt1, p.ld_t, R, du, p.ld_u, nullptr, 0);
+    for (int k = tid; k < E1; k += kThreads) {                      // de_i = du_i[:E1] + (1/H) sum_k du_k[E1:]
+        float m = 0.0f;
+        for (int h = 0; h < H; ++h) m += du[(size_t)h * p.ld_u + E1 + k];
+        m /= (float)H;
+        for (int h = 0; h < H; ++h) de[(size_t)h * p.ld_t + k] = du[(size_t)h * p.ld_u + k] + m;
+    }
+    st.bwd(2, df1, p.ld_f1, R, de, p.ld_t, e, p.ld_e, true);        // += df1 * W_mlp2.0   (begin_op's barrier publishes de)
+    wgrad(d, G, 1, de, p.ld_t, a1, p.ld_a1, R);
+    float *da1 = d1;
+    st.bwd(1, de, p.ld_t, R, da1, p.ld_a1, a1, p.ld_a1);
+    wgrad(d, G, 0, da1, p.ld_a1, xs, p.ld_x, R);
+    st.finish();
+}
+
+// MlpWorld's shared-memory plan (floats) for ns samples = ns rows
+struct MPlan { int ld_x, ld_a[3], ld_o; int x, a[3], o, d0, d1, total; };
+
+__host__ __device__ inline MPlan make_mplan(const NetDims &d, int ns)
+{
+    MPlan p;
+    int o = 0, wide = 0;
+    p.ld_x = pad4(d.L[0].in); p.x = o; o += ns * p.ld_x;
+    for (int i = 0; i < 3; ++i) { p.ld_a[i] = pad4(d.L[i].out); p.a[i] = o; o += ns * p.ld_a[i]; wide = max(wide, p.ld_a[i]); }
+    p.ld_o = pad4(d.L[3].out); p.o = o; o += ns * p.ld_o; wide = max(wide, p.ld_o);
+    p.d0 = o; o += ns * wide;
+    p.d1 = o; o += ns * wide;
+    p.total = o;
+    return p;
+}
+
+// Inverted dropout (torch.nn.Dropout in training mode) on the post-ReLU activations a[ns][units] of `layer`: a unit is kept
+// with probability 1 - p and then scaled by 1 / (1 - p).  The draw of (batch position s0 + s, layer, unit) is word 0 of the
+// Philox block with counter (unit, layer, position, step) and key seed: independent of how the batch is split into CTAs.
+__device__ __noinline__ void dropout_fwd(float *a, int ld, int ns, int units, int layer, int s0, const WorldStep &w, int mask_ld,
+                                         int mask_off)
+{
+    const float scale = 1.0f / (1.0f - w.p);
+    for (int idx = threadIdx.x; idx < ns * units; idx += kThreads) {
+        const int s = idx / units, k = idx - s * units;
+        Philox ph;
+        ph.key[0] = (uint32_t)w.seed; ph.key[1] = (uint32_t)(w.seed >> 32);
+        ph.ctr[0] = (uint32_t)k; ph.ctr[1] = (uint32_t)layer; ph.ctr[2] = (uint32_t)(s0 + s); ph.ctr[3] = w.step;
+        uint32_t r[4];
+        ph.block(r);
+        const bool keep = (float)(r[0] >> 8) * (1.0f / 16777216.0f) >= w.p;
+        float &v = a[(size_t)s * ld + k];
+        v = keep ? v * scale : 0.0f;
+        if (w.mask) w.mask[(size_t)(s0 + s) * mask_ld + mask_off + k] = keep ? 1 : 0;
+    }
+}
+
+// d(post-ReLU activation) -> times 1 / (1 - p): the dropped units were already zeroed by the ReLU gate (their activation is 0)
+__device__ __forceinline__ void dropout_bwd(float *g, int ld, int ns, int units, float p)
+{
+    const float scale = 1.0f / (1.0f - p);
+    for (int idx = threadIdx.x; idx < ns * units; idx += kThreads) {
+        const int s = idx / units, k = idx - s * units;
+        g[(size_t)s * ld + k] *= scale;
+    }
+    __syncthreads();
+}
+
+// MlpWorld: mlp (4H -> 128 -> 64 -> 12 -> 2H) on one row per sample, ReLU + dropout after layers 0 and 1, ReLU after layer 2,
+// tanh at the end; spc samples per CTA (CADRL's layout: every layer is one pass over its weight block).  Op list: forward
+// 0..3, backward-data 3, 2, 1 (no gradient w.r.t. the input).
+__global__ void __launch_bounds__(kThreads, 1)
+world_mlp_fwd_bwd_kernel(NetDims d, const float *__restrict__ Wt, const float *__restrict__ Wa, const float *__restrict__ X,
+                         const float *__restrict__ target, const int64_t *__restrict__ index, int B, int spc, int nbuf,
+                         WorldStep w, float *__restrict__ gpart, float *__restrict__ loss_part)
+{
+    extern __shared__ __align__(16) float sm[];
+    const int s0 = blockIdx.x * spc;
+    const int ns = min(spc, B - s0);
+    const MPlan p = make_mplan(d, ns);
+    const MPlan pmax = make_mplan(d, spc);              // the staging buffers sit behind the largest activation plan
+    const int tid = threadIdx.x, IN = d.L[0].in, O = d.L[3].out, U0 = d.L[0].out, U1 = d.L[1].out;
+    float *xs = sm + p.x, *o = sm + p.o, *d0 = sm + p.d0, *d1 = sm + p.d1;
+    float *a[3] = {sm + p.a[0], sm + p.a[1], sm + p.a[2]};
+    const bool drop = w.p > 0.0f && !w.fwd_only;
+    Staging st(d, Wt, Wa, sm + pad4(pmax.total), nbuf);
+
+    for (int idx = tid; idx < ns * p.ld_x; idx += kThreads) {
+        const int s = idx / p.ld_x, k = idx - s * p.ld_x;
+        const size_t item = index ? (size_t)index[s0 + s] : (size_t)(s0 + s);
+        xs[idx] = k < IN ? X[item * IN + k] : 0.0f;
+    }
+    st.fwd(0, xs, p.ld_x, ns, a[0], p.ld_a[0], true);
+    if (drop) dropout_fwd(a[0], p.ld_a[0], ns, U0, 0, s0, w, U0 + U1, 0);
+    st.fwd(1, a[0], p.ld_a[0], ns, a[1], p.ld_a[1], true);     // (begin_op's barrier publishes the dropout)
+    if (drop) dropout_fwd(a[1], p.ld_a[1], ns, U1, 1, s0, w, U0 + U1, U0);
+    st.fwd(2, a[1], p.ld_a[1], ns, a[2], p.ld_a[2], true);
+    st.fwd(3, a[2], p.ld_a[2], ns, o, p.ld_o, false);
+    for (int idx = tid; idx < ns * O; idx += kThreads) {
+        float &v = o[(size_t)(idx / O) * p.ld_o + idx % O];
+        v = tanhf(v);
+    }
+    __syncthreads();
+
+    // MSELoss(mean) over B x O outputs; tanh' = 1 - out^2
+    if (tid == 0) {
+        float ls = 0.0f;
+        for (int s = 0; s < ns; ++s) {
+            const float *y = target + (index ? (size_t)index[s0 + s] : (size_t)(s0 + s)) * O;
+            for (int k = 0; k < O; ++k) { const float df = o[(size_t)s * p.ld_o + k] - y[k]; ls += df * df; }
+        }
+        loss_part[blockIdx.x] = ls;
+    }
+    if (w.fwd_only) { st.finish(); return; }
+    float *G = gpart + (size_t)blockIdx.x * d.n_params;
+    const float norm = 2.0f / (float)((int64_t)B * O);
+    for (int idx = tid; idx < ns * O; idx += kThreads) {
+        const int s = idx / O, k = idx - s * O;
+        const float *y = target + (index ? (size_t)index[s0 + s] : (size_t)(s0 + s)) * O;
+        const float v = o[(size_t)s * p.ld_o + k];
+        d0[(size_t)s * p.ld_o + k] = norm * (v - y[k]) * (1.0f - v * v);
+    }
+    __syncthreads();
+    wgrad(d, G, 3, d0, p.ld_o, a[2], p.ld_a[2], ns);
+    st.bwd(3, d0, p.ld_o, ns, d1, p.ld_a[2], a[2], p.ld_a[2]);
+    wgrad(d, G, 2, d1, p.ld_a[2], a[1], p.ld_a[1], ns);
+    st.bwd(2, d1, p.ld_a[2], ns, d0, p.ld_a[1], a[1], p.ld_a[1]);
+    if (drop) dropout_bwd(d0, p.ld_a[1], ns, U1, w.p);
+    wgrad(d, G, 1, d0, p.ld_a[1], a[0], p.ld_a[0], ns);
+    st.bwd(1, d0, p.ld_a[1], ns, d1, p.ld_a[0], a[0], p.ld_a[0]);
+    if (drop) dropout_bwd(d1, p.ld_a[0], ns, U0, w.p);
+    wgrad(d, G, 0, d1, p.ld_a[0], xs, p.ld_x, ns);
+    st.finish();
+}
+
+constexpr int kWorldMlpSPC = kCadrlSPC;
+
 }  // namespace
 
-int trainer_spc(const NetDims &d) { return d.net == CN_NET_SARL ? kSarlSPC : d.net == CN_NET_CADRL ? kCadrlSPC : 1; }
+int trainer_spc(const NetDims &d)
+{
+    if (d.net == kNetWorldMlp) return kWorldMlpSPC;
+    return d.net == CN_NET_SARL ? kSarlSPC : d.net == CN_NET_CADRL ? kCadrlSPC : 1;
+}
 
 size_t trainer_smem(const NetDims &d, int H, int nbuf)
 {
-    const int act = d.net == CN_NET_SARL ? make_plan(d, H, kSarlSPC).total : make_nplan(d, H, trainer_spc(d)).total;
+    int act;
+    if (d.net == kNetWorldAttention) act = make_wplan(d, H).total;
+    else if (d.net == kNetWorldMlp) act = make_mplan(d, kWorldMlpSPC).total;
+    else act = d.net == CN_NET_SARL ? make_plan(d, H, kSarlSPC).total : make_nplan(d, H, trainer_spc(d)).total;
     return sizeof(float) * ((size_t)pad4(act) + (size_t)nbuf * d.wbuf_floats);
 }
 
 cudaError_t trainer_configure(const NetDims &d)
 {
-    const void *kernel = d.net == CN_NET_SARL ? (const void *)trainer_fwd_bwd_kernel : (const void *)trainer_nets_fwd_bwd_kernel;
+    const void *kernel = d.net == CN_NET_SARL ? (const void *)trainer_fwd_bwd_kernel
+                         : d.net == kNetWorldAttention ? (const void *)world_attention_fwd_bwd_kernel
+                         : d.net == kNetWorldMlp ? (const void *)world_mlp_fwd_bwd_kernel
+                                                 : (const void *)trainer_nets_fwd_bwd_kernel;
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTrainerMaxSmem);
 }
 
 int trainer_launch(const NetDims &d, const float *Wt, const float *Wa, const float *X, const float *target,
-                   const int64_t *index, int batch, int H, float *gpart, float *loss_part, int *nparts, cudaStream_t s)
+                   const int64_t *index, int batch, int H, float *gpart, float *loss_part, int *nparts, cudaStream_t s,
+                   const WorldStep *w)
 {
     const int spc = trainer_spc(d);
     *nparts = (batch + spc - 1) / spc;
@@ -518,6 +836,12 @@ int trainer_launch(const NetDims &d, const float *Wt, const float *Wa, const flo
     const size_t smem = trainer_smem(d, H, nbuf);
     if (d.net == CN_NET_SARL)
         trainer_fwd_bwd_kernel<<<*nparts, kThreads, smem, s>>>(d, Wt, Wa, X, target, index, batch, H, nbuf, gpart, loss_part);
+    else if (d.net == kNetWorldAttention)
+        world_attention_fwd_bwd_kernel<<<*nparts, kThreads, smem, s>>>(d, Wt, Wa, X, target, index, batch, H, nbuf, w->fwd_only,
+                                                                       gpart, loss_part);
+    else if (d.net == kNetWorldMlp)
+        world_mlp_fwd_bwd_kernel<<<*nparts, kThreads, smem, s>>>(d, Wt, Wa, X, target, index, batch, spc, nbuf, *w, gpart,
+                                                                 loss_part);
     else
         trainer_nets_fwd_bwd_kernel<<<*nparts, kThreads, smem, s>>>(d, Wt, Wa, X, target, index, batch, H, spc, nbuf, gpart,
                                                                     loss_part);

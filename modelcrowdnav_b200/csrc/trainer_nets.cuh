@@ -34,16 +34,42 @@ struct NetDims {
     int wbuf_floats;           // size of one staging buffer = the largest block
 };
 
+// The learned human-motion models (world_trainer.cu), next to the value networks' CN_NET_* kinds:
+// AttentionWorld: L[0..10] = mlp1.{0,2}, mlp2.{0,2}, attention.{0,2,4}, mlp3.{0,2,4,6} -- SARL's layers, in = 4, mlp3 on
+//   every human row with 2 outputs; one sample (H rows) per CTA.
+// MlpWorld: L[0..3] = mlp.{0,3,6,8} (4H -> 128 -> 64 -> 12 -> 2H, tanh at the end); several samples per CTA.
+constexpr int kNetWorldAttention = 16;
+constexpr int kNetWorldMlp = 17;
+
+// What a world-model step adds to a value-network step: inverted dropout after the ReLUs of MlpWorld's layers 0 and 1
+// (p = 0: none), and the forward-only form (validation: squared errors only, no gradient).
+struct WorldStep {
+    float p;                   // drop probability
+    uint64_t seed;
+    uint32_t step;             // the mask of (sample position, layer, unit) is a Philox draw keyed by (seed, step)
+    uint8_t *mask;             // optional [batch][L[0].out + L[1].out]: 1 = unit kept
+    int fwd_only;
+};
+
 // 227 kB: the opt-in dynamic shared memory of one CTA on sm_100
 constexpr size_t kTrainerMaxSmem = 232448;
 
-// Samples per CTA of the network (one SARL or LSTM-RL sample per CTA, several CADRL rows).
+// Samples per CTA of the network (one SARL, LSTM-RL or AttentionWorld sample per CTA, several CADRL / MlpWorld rows).
 int trainer_spc(const NetDims &d);
 // Shared memory of one CTA: activations for `H` humans and nbuf staging buffers (bytes).
 size_t trainer_smem(const NetDims &d, int H, int nbuf);
 // The network's kernel may use kTrainerMaxSmem (call after cudaSetDevice).
 cudaError_t trainer_configure(const NetDims &d);
 // Forward + backward of `batch` samples (item index[s] of X / target, or sample s itself when index is NULL) -> per-CTA
-// partial gradients gpart[cta][n_params] and squared errors loss_part[cta]; *nparts = CTAs launched.
+// partial gradients gpart[cta][n_params] and squared errors loss_part[cta]; *nparts = CTAs launched.  The world models
+// need `w` (their targets are batch x H x 2 velocities); with w->fwd_only the op list of d must end after the forward.
 int trainer_launch(const NetDims &d, const float *Wt, const float *Wa, const float *X, const float *target,
-                   const int64_t *index, int batch, int H, float *gpart, float *loss_part, int *nparts, cudaStream_t s);
+                   const int64_t *index, int batch, int H, float *gpart, float *loss_part, int *nparts, cudaStream_t s,
+                   const WorldStep *w = nullptr);
+
+// The transposed / aligned weight copies of d.L (t_off, a_off, t_size, a_size, wbuf_floats; trainer.cu) and the maps from
+// the flat block into them (flat index -> Wt index, -> Wa index).
+void trainer_layout(NetDims &d);
+void trainer_maps(const NetDims &d, int32_t *tmap, int32_t *amap);
+// Wt / Wa <- the flat block W (trainer.cu)
+int trainer_refresh(int n_params, const float *W, float *Wt, float *Wa, const int32_t *tmap, const int32_t *amap, cudaStream_t s);

@@ -168,7 +168,40 @@ mlp_world_kernel(WDims d, EnvDims ed, const float *__restrict__ W, const double 
     }
 }
 
+// cn_world_load_weights_device: the flat state-dict block (weight [out][in], bias per layer) -> W ([in][out], bias)
+__global__ void world_load_kernel(WDims d, int n, const float *__restrict__ flat, float *__restrict__ W)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    int base = 0;
+    for (int l = 0; l < d.n_layers; ++l) {
+        const WLayer &L = d.L[l];
+        const int nw = L.in * L.out;
+        if (i < base + nw) {
+            const int o = (i - base) / L.in, k = (i - base) - o * L.in;
+            W[L.w_off + k * L.out + o] = flat[i];
+            return;
+        }
+        if (i < base + nw + L.out) { W[L.b_off + i - base - nw] = flat[i]; return; }
+        base += nw + L.out;
+    }
+}
+
 }  // namespace
+
+int world_layer_dims(int kind, int human_num, int *ins, int *outs)
+{
+    if (kind == CN_WORLD_ATTENTION) {          // world_model.py:56-69
+        const int in_[11] = {4, 150, 100, 100, 200, 100, 100, 54, 150, 100, 100};
+        const int out_[11] = {150, 100, 100, 50, 100, 100, 1, 150, 100, 100, 2};
+        for (int i = 0; i < 11; ++i) { ins[i] = in_[i]; outs[i] = out_[i]; }
+        return 11;
+    }
+    const int in_[4] = {human_num * 4, 128, 64, 12};   // world_model.py:25-37
+    const int out_[4] = {128, 64, 12, human_num * 2};
+    for (int i = 0; i < 4; ++i) { ins[i] = in_[i]; outs[i] = out_[i]; }
+    return 4;
+}
 
 struct cn_world {
     int device;
@@ -192,17 +225,9 @@ int cn_world_create(int32_t kind, int32_t human_num, int device, cn_world **out)
     w->device = device;
     WDims &d = w->d;
     d.kind = kind; d.H = human_num;
-    if (kind == CN_WORLD_ATTENTION) {          // world_model.py:56-69
-        const int ins[11] = {4, 150, 100, 100, 200, 100, 100, 54, 150, 100, 100};
-        const int outs[11] = {150, 100, 100, 50, 100, 100, 1, 150, 100, 100, 2};
-        d.n_layers = 11;
-        for (int i = 0; i < 11; ++i) { d.L[i].in = ins[i]; d.L[i].out = outs[i]; }
-    } else {                                   // world_model.py:25-37
-        const int ins[4] = {human_num * 4, 128, 64, 12};
-        const int outs[4] = {128, 64, 12, human_num * 2};
-        d.n_layers = 4;
-        for (int i = 0; i < 4; ++i) { d.L[i].in = ins[i]; d.L[i].out = outs[i]; }
-    }
+    int ins[kMaxLayers], outs[kMaxLayers];
+    d.n_layers = world_layer_dims(kind, human_num, ins, outs);
+    for (int i = 0; i < d.n_layers; ++i) { d.L[i].in = ins[i]; d.L[i].out = outs[i]; }
     int off = 0;
     for (int i = 0; i < d.n_layers; ++i) {
         d.L[i].w_off = off; off += d.L[i].in * d.L[i].out;
@@ -250,6 +275,17 @@ int cn_world_load_weights(cn_world *w, const float *flat_host, int64_t n, void *
     }
     CN_CUDA_CHECK(cudaMemcpyAsync(w->W, t.data(), sizeof(float) * n, cudaMemcpyHostToDevice, s));
     CN_CUDA_CHECK(cudaStreamSynchronize(s));
+    w->loaded = 1;
+    return CN_OK;
+}
+
+int cn_world_load_weights_device(cn_world *w, const float *flat_dev, int64_t n, void *stream)
+{
+    if (!w || !flat_dev) { cn_set_error("null argument"); return CN_EINVAL; }
+    if (n != w->n_params) { cn_set_error("expected %lld parameters, got %lld", (long long)w->n_params, (long long)n); return CN_EINVAL; }
+    CN_CUDA_CHECK(cudaSetDevice(w->device));
+    world_load_kernel<<<(int)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(w->d, (int)n, flat_dev, w->W);
+    CN_LAUNCH_CHECK();
     w->loaded = 1;
     return CN_OK;
 }

@@ -96,6 +96,7 @@ class MlpWorld(_DeviceWorld):
     def __init__(self, num_human, drop_rate=0.5, multihuman=True):
         super().__init__()
         self.num_human = num_human if multihuman else 1
+        self.drop_rate = drop_rate          # the Dropout layers' p in training mode (world_trainer.WorldTrainer)
         self.mlp = _linear_stack([self.num_human * 4, 128, 64, 12, self.num_human * 2], [0, 3, 6, 8])
         self._init_device_state()
 
